@@ -3,11 +3,13 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
                     [--precision bf16|bf16x3|fp32] [--clips-per-gpu C] [--chunk M] [--no-configs]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (K2 STCNN + visual stats | K1 MFCC stats for 41 shifts -> K4
 scores + arg-max, plus the cross-rank score gather when N > 1) over one batch of synthetic clips:
 C clips per GPU, fixed as N grows (weak scaling; N = 8, C = 1024 is BASELINE config 3's 8192 clips).
-Prints ONE JSON line (rank 0).
+Prints ONE JSON line (rank 0).  --dump-outputs DIR also writes what the last timed step returned (see dump_outputs):
+inputs and weights come from fixed seeds, so two builds run with the same arguments can be compared output for output.
 
   value      device-resident throughput (inputs already in HBM), CUDA events, max over ranks
   e2e        the same sweep through the host-buffer entry point: pinned host inputs, H2D / D2H inside the timed
@@ -149,6 +151,24 @@ def frames_f32(frames_u8: torch.Tensor, pin: bool = True) -> torch.Tensor:
     for i in range(0, frames_u8.shape[0], 64):
         out[i:i + 64] = (frames_u8[i:i + 64].to(torch.float64) / 255.0).to(torch.float32)
     return out
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, scores: np.ndarray, best: np.ndarray):
+    """Writes the sweep's results as out_dir/scores.npy (float32 [clips, 41], sigmoid score of every offset) and
+    out_dir/best.npy (float64 [clips], best offset in frames).  Should they exceed 64 MB, a fixed seeded sample of
+    clips is written instead, with the sampled clip indices in out_dir/clips.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    n, k = scores.shape
+    row_bytes = 4 * k + 8
+    if n * row_bytes > DUMP_BYTES - 4096:                  # 4096: room for the .npy headers
+        keep = np.sort(np.random.default_rng(0).choice(n, (DUMP_BYTES - 4096) // (row_bytes + 8), replace=False))
+        scores, best = scores[keep], best[keep]
+        np.save(os.path.join(out_dir, "clips.npy"), keep.astype(np.float64))
+    np.save(os.path.join(out_dir, "scores.npy"), scores.astype(np.float32))
+    np.save(os.path.join(out_dir, "best.npy"), best.astype(np.float64))
 
 
 def parity_stats(scores, best, scores_ref, best_ref):
@@ -414,7 +434,13 @@ def main():
     ap.add_argument("--cpu-clips", type=int, default=16, help="timed clips of the cpu_baseline sample (0 = skip)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the other BASELINE configs and the parity pass")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the scores and best offsets of the last timed step "
+                                                           "to DIR/*.npy (native arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs needs --impl native")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -424,8 +450,7 @@ def main():
         return
     if world != args.gpus and world > 1:
         raise SystemExit(f"--gpus {args.gpus} but WORLD_SIZE={world}")
-    if args.steps < 1 or args.warmup < 3:
-        args.warmup = max(args.warmup, 3)
+    args.warmup = max(args.warmup, 3)
 
     import torch.distributed as dist
     import avsync_b200 as A
@@ -477,6 +502,8 @@ def main():
     ev1.record()
     barrier()
     L.avs_prof_enable(0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, scores.cpu().numpy(), best.cpu().numpy())
     # a timed region shorter than ~0.4 s may see fewer than three 100 ms samples: keep the GPU under the identical load
     # (untimed steps, all ranks) until three have been taken
     extra = torch.zeros(1, device=dev, dtype=torch.int32)
