@@ -17,6 +17,7 @@
 #include <cmath>
 #include <map>
 #include <tuple>
+#include <unordered_map>
 #include <vector>
 #include "stcnn.cuh"
 
@@ -30,10 +31,9 @@ constexpr int kMaxQ = 40;
 
 }  // namespace avs
 
-struct avs_mfcc_plan {
-  int n_samples, sr, hop, n_mfcc, n_shifts, n_frames, n_unique;
-  int4* d_frames = nullptr;     // [U] (p, a, b, 0): window start, valid range in original-signal coordinates
-  int* d_map = nullptr;         // [K][F] -> unique frame id
+namespace avs {
+// Device tables shared by every frame plan of one (sample rate, n_mfcc): window, FFT twiddles, mel filterbank, DCT.
+struct MfccTables {
   float* d_window = nullptr;    // [2048] periodic Hann
   float2* d_tw = nullptr;       // [32 k1][32 lanes] exp(-2 pi i (lane * k1) / 1024): lane-major, one 256-byte run per k1
   float2* d_tw2 = nullptr;      // [1025] exp(-2 pi i k / 2048)
@@ -41,6 +41,20 @@ struct avs_mfcc_plan {
   float* d_mel_w = nullptr;     // non-zero filter weights, lane-major per quartile of bands: [quartile][i][32 bands], zero padded
   float* d_dct = nullptr;       // [128][kMaxQ] DCT-II ortho basis, transposed, zero padded (statistics kernel)
   float4* d_dct_lane = nullptr; // the same basis lane-major for the log-mel kernel: [4 quartiles][kMaxQ / 4][32 bands] float4
+};
+// Per-clip descriptor of a ragged plan: where the clip's audio starts in the packed buffer, where its unique frames start
+// in the plan's flat frame list (and in the per-frame tables), where its [K][n_frames] map starts, and its frame count.
+struct RaggedClip {
+  long long audio_off;
+  int ubase, map_base, n_frames, pad;
+};
+}  // namespace avs
+
+struct avs_mfcc_plan {
+  int n_samples, sr, hop, n_mfcc, n_shifts, n_frames, n_unique;
+  int4* d_frames = nullptr;     // [U] (p, a, b, 0): window start, valid range in original-signal coordinates
+  int* d_map = nullptr;         // [K][F] -> unique frame id
+  avs::MfccTables tab;
 };
 
 namespace avs {
@@ -120,12 +134,16 @@ __host__ __device__ constexpr int bitrev5(int i) {
 
 // SCHED = false: one-warp CTAs, frame = blockIdx.x.  SCHED = true: four-warp CTAs, two frames per CTA, taken by the warps
 // that sit on schedulers 0 and 2 (see kFftCtaWarps).  NQ: padded n_mfcc (20 or 40) of the fused per-frame DCT.
-template <bool SCHED, int NQ>
+// RAGGED = false: clip = blockIdx.y, frame u of the clip's n_unique, audio [clip][n_samples].  RAGGED = true: u indexes the
+// launch's flat list of n_unique (clip, unique frame) pairs, the frame's 4th int is its clip, clips[clip].audio_off finds the
+// clip's audio in the packed buffer, and the per-frame tables are indexed by u.
+template <bool SCHED, int NQ, bool RAGGED = false>
 __global__ void __launch_bounds__(SCHED ? 32 * kFftCtaWarps : 32 * kWarpFftWarps)
 mfcc_logmel_warp_kernel(const float* __restrict__ audio, int n_samples, const int4* __restrict__ frames, int n_unique,
                         const float* __restrict__ window, const float2* __restrict__ tw, const float2* __restrict__ tw2,
                         const int4* __restrict__ mel_tab, const float* __restrict__ mel_w, const float4* __restrict__ dct_lane,
-                        float* __restrict__ logmel, float* __restrict__ frame_mfcc, float2* __restrict__ frame_range) {
+                        float* __restrict__ logmel, float* __restrict__ frame_mfcc, float2* __restrict__ frame_range,
+                        const RaggedClip* __restrict__ clips) {
   // one 32 x 33 float plane per warp (4.2 KB): the transposes move the real and the imaginary parts one after the other,
   // so that twice as many of these one-warp CTAs fit into the shared memory the persistent conv kernels leave free
   __shared__ float s_z[SCHED ? kFftCtaFrames : kWarpFftWarps][32 * 33];
@@ -164,6 +182,7 @@ mfcc_logmel_warp_kernel(const float* __restrict__ audio, int n_samples, const in
   float* z = s_z[zslot];
   const float* x = audio + static_cast<size_t>(clip) * n_samples;
   const int4 fr = frames[u];
+  if (RAGGED) x = audio + clips[fr.w].audio_off;
   float2 v[32];
   // z[n] = w[2n] x[p+2n] + i w[2n+1] x[p+2n+1] (zero outside [lo, hi)), n = 32*n1 + lane: lane = n2
   // interior frames (the window lies inside the valid range and starts on an 8-byte boundary: every frame of the
@@ -260,7 +279,7 @@ mfcc_logmel_warp_kernel(const float* __restrict__ audio, int n_samples, const in
   // load request — the kernel sat at 68 % of the L1 throughput alone, and beside a conv CTA, whose operand fetch owns
   // that pipe, it ran four times slower).  Zero weights leave the sums bit-identical; the padded reads stay inside the
   // plane (index clamped to the last bin).
-  float* out = logmel + (static_cast<size_t>(clip) * n_unique + u) * kMels;
+  float* out = logmel + (RAGGED ? static_cast<size_t>(u) : static_cast<size_t>(clip) * n_unique + u) * kMels;
   float lm[kMels / 32];
 #pragma unroll
   for (int r = 0; r < kMels / 32; ++r) {
@@ -283,7 +302,7 @@ mfcc_logmel_warp_kernel(const float* __restrict__ audio, int n_samples, const in
   float mx = fmaxf(fmaxf(lm[0], lm[1]), fmaxf(lm[2], lm[3])), mn = fminf(fminf(lm[0], lm[1]), fminf(lm[2], lm[3]));
   mx = warp_max(mx);
   mn = -warp_max(-mn);
-  const size_t f = static_cast<size_t>(clip) * n_unique + u;
+  const size_t f = RAGGED ? static_cast<size_t>(u) : static_cast<size_t>(clip) * n_unique + u;
   // DCT: every lane forms the partial sums of its four bands for all NQ coefficients (the basis row of a band is NQ
   // consecutive floats), then the 32 partial vectors are summed with a halving exchange: in the round for lane bit b a
   // lane keeps one half of its remaining coefficients and ships the other half to lane ^ (1 << b), so the reduction
@@ -327,19 +346,23 @@ mfcc_logmel_warp_kernel(const float* __restrict__ audio, int n_samples, const in
 // One CTA per (shift, clip).  128 threads; thread j owns frames j, j+128, ...  The shift's frames are gathered through
 // the map: top_db floor from the per-frame maxima, then per frame either the precomputed DCT (the clamp does not touch
 // the frame: its min is above the floor) or, for frames the clamp does touch, DCT(max(x, floor)) recomputed here.
-template <int NQ>
+// RAGGED: the clip's frame count and map come from clips[clip]; n_unique is then the flat index of the first frame the
+// per-frame tables hold, and out_mfcc is not written.
+template <int NQ, bool RAGGED = false>
 __global__ void __launch_bounds__(128)
 mfcc_stats_kernel(const float* __restrict__ logmel, const float* __restrict__ frame_mfcc, const float2* __restrict__ frame_range,
                   const int* __restrict__ map, int n_unique, int n_frames, int n_shifts, int n_mfcc,
-                  const float* __restrict__ dct_t, float* __restrict__ out_stats, float* __restrict__ out_mfcc) {
+                  const float* __restrict__ dct_t, float* __restrict__ out_stats, float* __restrict__ out_mfcc,
+                  const RaggedClip* __restrict__ clips) {
   extern __shared__ float smem[];
   float* s_dct = smem;                       // [128][NQ], filled only when some frame needs the clamp
   float* s_mfcc = smem + kMels * NQ;         // [F][NQ]
   __shared__ float s_red[4];
   const int tid = threadIdx.x;
   const int k = blockIdx.x, clip = blockIdx.y;
-  const int* mp = map + static_cast<size_t>(k) * n_frames;
-  const size_t cbase = static_cast<size_t>(clip) * n_unique;
+  if (RAGGED) n_frames = clips[clip].n_frames;
+  const int* mp = map + (RAGGED ? clips[clip].map_base : 0) + static_cast<size_t>(k) * n_frames;
+  const size_t cbase = RAGGED ? static_cast<size_t>(clips[clip].ubase - n_unique) : static_cast<size_t>(clip) * n_unique;
   const float* lm = logmel + cbase * kMels;
 
   // global max over this shifted signal's [n_mels, n_frames] log-mel array (power_to_db top_db reference)
@@ -395,7 +418,7 @@ mfcc_stats_kernel(const float* __restrict__ logmel, const float* __restrict__ fr
     for (int q = 0; q < NQ; ++q) s_mfcc[j * NQ + q] = acc[q];
   }
   __syncthreads();
-  if (out_mfcc != nullptr) {
+  if (!RAGGED && out_mfcc != nullptr) {
     float* om = out_mfcc + (static_cast<size_t>(clip) * n_shifts + k) * n_frames * n_mfcc;
     for (int i = tid; i < n_frames * n_mfcc; i += 128) om[i] = s_mfcc[(i / n_mfcc) * NQ + (i % n_mfcc)];
   }
@@ -431,6 +454,114 @@ static int upload(T** dst, const std::vector<T>& v) {
   AVS_CUDA(cudaMalloc(reinterpret_cast<void**>(dst), std::max<size_t>(v.size(), 1) * sizeof(T)));
   if (!v.empty()) AVS_CUDA(cudaMemcpy(*dst, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
   return AVS_OK;
+}
+// Stream-ordered upload: allocation and copy are queued on `st` and wait for nothing else.  A copy from pageable memory
+// returns once the source has been staged, so `v` may be released as soon as this returns.
+template <class T>
+static int upload_async(T** dst, const std::vector<T>& v, cudaStream_t st) {
+  AVS_CUDA(cudaMallocAsync(reinterpret_cast<void**>(dst), std::max<size_t>(v.size(), 1) * sizeof(T), st));
+  if (!v.empty()) AVS_CUDA(cudaMemcpyAsync(*dst, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice, st));
+  return AVS_OK;
+}
+
+// Host images of the constant tables (computed in double, stored in float).
+struct HostTables {
+  std::vector<float> window, mel_w, dct;
+  std::vector<float2> tw, tw2;
+  std::vector<int4> mel_tab;
+  std::vector<float4> dct_lane;
+};
+static void build_tables(int sample_rate, int n_mfcc, HostTables& t) {
+  const double kPi = 3.14159265358979323846;
+  std::vector<float>& window = t.window;
+  window.resize(kNfft);
+  for (int n = 0; n < kNfft; ++n) window[n] = static_cast<float>(0.5 - 0.5 * std::cos(2.0 * kPi * n / kNfft));
+  std::vector<float2>& tw = t.tw;
+  std::vector<float2>& tw2 = t.tw2;
+  tw.resize(32 * 32);
+  tw2.resize(kBins);
+  for (int k1 = 0; k1 < 32; ++k1)
+    for (int lane = 0; lane < 32; ++lane) {
+      const int e = (lane * k1) & (kHalf - 1);
+      tw[32 * k1 + lane] = make_float2(static_cast<float>(std::cos(2.0 * kPi * e / kHalf)), static_cast<float>(-std::sin(2.0 * kPi * e / kHalf)));
+    }
+  for (int k = 0; k < kBins; ++k)
+    tw2[k] = make_float2(static_cast<float>(std::cos(2.0 * kPi * k / kNfft)), static_cast<float>(-std::sin(2.0 * kPi * k / kNfft)));
+  // librosa.filters.mel(sr, n_fft=2048, n_mels=128, fmin=0, fmax=sr/2, htk=False, norm='slaney')
+  std::vector<double> mel_f(kMels + 2);
+  const double mmin = hz_to_mel(0.0), mmax = hz_to_mel(sample_rate / 2.0);
+  for (int i = 0; i < kMels + 2; ++i) mel_f[i] = mel_to_hz(mmin + (mmax - mmin) * i / (kMels + 1));
+  std::vector<int4>& rng = t.mel_tab;
+  rng.resize(kMels);
+  std::vector<std::vector<float>> band(kMels);
+  for (int m = 0; m < kMels; ++m) {
+    const double enorm = 2.0 / (mel_f[m + 2] - mel_f[m]);
+    int first = -1, last = -2;
+    std::vector<float> row(kBins);
+    for (int k = 0; k < kBins; ++k) {
+      const double f = static_cast<double>(k) * sample_rate / kNfft;
+      const double lower = (f - mel_f[m]) / (mel_f[m + 1] - mel_f[m]);
+      const double upper = (mel_f[m + 2] - f) / (mel_f[m + 2] - mel_f[m + 1]);
+      const float w32 = static_cast<float>(std::max(0.0, std::min(lower, upper)));
+      row[k] = static_cast<float>(static_cast<double>(w32) * enorm);
+      if (row[k] != 0.f) {
+        if (first < 0) first = k;
+        last = k;
+      }
+    }
+    if (first < 0) first = 0, last = -1;
+    rng[m] = make_int4(first, 0, 0, last - first + 1);
+    for (int k = first; k <= last; ++k) band[m].push_back(row[k]);
+  }
+  std::vector<float>& mw = t.mel_w;
+  for (int r = 0; r < kMels / 32; ++r) {  // lane-major weights of the quartile's 32 bands, zero padded to an even length
+    size_t longest = 0;
+    for (int l = 0; l < 32; ++l) longest = std::max(longest, band[32 * r + l].size());
+    longest = (longest + 1) & ~static_cast<size_t>(1);
+    const int off = static_cast<int>(mw.size());
+    mw.resize(mw.size() + longest * 32, 0.f);
+    for (int l = 0; l < 32; ++l) {
+      for (size_t i = 0; i < band[32 * r + l].size(); ++i) mw[off + i * 32 + l] = band[32 * r + l][i];
+      rng[32 * r + l].y = static_cast<int>(longest);
+      rng[32 * r + l].z = off;
+    }
+  }
+  std::vector<float>& dct = t.dct;
+  dct.assign(static_cast<size_t>(kMels) * kMaxQ, 0.f);
+  for (int q = 0; q < n_mfcc; ++q)
+    for (int m = 0; m < kMels; ++m) {
+      double v = std::cos(kPi * q * (2 * m + 1) / (2.0 * kMels)) * std::sqrt(2.0 / kMels);
+      if (q == 0) v *= std::sqrt(0.5);
+      dct[static_cast<size_t>(m) * kMaxQ + q] = static_cast<float>(v);
+    }
+  std::vector<float4>& dct_lane = t.dct_lane;
+  dct_lane.resize(static_cast<size_t>(kMels / 32) * (kMaxQ / 4) * 32);
+  for (int m = 0; m < kMels; ++m)
+    for (int q4 = 0; q4 < kMaxQ / 4; ++q4) {
+      const float* d = &dct[static_cast<size_t>(m) * kMaxQ + 4 * q4];
+      dct_lane[(static_cast<size_t>(m / 32) * (kMaxQ / 4) + q4) * 32 + (m & 31)] = make_float4(d[0], d[1], d[2], d[3]);
+    }
+}
+// Device copies of the constant tables: synchronous for the uniform plan, queued on `st` for the ragged one.
+static int upload_tables(MfccTables& d, const HostTables& h, cudaStream_t st, bool async) {
+  int rc;
+  if (async) {
+    if ((rc = upload_async(&d.d_window, h.window, st)) || (rc = upload_async(&d.d_tw, h.tw, st)) ||
+        (rc = upload_async(&d.d_tw2, h.tw2, st)) || (rc = upload_async(&d.d_mel_tab, h.mel_tab, st)) ||
+        (rc = upload_async(&d.d_mel_w, h.mel_w, st)) || (rc = upload_async(&d.d_dct, h.dct, st)) ||
+        (rc = upload_async(&d.d_dct_lane, h.dct_lane, st)))
+      return rc;
+    return AVS_OK;
+  }
+  if ((rc = upload(&d.d_window, h.window)) || (rc = upload(&d.d_tw, h.tw)) || (rc = upload(&d.d_tw2, h.tw2)) ||
+      (rc = upload(&d.d_mel_tab, h.mel_tab)) || (rc = upload(&d.d_mel_w, h.mel_w)) || (rc = upload(&d.d_dct, h.dct)) ||
+      (rc = upload(&d.d_dct_lane, h.dct_lane)))
+    return rc;
+  return AVS_OK;
+}
+static void free_tables(MfccTables& d) {
+  cudaFree(d.d_window); cudaFree(d.d_tw); cudaFree(d.d_tw2); cudaFree(d.d_mel_tab); cudaFree(d.d_mel_w); cudaFree(d.d_dct);
+  cudaFree(d.d_dct_lane);
 }
 
 // Host-side frame plan: every (shift, frame) pair becomes a key (start, lo, hi) in ORIGINAL-signal
@@ -527,73 +658,10 @@ extern "C" int avs_mfcc_plan_create(int n_samples, int sample_rate, int n_mfcc, 
   build_frame_plan(n_samples, p->hop, shift_samples, n_shifts, p->n_frames, frames, map);
   p->n_unique = static_cast<int>(frames.size());
 
-  // ---- constant tables (computed in double, stored in float)
-  const double kPi = 3.14159265358979323846;
-  std::vector<float> window(kNfft);
-  for (int n = 0; n < kNfft; ++n) window[n] = static_cast<float>(0.5 - 0.5 * std::cos(2.0 * kPi * n / kNfft));
-  std::vector<float2> tw(32 * 32), tw2(kBins);
-  for (int k1 = 0; k1 < 32; ++k1)
-    for (int lane = 0; lane < 32; ++lane) {
-      const int e = (lane * k1) & (kHalf - 1);
-      tw[32 * k1 + lane] = make_float2(static_cast<float>(std::cos(2.0 * kPi * e / kHalf)), static_cast<float>(-std::sin(2.0 * kPi * e / kHalf)));
-    }
-  for (int k = 0; k < kBins; ++k)
-    tw2[k] = make_float2(static_cast<float>(std::cos(2.0 * kPi * k / kNfft)), static_cast<float>(-std::sin(2.0 * kPi * k / kNfft)));
-  // librosa.filters.mel(sr, n_fft=2048, n_mels=128, fmin=0, fmax=sr/2, htk=False, norm='slaney')
-  std::vector<double> mel_f(kMels + 2);
-  const double mmin = hz_to_mel(0.0), mmax = hz_to_mel(sample_rate / 2.0);
-  for (int i = 0; i < kMels + 2; ++i) mel_f[i] = mel_to_hz(mmin + (mmax - mmin) * i / (kMels + 1));
-  std::vector<int4> rng(kMels);
-  std::vector<std::vector<float>> band(kMels);
-  for (int m = 0; m < kMels; ++m) {
-    const double enorm = 2.0 / (mel_f[m + 2] - mel_f[m]);
-    int first = -1, last = -2;
-    std::vector<float> row(kBins);
-    for (int k = 0; k < kBins; ++k) {
-      const double f = static_cast<double>(k) * sample_rate / kNfft;
-      const double lower = (f - mel_f[m]) / (mel_f[m + 1] - mel_f[m]);
-      const double upper = (mel_f[m + 2] - f) / (mel_f[m + 2] - mel_f[m + 1]);
-      const float w32 = static_cast<float>(std::max(0.0, std::min(lower, upper)));
-      row[k] = static_cast<float>(static_cast<double>(w32) * enorm);
-      if (row[k] != 0.f) {
-        if (first < 0) first = k;
-        last = k;
-      }
-    }
-    if (first < 0) first = 0, last = -1;
-    rng[m] = make_int4(first, 0, 0, last - first + 1);
-    for (int k = first; k <= last; ++k) band[m].push_back(row[k]);
-  }
-  std::vector<float> mw;
-  for (int r = 0; r < kMels / 32; ++r) {  // lane-major weights of the quartile's 32 bands, zero padded to an even length
-    size_t longest = 0;
-    for (int l = 0; l < 32; ++l) longest = std::max(longest, band[32 * r + l].size());
-    longest = (longest + 1) & ~static_cast<size_t>(1);
-    const int off = static_cast<int>(mw.size());
-    mw.resize(mw.size() + longest * 32, 0.f);
-    for (int l = 0; l < 32; ++l) {
-      for (size_t i = 0; i < band[32 * r + l].size(); ++i) mw[off + i * 32 + l] = band[32 * r + l][i];
-      rng[32 * r + l].y = static_cast<int>(longest);
-      rng[32 * r + l].z = off;
-    }
-  }
-  std::vector<float> dct(static_cast<size_t>(kMels) * kMaxQ, 0.f);
-  for (int q = 0; q < n_mfcc; ++q)
-    for (int m = 0; m < kMels; ++m) {
-      double v = std::cos(kPi * q * (2 * m + 1) / (2.0 * kMels)) * std::sqrt(2.0 / kMels);
-      if (q == 0) v *= std::sqrt(0.5);
-      dct[static_cast<size_t>(m) * kMaxQ + q] = static_cast<float>(v);
-    }
-  std::vector<float4> dct_lane(static_cast<size_t>(kMels / 32) * (kMaxQ / 4) * 32);
-  for (int m = 0; m < kMels; ++m)
-    for (int q4 = 0; q4 < kMaxQ / 4; ++q4) {
-      const float* d = &dct[static_cast<size_t>(m) * kMaxQ + 4 * q4];
-      dct_lane[(static_cast<size_t>(m / 32) * (kMaxQ / 4) + q4) * 32 + (m & 31)] = make_float4(d[0], d[1], d[2], d[3]);
-    }
+  HostTables tabs;
+  build_tables(sample_rate, n_mfcc, tabs);
   int rc;
-  if ((rc = upload(&p->d_frames, frames)) || (rc = upload(&p->d_map, map)) || (rc = upload(&p->d_window, window)) ||
-      (rc = upload(&p->d_tw, tw)) || (rc = upload(&p->d_tw2, tw2)) || (rc = upload(&p->d_mel_tab, rng)) || (rc = upload(&p->d_mel_w, mw)) || (rc = upload(&p->d_dct, dct)) ||
-      (rc = upload(&p->d_dct_lane, dct_lane))) {
+  if ((rc = upload(&p->d_frames, frames)) || (rc = upload(&p->d_map, map)) || (rc = upload_tables(p->tab, tabs, nullptr, false))) {
     avs_mfcc_plan_destroy(p);
     return rc;
   }
@@ -603,32 +671,37 @@ extern "C" int avs_mfcc_plan_create(int n_samples, int sample_rate, int n_mfcc, 
 
 extern "C" void avs_mfcc_plan_destroy(avs_mfcc_plan* p) {
   if (!p) return;
-  cudaFree(p->d_frames); cudaFree(p->d_map); cudaFree(p->d_window); cudaFree(p->d_tw); cudaFree(p->d_tw2);
-  cudaFree(p->d_mel_tab); cudaFree(p->d_mel_w); cudaFree(p->d_dct); cudaFree(p->d_dct_lane);
+  cudaFree(p->d_frames); cudaFree(p->d_map);
+  free_tables(p->tab);
   delete p;
 }
 extern "C" int avs_mfcc_plan_unique_frames(const avs_mfcc_plan* p) { return p ? p->n_unique : AVS_EINVAL; }
 extern "C" int avs_mfcc_plan_frames(const avs_mfcc_plan* p) { return p ? p->n_frames : AVS_EINVAL; }
+// log-mel rows, per-frame DCT rows, per-frame (max, min) of n_fr frames
+size_t avs::mfcc_frame_ws_bytes(size_t n_fr) {
+  return align_up(n_fr * kMels * sizeof(float), 256) + align_up(n_fr * kMaxQ * sizeof(float), 256) +
+         align_up(n_fr * sizeof(float2), 256);
+}
 extern "C" size_t avs_mfcc_workspace_bytes(const avs_mfcc_plan* p, int n_clips) {
   if (!p || n_clips <= 0) return 0;
-  // log-mel rows, per-frame DCT rows, per-frame (max, min)
-  const size_t frames = static_cast<size_t>(n_clips) * p->n_unique;
-  return align_up(frames * kMels * sizeof(float), 256) + align_up(frames * kMaxQ * sizeof(float), 256) +
-         align_up(frames * sizeof(float2), 256);
+  return mfcc_frame_ws_bytes(static_cast<size_t>(n_clips) * p->n_unique);
 }
 
 namespace {
 struct MfccWs {
   float* logmel; float* frame_mfcc; float2* frame_range;
 };
-// placement of the three per-frame tables in a workspace carved for n_clips clips
-MfccWs carve_mfcc_ws(const avs_mfcc_plan* p, int n_clips, void* workspace) {
-  const size_t n_fr = static_cast<size_t>(n_clips) * p->n_unique;
+// placement of the three per-frame tables of n_fr frames in a workspace
+MfccWs carve_frame_ws(size_t n_fr, void* workspace) {
   MfccWs w;
   w.logmel = static_cast<float*>(workspace);
   w.frame_mfcc = reinterpret_cast<float*>(static_cast<uint8_t*>(workspace) + align_up(n_fr * kMels * sizeof(float), 256));
   w.frame_range = reinterpret_cast<float2*>(reinterpret_cast<uint8_t*>(w.frame_mfcc) + align_up(n_fr * kMaxQ * sizeof(float), 256));
   return w;
+}
+// the same for a workspace carved for n_clips clips of a uniform plan
+MfccWs carve_mfcc_ws(const avs_mfcc_plan* p, int n_clips, void* workspace) {
+  return carve_frame_ws(static_cast<size_t>(n_clips) * p->n_unique, workspace);
 }
 int check_mfcc_ws(const avs_mfcc_plan* p, int n_clips, size_t workspace_bytes) {
   if (workspace_bytes < avs_mfcc_workspace_bytes(p, n_clips)) {
@@ -657,7 +730,7 @@ int avs::mfcc_logmel_part(const avs_mfcc_plan* p, const float* audio, int n_clip
     float2* frg = w.frame_range + static_cast<size_t>(c0) * p->n_unique;
     const float* au = audio + static_cast<size_t>(c0) * p->n_samples;
     ProfScope ps(PROF_LOGMEL, st);
-#define AVS_LOGMEL_ARGS au, p->n_samples, p->d_frames, p->n_unique, p->d_window, p->d_tw, p->d_tw2, p->d_mel_tab, p->d_mel_w, p->d_dct_lane, lm, fmf, frg
+#define AVS_LOGMEL_ARGS au, p->n_samples, p->d_frames, p->n_unique, p->tab.d_window, p->tab.d_tw, p->tab.d_tw2, p->tab.d_mel_tab, p->tab.d_mel_w, p->tab.d_dct_lane, lm, fmf, frg, nullptr
 #ifdef AVS_EXPERIMENTS
     if (fft_sched_mode()) {
       const dim3 g1(cdiv(p->n_unique, kFftCtaFrames), nc);
@@ -701,12 +774,12 @@ int avs::mfcc_stats_part(const avs_mfcc_plan* p, int n_clips, float* out_stats, 
       const size_t sm = (static_cast<size_t>(kMels) * 20 + static_cast<size_t>(p->n_frames) * 20) * sizeof(float);
       AVS_CUDA(cudaFuncSetAttribute(mfcc_stats_kernel<20>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(sm)));
       mfcc_stats_kernel<20><<<g2, 128, sm, st>>>(lm, fmf, frg, p->d_map, p->n_unique, p->n_frames, p->n_shifts, p->n_mfcc,
-                                                 p->d_dct, os, om);
+                                                 p->tab.d_dct, os, om, nullptr);
     } else {
       const size_t sm = (static_cast<size_t>(kMels) * kMaxQ + static_cast<size_t>(p->n_frames) * kMaxQ) * sizeof(float);
       AVS_CUDA(cudaFuncSetAttribute(mfcc_stats_kernel<kMaxQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(sm)));
       mfcc_stats_kernel<kMaxQ><<<g2, 128, sm, st>>>(lm, fmf, frg, p->d_map, p->n_unique, p->n_frames, p->n_shifts, p->n_mfcc,
-                                                    p->d_dct, os, om);
+                                                    p->tab.d_dct, os, om, nullptr);
     }
     AVS_LAUNCHED();
   }
@@ -737,4 +810,415 @@ extern "C" __attribute__((visibility("hidden"))) int avs_mfcc_plan_nshifts_inter
   *n_mfcc = p->n_mfcc;
   *n_samples = p->n_samples;
   return AVS_OK;
+}
+
+// ================================================================================================ ragged plans
+// A batch of clips with their own lengths and their own rows of shifts (a clip's row follows from its frame rate), at
+// one sample rate and one n_mfcc.  Clip i's audio sits at audio_off[i] of one packed buffer (offsets rounded up to 4
+// samples, so that interior frames keep the paired-load path of the log-mel kernel); its unique frames are the range
+// [ubase[i], ubase[i+1]) of one flat frame list, each frame carrying its clip in the 4th int; its [K][F_i] map holds
+// clip-local ids.  Per clip the frames and the map are exactly those of a uniform plan of that clip alone (same keys,
+// same map resolved to keys), so the kernels compute the same values and sum them in the same order.
+struct avs_mfcc_ragged_plan {
+  int n_clips, sr, hop, n_mfcc, n_shifts, max_frames;
+  std::vector<long long> audio_off;  // [n_clips + 1] packed-audio offsets in samples; the last one is the buffer's size
+  std::vector<int> ubase;            // [n_clips + 1] first unique frame of each clip in the flat frame list
+  int4* d_frames = nullptr;          // [U] (start, lo, hi, clip)
+  int* d_map = nullptr;              // per clip [K][F_i] -> clip-local unique frame id
+  avs::RaggedClip* d_clips = nullptr;
+  avs::MfccTables tab;
+};
+
+namespace avs {
+namespace {
+
+constexpr int kStatsSmemLimit = 227 * 1024;  // dynamic shared memory of one block on sm_100
+// mfcc_stats_kernel holds the DCT basis and the coefficients of every frame of one shifted signal: (128 + F) * NQ floats
+int max_frames_for(int n_mfcc) {
+  const int nq = n_mfcc <= 20 ? 20 : kMaxQ;
+  return kStatsSmemLimit / (nq * static_cast<int>(sizeof(float))) - kMels;
+}
+
+long long floor_div(long long a, long long b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
+
+int validate_ragged(int n_clips, const int32_t* lengths, int sample_rate, const int32_t* shifts, int n_shifts,
+                    int max_frames, int n_mfcc) {
+  AVS_REQUIRE(lengths != nullptr && shifts != nullptr, "null argument");
+  AVS_REQUIRE(n_clips > 0, "a ragged plan needs at least one clip");
+  AVS_REQUIRE(sample_rate > 0 && n_shifts > 0, "empty problem");
+  const int hop = std::max(1, sample_rate / 40);
+  long long map_total = 0;
+  for (int i = 0; i < n_clips; ++i) {
+    if (lengths[i] <= 0) {
+      set_error("ragged plan: clip %d has %d samples; every clip needs at least one", i, lengths[i]);
+      return AVS_EINVAL;
+    }
+    const int F = 1 + lengths[i] / hop;
+    if (max_frames > 0 && F > max_frames) {
+      set_error("ragged plan: clip %d has %d samples = %d STFT frames; at n_mfcc = %d the statistics kernel holds at most "
+                "%d frames (%d KB of shared memory)", i, lengths[i], F, n_mfcc, max_frames, kStatsSmemLimit / 1024);
+      return AVS_EINVAL;
+    }
+    map_total += static_cast<long long>(n_shifts) * F;
+  }
+  AVS_REQUIRE(map_total < (1LL << 31), "ragged plan: more than 2^31 (shift, frame) pairs in one batch");
+  return AVS_OK;
+}
+
+// Frames of one shift row that end inside the valid range, "stable" frames: the window [start, start + 2048) ends at or
+// before hi = n - max(0, s).  Their keys (start, max(start, lo), start + 2048), or the all-zero key, do not depend on the
+// length n, and a frame stable at length n is stable at every longer length: each key has a least length `need` from
+// which on some (shift, frame) of the row produces it.  Keys are numbered by ascending need, so a clip of length n has
+// exactly the first P(n) of them with the row's ids, and its map entries for stable frames are a copy of the row's map.
+// Only the frames that run past hi (about 2048 / hop per shift) are keyed per length.
+struct RowPlan {
+  const int32_t* shifts = nullptr;
+  int n_max = 0, jmax = 0, zero_id = -1;
+  std::vector<int4> keys;  // (start, lo, hi, need) by ascending need
+  std::vector<int> need;
+  std::vector<int> map;    // [K][jmax]: id of stable frame j of shift k (-1: not stable at n_max)
+};
+
+void build_row(RowPlan& r, int K, int hop) {
+  r.jmax = 1 + r.n_max / hop;
+  struct E { int start, a, b, need, slot; };
+  std::vector<E> es;
+  es.reserve(static_cast<size_t>(K) * r.jmax);
+  for (int k = 0; k < K; ++k) {
+    const long long s = r.shifts[k];
+    const long long lo = std::max<long long>(0, -s);
+    for (int j = 0; j < r.jmax; ++j) {
+      const long long start = static_cast<long long>(hop) * j - kHalf - s;
+      // stable at n  <=>  j < 1 + n / hop,  start + 2048 <= n - max(0, s),  |s| < n
+      const long long need = std::max({start + kNfft + std::max<long long>(0, s), std::llabs(s) + 1, static_cast<long long>(hop) * j});
+      if (need > r.n_max) continue;
+      const long long a = std::max(start, lo), b = start + kNfft;
+      if (a >= b) es.push_back(E{0, 0, 0, static_cast<int>(need), k * r.jmax + j});
+      else es.push_back(E{static_cast<int>(start), static_cast<int>(a), static_cast<int>(b), static_cast<int>(need), k * r.jmax + j});
+    }
+  }
+  auto key_less = [](const E& x, const E& y) { return std::tie(x.start, x.a, x.b) < std::tie(y.start, y.a, y.b); };
+  std::sort(es.begin(), es.end(), key_less);
+  std::vector<int4> uniq;  // (start, a, b, need = min over producers)
+  std::vector<int> group(es.size());
+  for (size_t i = 0; i < es.size(); ++i) {
+    if (i == 0 || key_less(es[i - 1], es[i])) uniq.push_back(make_int4(es[i].start, es[i].a, es[i].b, es[i].need));
+    else uniq.back().w = std::min(uniq.back().w, es[i].need);
+    group[i] = static_cast<int>(uniq.size()) - 1;
+  }
+  std::vector<int> order(uniq.size());
+  for (size_t i = 0; i < order.size(); ++i) order[i] = static_cast<int>(i);
+  std::sort(order.begin(), order.end(), [&](int x, int y) {
+    return std::tie(uniq[x].w, uniq[x].x, uniq[x].y, uniq[x].z) < std::tie(uniq[y].w, uniq[y].x, uniq[y].y, uniq[y].z);
+  });
+  std::vector<int> id(uniq.size());
+  r.keys.resize(uniq.size());
+  r.need.resize(uniq.size());
+  for (size_t i = 0; i < order.size(); ++i) {
+    id[order[i]] = static_cast<int>(i);
+    r.keys[i] = uniq[order[i]];
+    r.need[i] = uniq[order[i]].w;
+    if (r.keys[i].x == 0 && r.keys[i].y == 0 && r.keys[i].z == 0) r.zero_id = static_cast<int>(i);
+  }
+  r.map.assign(static_cast<size_t>(K) * r.jmax, -1);
+  for (size_t i = 0; i < es.size(); ++i) r.map[es[i].slot] = id[group[i]];
+}
+
+// Open-addressing table of one clip's end-touching keys; generation stamps spare the clearing between clips.
+struct TailKeys {
+  std::vector<int4> slot;  // (start, lo, hi, id)
+  std::vector<unsigned> stamp;
+  unsigned gen = 0;
+  size_t mask = 0;
+  void reset(size_t expect) {
+    size_t want = 64;
+    while (want < 2 * expect) want <<= 1;
+    if (slot.size() < want) {
+      slot.resize(want);
+      stamp.assign(want, 0u);
+      gen = 0;
+    }
+    mask = slot.size() - 1;
+    if (++gen == 0) {
+      std::fill(stamp.begin(), stamp.end(), 0u);
+      gen = 1;
+    }
+  }
+  // id of the key, or -1 after inserting it with id `next`
+  int find_or_insert(int start, int a, int b, int next) {
+    uint32_t h = static_cast<uint32_t>(start) * 0x9E3779B1u ^ static_cast<uint32_t>(a) * 0x85EBCA77u ^ static_cast<uint32_t>(b) * 0xC2B2AE3Du;
+    h ^= h >> 15;
+    for (size_t i = h & mask;; i = (i + 1) & mask) {
+      if (stamp[i] != gen) {
+        stamp[i] = gen;
+        slot[i] = make_int4(start, a, b, next);
+        return -1;
+      }
+      if (slot[i].x == start && slot[i].y == a && slot[i].z == b) return slot[i].w;
+    }
+  }
+};
+
+struct RaggedHostPlan {
+  std::vector<long long> audio_off;  // [n + 1]
+  std::vector<int> n_frames;         // [n]
+  std::vector<int> ubase;            // [n + 1]
+  std::vector<long long> mbase;      // [n + 1]
+  std::vector<int4> frames;          // flat (start, lo, hi, clip)
+  std::vector<int> map;              // flat, clip-local ids
+};
+
+// Host plan of a validated batch.  Rows are shared by the clips that have them (one per frame rate in practice); a clip
+// whose (length, row) pair came before copies that clip's frames and map.
+void build_ragged(int n_clips, const int32_t* lengths, int sample_rate, const int32_t* shifts, int K, RaggedHostPlan& h) {
+  const int hop = std::max(1, sample_rate / 40);
+  std::map<std::vector<int32_t>, int> row_ids;
+  std::vector<RowPlan> rows;
+  std::vector<int> row_of(n_clips);
+  std::vector<int32_t> key;
+  for (int i = 0; i < n_clips; ++i) {
+    key.assign(shifts + static_cast<size_t>(i) * K, shifts + static_cast<size_t>(i + 1) * K);
+    auto it = row_ids.find(key);
+    if (it == row_ids.end()) {
+      it = row_ids.emplace(key, static_cast<int>(rows.size())).first;
+      rows.emplace_back();
+      rows.back().shifts = shifts + static_cast<size_t>(i) * K;
+    }
+    row_of[i] = it->second;
+    rows[it->second].n_max = std::max(rows[it->second].n_max, lengths[i]);
+  }
+  for (RowPlan& r : rows) build_row(r, K, hop);
+
+  h.audio_off.resize(n_clips + 1);
+  h.n_frames.resize(n_clips);
+  h.ubase.resize(n_clips + 1);
+  h.mbase.resize(n_clips + 1);
+  h.audio_off[0] = 0;
+  h.mbase[0] = 0;
+  for (int i = 0; i < n_clips; ++i) {
+    h.audio_off[i + 1] = (h.audio_off[i] + lengths[i] + 3) & ~3LL;
+    h.n_frames[i] = 1 + lengths[i] / hop;
+    h.mbase[i + 1] = h.mbase[i] + static_cast<long long>(K) * h.n_frames[i];
+  }
+  h.map.resize(h.mbase[n_clips]);
+  h.frames.clear();
+  size_t reserve = 0;  // row keys plus the end-touching keys, at most 2048 / hop + 2 per shift
+  for (int i = 0; i < n_clips; ++i) reserve += rows[row_of[i]].keys.size() + static_cast<size_t>(K) * (kNfft / hop + 2);
+  h.frames.reserve(reserve);
+  std::unordered_map<uint64_t, int> seen;  // (row, length) -> first clip with it
+  TailKeys tail;
+  for (int i = 0; i < n_clips; ++i) {
+    const int n = lengths[i], F = h.n_frames[i];
+    const RowPlan& r = rows[row_of[i]];
+    int* map = h.map.data() + h.mbase[i];
+    h.ubase[i] = static_cast<int>(h.frames.size());
+    const auto prev = seen.emplace((static_cast<uint64_t>(row_of[i]) << 32) | static_cast<uint32_t>(n), i);
+    if (!prev.second) {
+      const int c = prev.first->second;
+      for (int u = h.ubase[c]; u < h.ubase[c + 1]; ++u) h.frames.push_back(make_int4(h.frames[u].x, h.frames[u].y, h.frames[u].z, i));
+      std::copy(h.map.begin() + h.mbase[c], h.map.begin() + h.mbase[c + 1], map);
+      continue;
+    }
+    const int P = static_cast<int>(std::upper_bound(r.need.begin(), r.need.end(), n) - r.need.begin());
+    h.frames.resize(h.ubase[i] + P);
+    int4* fr = h.frames.data() + h.ubase[i];
+    for (int u = 0; u < P; ++u) fr[u] = make_int4(r.keys[u].x, r.keys[u].y, r.keys[u].z, i);
+    int next = P;
+    int zero = r.zero_id >= 0 && r.zero_id < P ? r.zero_id : -1;
+    // frames of shift k: [0, jt) stable (copied from the row), [jt, F) touching the end
+    auto stable_count = [&](long long s, long long hi) {
+      if (s >= n || -s >= n) return 0;
+      return static_cast<int>(std::min<long long>(F, std::max<long long>(0, floor_div(hi - kHalf + s, hop) + 1)));
+    };
+    size_t n_tail = 0;
+    for (int k = 0; k < K; ++k) {
+      const long long s = r.shifts[k];
+      n_tail += F - stable_count(s, std::min<long long>(n, n - s));
+    }
+    tail.reset(n_tail);
+    for (int k = 0; k < K; ++k) {
+      const long long s = r.shifts[k];
+      // shift_audio (:100-114): y[n] = x[n - s] for n in [max(0,s), min(N, N+s)), zero elsewhere; |s| >= N -> all zeros
+      long long lo = std::max<long long>(0, -s), hi = std::min<long long>(n, n - s);
+      if (s >= n || -s >= n) lo = hi = 0;
+      const int jt = stable_count(s, hi);
+      std::copy(r.map.begin() + static_cast<size_t>(k) * r.jmax, r.map.begin() + static_cast<size_t>(k) * r.jmax + jt, map + static_cast<size_t>(k) * F);
+      for (int j = jt; j < F; ++j) {
+        const long long start = static_cast<long long>(hop) * j - kHalf - s;
+        const long long a = std::max(start, lo), b = std::min(start + kNfft, hi);
+        int id;
+        if (a >= b) {
+          if (zero < 0) {
+            zero = next++;
+            h.frames.push_back(make_int4(0, 0, 0, i));
+          }
+          id = zero;
+        } else {
+          id = tail.find_or_insert(static_cast<int>(start), static_cast<int>(a), static_cast<int>(b), next);
+          if (id < 0) {
+            id = next++;
+            h.frames.push_back(make_int4(static_cast<int>(start), static_cast<int>(a), static_cast<int>(b), i));
+          }
+        }
+        map[static_cast<size_t>(k) * F + j] = id;
+      }
+    }
+  }
+  h.ubase[n_clips] = static_cast<int>(h.frames.size());
+}
+
+}  // namespace
+}  // namespace avs
+
+extern "C" int avs_mfcc_ragged_plan_describe(int n_clips, const int32_t* lengths, int sample_rate,
+                                             const int32_t* shift_samples, int n_shifts, int64_t* audio_offsets,
+                                             int32_t* n_frames, int32_t* n_unique, int32_t* frames_out, int32_t* map_out) {
+  AVS_REQUIRE(audio_offsets && n_frames && n_unique, "null argument");
+  int rc;
+  if ((rc = validate_ragged(n_clips, lengths, sample_rate, shift_samples, n_shifts, 0, 0))) return rc;
+  RaggedHostPlan h;
+  build_ragged(n_clips, lengths, sample_rate, shift_samples, n_shifts, h);
+  for (int i = 0; i <= n_clips; ++i) audio_offsets[i] = h.audio_off[i];
+  for (int i = 0; i < n_clips; ++i) {
+    n_frames[i] = h.n_frames[i];
+    n_unique[i] = h.ubase[i + 1] - h.ubase[i];
+  }
+  if (frames_out)
+    for (size_t u = 0; u < h.frames.size(); ++u) {
+      frames_out[3 * u] = h.frames[u].x; frames_out[3 * u + 1] = h.frames[u].y; frames_out[3 * u + 2] = h.frames[u].z;
+    }
+  if (map_out) std::copy(h.map.begin(), h.map.end(), map_out);
+  return AVS_OK;
+}
+
+extern "C" int avs_mfcc_ragged_plan_create(int n_clips, const int32_t* lengths, int sample_rate, int n_mfcc,
+                                           const int32_t* shift_samples, int n_shifts, void* stream,
+                                           avs_mfcc_ragged_plan** out) {
+  AVS_REQUIRE(out != nullptr, "null argument");
+  AVS_REQUIRE(n_mfcc >= 1 && n_mfcc <= kMaxQ, "n_mfcc must be in [1, 40]");
+  int rc;
+  if ((rc = validate_ragged(n_clips, lengths, sample_rate, shift_samples, n_shifts, max_frames_for(n_mfcc), n_mfcc))) return rc;
+  RaggedHostPlan h;
+  build_ragged(n_clips, lengths, sample_rate, shift_samples, n_shifts, h);
+  avs_mfcc_ragged_plan* p = new avs_mfcc_ragged_plan();
+  p->n_clips = n_clips;
+  p->sr = sample_rate;
+  p->hop = std::max(1, sample_rate / 40);
+  p->n_mfcc = n_mfcc;
+  p->n_shifts = n_shifts;
+  p->max_frames = *std::max_element(h.n_frames.begin(), h.n_frames.end());
+  p->audio_off = h.audio_off;
+  p->ubase = h.ubase;
+  std::vector<RaggedClip> clips(n_clips);
+  for (int i = 0; i < n_clips; ++i)
+    clips[i] = RaggedClip{h.audio_off[i], h.ubase[i], static_cast<int>(h.mbase[i]), h.n_frames[i], 0};
+  HostTables tabs;
+  build_tables(sample_rate, n_mfcc, tabs);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if ((rc = upload_async(&p->d_frames, h.frames, st)) || (rc = upload_async(&p->d_map, h.map, st)) ||
+      (rc = upload_async(&p->d_clips, clips, st)) || (rc = upload_tables(p->tab, tabs, st, true))) {
+    avs_mfcc_ragged_plan_destroy(p);
+    return rc;
+  }
+  *out = p;
+  return AVS_OK;
+}
+
+extern "C" void avs_mfcc_ragged_plan_destroy(avs_mfcc_ragged_plan* p) {
+  if (!p) return;
+  // the buffers come from the stream-ordered allocator, which cudaFree does not wait for: kernels still queued may use them
+  cudaDeviceSynchronize();
+  cudaFree(p->d_frames); cudaFree(p->d_map); cudaFree(p->d_clips);
+  free_tables(p->tab);
+  delete p;
+}
+
+extern "C" int avs_mfcc_ragged_plan_audio_offsets(const avs_mfcc_ragged_plan* p, int64_t* audio_offsets) {
+  AVS_REQUIRE(p && audio_offsets, "null argument");
+  std::copy(p->audio_off.begin(), p->audio_off.end(), audio_offsets);
+  return AVS_OK;
+}
+
+extern "C" size_t avs_mfcc_ragged_workspace_bytes(const avs_mfcc_ragged_plan* p) {
+  return p ? mfcc_frame_ws_bytes(static_cast<size_t>(p->ubase[p->n_clips])) : 0;
+}
+
+size_t avs::mfcc_ragged_frames(const avs_mfcc_ragged_plan* p, int c0, int n) {
+  return static_cast<size_t>(p->ubase[c0 + n] - p->ubase[c0]);
+}
+void avs::mfcc_ragged_shape(const avs_mfcc_ragged_plan* p, int* n_clips, int* n_shifts, int* n_mfcc) {
+  *n_clips = p->n_clips;
+  *n_shifts = p->n_shifts;
+  *n_mfcc = p->n_mfcc;
+}
+
+namespace {
+int check_ragged_range(const avs_mfcc_ragged_plan* p, int c0, int n, size_t workspace_bytes) {
+  AVS_REQUIRE(c0 >= 0 && n >= 0 && c0 + n <= p->n_clips, "clip range outside the ragged plan");
+  const size_t need = mfcc_frame_ws_bytes(mfcc_ragged_frames(p, c0, n));
+  if (workspace_bytes < need) {
+    set_error("mfcc workspace too small: %zu < %zu", workspace_bytes, need);
+    return AVS_EWORKSPACE;
+  }
+  return AVS_OK;
+}
+}  // namespace
+
+int avs::mfcc_ragged_logmel_part(const avs_mfcc_ragged_plan* p, const float* audio, int c0, int n, void* workspace,
+                                 size_t workspace_bytes, void* stream) {
+  AVS_REQUIRE(p && audio && workspace, "null argument");
+  int rc;
+  if ((rc = check_ragged_range(p, c0, n, workspace_bytes))) return rc;
+  const int nu = static_cast<int>(mfcc_ragged_frames(p, c0, n));
+  if (nu == 0) return AVS_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const MfccWs w = carve_frame_ws(nu, workspace);
+  const int4* fr = p->d_frames + p->ubase[c0];
+  ProfScope ps(PROF_LOGMEL, st);
+  if (p->n_mfcc <= 20)
+    mfcc_logmel_warp_kernel<false, 20, true><<<nu, 32, 0, st>>>(audio, 0, fr, nu, p->tab.d_window, p->tab.d_tw, p->tab.d_tw2,
+                                                                p->tab.d_mel_tab, p->tab.d_mel_w, p->tab.d_dct_lane, w.logmel,
+                                                                w.frame_mfcc, w.frame_range, p->d_clips);
+  else
+    mfcc_logmel_warp_kernel<false, kMaxQ, true><<<nu, 32, 0, st>>>(audio, 0, fr, nu, p->tab.d_window, p->tab.d_tw, p->tab.d_tw2,
+                                                                   p->tab.d_mel_tab, p->tab.d_mel_w, p->tab.d_dct_lane, w.logmel,
+                                                                   w.frame_mfcc, w.frame_range, p->d_clips);
+  AVS_LAUNCHED();
+  return AVS_OK;
+}
+
+int avs::mfcc_ragged_stats_part(const avs_mfcc_ragged_plan* p, int c0, int n, float* out_stats, void* workspace,
+                                size_t workspace_bytes, void* stream) {
+  AVS_REQUIRE(p && out_stats && workspace, "null argument");
+  int rc;
+  if ((rc = check_ragged_range(p, c0, n, workspace_bytes))) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const MfccWs w = carve_frame_ws(mfcc_ragged_frames(p, c0, n), workspace);
+  const int nq = p->n_mfcc <= 20 ? 20 : kMaxQ;
+  const size_t sm = static_cast<size_t>(kMels + p->max_frames) * nq * sizeof(float);
+  if (nq == 20) AVS_CUDA(cudaFuncSetAttribute(mfcc_stats_kernel<20, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(sm)));
+  else AVS_CUDA(cudaFuncSetAttribute(mfcc_stats_kernel<kMaxQ, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(sm)));
+  for (int s0 = 0; s0 < n; s0 += 32768) {  // gridDim.y limit
+    const int nc = std::min(32768, n - s0);
+    float* os = out_stats + static_cast<size_t>(s0) * p->n_shifts * 2 * p->n_mfcc;
+    const RaggedClip* cl = p->d_clips + c0 + s0;
+    const dim3 g2(p->n_shifts, nc);
+    ProfScope ps2(PROF_MFCC_STATS, st);
+    if (nq == 20)
+      mfcc_stats_kernel<20, true><<<g2, 128, sm, st>>>(w.logmel, w.frame_mfcc, w.frame_range, p->d_map, p->ubase[c0], 0,
+                                                       p->n_shifts, p->n_mfcc, p->tab.d_dct, os, nullptr, cl);
+    else
+      mfcc_stats_kernel<kMaxQ, true><<<g2, 128, sm, st>>>(w.logmel, w.frame_mfcc, w.frame_range, p->d_map, p->ubase[c0], 0,
+                                                          p->n_shifts, p->n_mfcc, p->tab.d_dct, os, nullptr, cl);
+    AVS_LAUNCHED();
+  }
+  return AVS_OK;
+}
+
+extern "C" int avs_mfcc_ragged_stats_sweep(const avs_mfcc_ragged_plan* p, const float* audio, float* out_stats,
+                                           void* workspace, size_t workspace_bytes, void* stream) {
+  AVS_REQUIRE(p && audio && out_stats && workspace, "null argument");
+  int rc;
+  if ((rc = mfcc_ragged_logmel_part(p, audio, 0, p->n_clips, workspace, workspace_bytes, stream))) return rc;
+  return mfcc_ragged_stats_part(p, 0, p->n_clips, out_stats, workspace, workspace_bytes, stream);
 }

@@ -4,6 +4,7 @@
 
 struct avs_stcnn;
 struct avs_mfcc_plan;
+struct avs_mfcc_ragged_plan;
 namespace avs {
 
 // K1 (mfcc.cu): the whole thing, or its two kernels separately (log-mel / per-frame DCT tables of a clip range of the
@@ -14,6 +15,16 @@ int mfcc_logmel_part(const avs_mfcc_plan* p, const float* audio, int n_clips, in
                      size_t workspace_bytes, void* stream);
 int mfcc_stats_part(const avs_mfcc_plan* p, int n_clips, float* out_stats, float* out_mfcc, void* workspace,
                     size_t workspace_bytes, void* stream);
+size_t mfcc_frame_ws_bytes(size_t n_frames);  // workspace of the per-frame tables of n_frames unique frames
+// The same two halves for clips [c0, c0 + n) of a ragged plan: the log-mel tables of those clips' unique frames (a
+// contiguous range of the plan's flat frame list) go to the start of the workspace; out_stats is clip c0's row.
+int mfcc_ragged_logmel_part(const avs_mfcc_ragged_plan* p, const float* audio, int c0, int n, void* workspace,
+                            size_t workspace_bytes, void* stream);
+int mfcc_ragged_stats_part(const avs_mfcc_ragged_plan* p, int c0, int n, float* out_stats, void* workspace,
+                           size_t workspace_bytes, void* stream);
+// unique frames of clips [c0, c0 + n) of a ragged plan
+size_t mfcc_ragged_frames(const avs_mfcc_ragged_plan* p, int c0, int n);
+void mfcc_ragged_shape(const avs_mfcc_ragged_plan* p, int* n_clips, int* n_shifts, int* n_mfcc);
 
 // fp32 CUDA-core layer: in NCDHW f32, w OIDHW f32, out addressed as b*o_sb + c*o_sc + t*o_st + ho*Wo + wo
 int conv_pool_ffma(const float* in, const float* w, const float* bias, float* out, int B, int Cin, int Cout, int T,

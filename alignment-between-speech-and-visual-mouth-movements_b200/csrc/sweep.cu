@@ -24,6 +24,7 @@ struct avs_sweep {
   // device buffers (per chunk)
   void* ws_stcnn = nullptr; size_t ws_stcnn_bytes = 0;
   void* ws_mfcc = nullptr;  size_t ws_mfcc_bytes = 0;
+  void* ws_ragged = nullptr; size_t ws_ragged_bytes = 0;  // K1 tables of a chunk of a ragged plan, grown with cudaMallocAsync
   // per-call buffers, sized by the largest n_clips seen (cap), grown geometrically with cudaMallocAsync
   void* ws_score = nullptr; size_t ws_score_bytes = 0;
   float* vstats = nullptr;  // [cap, 13824]
@@ -102,7 +103,7 @@ extern "C" int avs_sweep_create(const avs_stcnn* net, const avs_mfcc_plan* plan,
 extern "C" void avs_sweep_destroy(avs_sweep* s) {
   if (!s) return;
   if (s->has_last) cudaEventSynchronize(s->ev_last);  // the handle's last call may still be running
-  cudaFree(s->ws_stcnn); cudaFree(s->ws_mfcc); cudaFree(s->ws_score); cudaFree(s->vstats); cudaFree(s->astats);
+  cudaFree(s->ws_stcnn); cudaFree(s->ws_mfcc); cudaFree(s->ws_ragged); cudaFree(s->ws_score); cudaFree(s->vstats); cudaFree(s->astats);
   cudaFree(s->d_scores_all); cudaFree(s->d_best_all);
   for (int i = 0; i < 2; ++i) {
     cudaFree(s->d_frames[i]); cudaFree(s->d_audio[i]);
@@ -157,10 +158,12 @@ static int ensure_capacity(avs_sweep* s, int n_clips, cudaStream_t st) {
 }
 
 // statistics of one chunk (n <= s->chunk clips starting at clip c0); audio branch on the side stream, joined back
-// into `st` before returning.
+// into `st` before returning.  With a ragged plan (rp) `audio` is the whole packed buffer and the chunk's K1 tables go to
+// ws_ragged.
 struct AudioBranch {
   avs_sweep* s; const float* audio; float* ast; int n, head;
   cudaStream_t st; bool stats_after_conv2;
+  const avs_mfcc_ragged_plan* rp; int c0;
 };
 // host hook of the STCNN, called when layer 2 has been enqueued (ev_fork recorded behind layer 1): enqueue the rest of K1
 // on the side stream — the log-mel tables of the clips the head start did not take, then the statistics of all clips
@@ -169,18 +172,22 @@ static int enqueue_audio_branch(void* arg) {
   avs_sweep* s = a->s;
   int rc;
   AVS_CUDA(cudaStreamWaitEvent(s->side, s->ev_fork, 0));
-  if ((rc = mfcc_logmel_part(s->plan, a->audio, a->n, a->head, a->n, s->ws_mfcc, s->ws_mfcc_bytes, s->side))) return rc;
+  if (a->rp) rc = mfcc_ragged_logmel_part(a->rp, a->audio, a->c0, a->n, s->ws_ragged, s->ws_ragged_bytes, s->side);
+  else rc = mfcc_logmel_part(s->plan, a->audio, a->n, a->head, a->n, s->ws_mfcc, s->ws_mfcc_bytes, s->side);
+  if (rc) return rc;
   AVS_CUDA(cudaEventRecord(s->ev_logmel, s->side));
   if (a->stats_after_conv2) {  // the statistics kernel runs beside conv3, not beside conv2's last items
     AVS_CUDA(cudaEventRecord(s->ev_conv2, a->st));
     AVS_CUDA(cudaStreamWaitEvent(s->side, s->ev_conv2, 0));
   }
-  rc = mfcc_stats_part(s->plan, a->n, a->ast, nullptr, s->ws_mfcc, s->ws_mfcc_bytes, s->side);
+  if (a->rp) rc = mfcc_ragged_stats_part(a->rp, a->c0, a->n, a->ast, s->ws_ragged, s->ws_ragged_bytes, s->side);
+  else rc = mfcc_stats_part(s->plan, a->n, a->ast, nullptr, s->ws_mfcc, s->ws_mfcc_bytes, s->side);
   AVS_CUDA(cudaEventRecord(s->ev_join, s->side));
   return rc;
 }
 
-static int run_chunk(avs_sweep* s, const void* frames, bool frames_u8, const float* audio, int c0, int n, cudaStream_t st) {
+static int run_chunk(avs_sweep* s, const void* frames, bool frames_u8, const float* audio, int c0, int n, cudaStream_t st,
+                     const avs_mfcc_ragged_plan* rp = nullptr) {
   int rc;
   float* vst = s->vstats + static_cast<size_t>(c0) * AVS_VSTATS;
   float* ast = s->astats + static_cast<size_t>(c0) * s->K * 2 * s->n_mfcc;
@@ -199,7 +206,7 @@ static int run_chunk(avs_sweep* s, const void* frames, bool frames_u8, const flo
 #else
   constexpr int stats_after_conv2 = kStatsAfterConv2;
 #endif
-  AudioBranch ab{s, audio, ast, n, head_div > 0 ? n / head_div : 0, st, stats_after_conv2 != 0};
+  AudioBranch ab{s, audio, ast, n, head_div > 0 && !rp ? n / head_div : 0, st, stats_after_conv2 != 0, rp, c0};
   StcnnHooks hooks;
   hooks.after_layer1 = s->ev_fork;
   hooks.on_layer1 = enqueue_audio_branch;
@@ -207,7 +214,7 @@ static int run_chunk(avs_sweep* s, const void* frames, bool frames_u8, const flo
   hooks.before_layer3 = s->ev_logmel;
 #ifdef AVS_EXPERIMENTS
   static const int audio_mode = env_knob("AVS_AUDIO_MODE", 0);  // 1 serial, 2 conv3 does not wait for the FFT kernel
-  if (audio_mode == 1) {
+  if (audio_mode == 1 && !rp) {
     if ((rc = stcnn_forward_impl(s->net, frames, frames_u8, n, s->chunk, true, StcnnHooks{}, nullptr, vst, nullptr, nullptr, s->ws_stcnn, s->ws_stcnn_bytes, st)))
       return rc;
     return avs_mfcc_stats_sweep(s->plan, audio, n, ast, s->ws_mfcc, s->ws_mfcc_bytes, st);
@@ -260,6 +267,54 @@ extern "C" int avs_sweep_run(avs_sweep* s, const float* frames, const float* aud
 extern "C" int avs_sweep_run_u8(avs_sweep* s, const uint8_t* frames, const float* audio, int n_clips, float* out_scores,
                                 int32_t* out_best, void* stream) {
   return sweep_run_device(s, frames, true, audio, n_clips, out_scores, out_best, stream);
+}
+
+// K1 workspace of a ragged plan: the largest chunk's unique frames.  Grown like ensure_capacity, stream-ordered on `st`
+// (which already waits for the handle's previous call).
+static int ensure_ragged_ws(avs_sweep* s, const avs_mfcc_ragged_plan* rp, int n_clips, cudaStream_t st) {
+  size_t most = 0;
+  for (int c0 = 0; c0 < n_clips; c0 += s->chunk) most = std::max(most, mfcc_ragged_frames(rp, c0, std::min(s->chunk, n_clips - c0)));
+  const size_t need = mfcc_frame_ws_bytes(most);
+  if (need <= s->ws_ragged_bytes) return AVS_OK;
+  const size_t bytes = std::max(need, s->ws_ragged_bytes + s->ws_ragged_bytes / 2);
+  if (s->ws_ragged) AVS_CUDA(cudaFreeAsync(s->ws_ragged, st));
+  s->ws_ragged = nullptr;
+  s->ws_ragged_bytes = 0;
+  AVS_CUDA(cudaMallocAsync(&s->ws_ragged, bytes, st));
+  s->ws_ragged_bytes = bytes;
+  return AVS_OK;
+}
+
+static int sweep_run_ragged(avs_sweep* s, const avs_mfcc_ragged_plan* rp, const void* frames, bool frames_u8,
+                            const float* audio, int n_clips, float* out_scores, int32_t* out_best, void* stream) {
+  AVS_REQUIRE(s && rp && frames && audio && out_scores && out_best, "null argument");
+  int rn, rk, rq;
+  mfcc_ragged_shape(rp, &rn, &rk, &rq);
+  AVS_REQUIRE(n_clips == rn, "n_clips differs from the ragged plan's");
+  AVS_REQUIRE(rk == s->K, "the ragged plan's shift count differs from the sweep's");
+  AVS_REQUIRE(rq == s->n_mfcc, "the ragged plan's n_mfcc differs from the sweep's");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int rc;
+  if ((rc = begin_call(s, st)) || (rc = ensure_capacity(s, n_clips, st)) || (rc = ensure_ragged_ws(s, rp, n_clips, st))) return rc;
+  const size_t fstride = kFrameElems * (frames_u8 ? 1 : sizeof(float));
+  for (int c0 = 0; c0 < n_clips; c0 += s->chunk) {
+    const int n = std::min(s->chunk, n_clips - c0);
+    if ((rc = run_chunk(s, static_cast<const uint8_t*>(frames) + c0 * fstride, frames_u8, audio, c0, n, st, rp))) break;
+  }
+  if (!rc) rc = score_all(s, n_clips, out_scores, out_best, st);
+  const int rc2 = end_call(s, st);
+  return rc ? rc : rc2;
+}
+
+extern "C" int avs_sweep_run_ragged(avs_sweep* s, const avs_mfcc_ragged_plan* plan, const float* frames,
+                                    const float* audio_packed, int n_clips, float* out_scores, int32_t* out_best,
+                                    void* stream) {
+  return sweep_run_ragged(s, plan, frames, false, audio_packed, n_clips, out_scores, out_best, stream);
+}
+extern "C" int avs_sweep_run_ragged_u8(avs_sweep* s, const avs_mfcc_ragged_plan* plan, const uint8_t* frames,
+                                       const float* audio_packed, int n_clips, float* out_scores, int32_t* out_best,
+                                       void* stream) {
+  return sweep_run_ragged(s, plan, frames, true, audio_packed, n_clips, out_scores, out_best, stream);
 }
 
 static bool is_pinned(const void* p) {

@@ -4,12 +4,14 @@ lines 79-250, 299-318) and the batched +-S sync sweep built from it.
 Kept names / signatures: ``DetectorConfig``, ``get_video_fps``, ``shift_audio``, ``compute_audio_stats``,
 ``extract_visual_embeddings``, ``FeatureExtractor`` (``build_feature``), ``MisalignmentDetector``,
 ``load_lipnet``, ``save_detector``, ``load_detector``.  New batched entry points: ``SyncSweeper`` /
-``sync_sweep`` (all clips x all shifts in three kernels, SURVEY.md section 3.2).
+``sync_sweep`` (all clips x all shifts in three kernels, SURVEY.md section 3.2), with ``SyncSweeper.run_ragged`` and
+``audio_stats_sweep_ragged`` for batches whose clips differ in audio length and frame rate.
 All arithmetic runs in libavsync_b200 (K1, K2, K4); there is no CPU fallback.
 """
 from __future__ import annotations
 
 import ctypes
+from collections import OrderedDict
 from dataclasses import dataclass
 from typing import Dict, Optional, Sequence, Tuple
 
@@ -120,6 +122,90 @@ def audio_stats_sweep(audio: torch.Tensor, shifts_samples: Sequence[int], sample
     return out
 
 
+class _MfccRaggedPlan:
+    """K1 plan of a batch of clips with their own lengths and shift rows (include/avsync.h: avs_mfcc_ragged_plan)."""
+
+    def __init__(self, lengths: Sequence[int], sample_rate: int, n_mfcc: int, rows: np.ndarray):
+        B, K = rows.shape
+        ln = np.ascontiguousarray(lengths, dtype=np.int32)
+        rows = np.ascontiguousarray(rows, dtype=np.int32)
+        i32 = ctypes.POINTER(ctypes.c_int32)
+        L = N.lib()
+        h = N.c_void_p()
+        self.stream = torch.cuda.current_stream()          # the plan's upload is queued here
+        N.check(L.avs_mfcc_ragged_plan_create(B, ln.ctypes.data_as(i32), int(sample_rate), int(n_mfcc),
+                                              rows.ctypes.data_as(i32), K, N.stream_ptr(), ctypes.byref(h)),
+                "mfcc_ragged_plan_create")
+        self.handle = N.Handle(h, L.avs_mfcc_ragged_plan_destroy)
+        off = (ctypes.c_int64 * (B + 1))()
+        N.check(L.avs_mfcc_ragged_plan_audio_offsets(h, off), "mfcc_ragged_plan_audio_offsets")
+        self.offsets = list(off)
+        self.n_clips, self.n_shifts, self.n_mfcc = B, K, n_mfcc
+
+    def pack(self, audio: Sequence[torch.Tensor]) -> torch.Tensor:
+        """The clips' audio in one buffer at the plan's offsets (one device copy; the gaps are never read)."""
+        torch.cuda.current_stream().wait_stream(self.stream)
+        pad = torch.zeros(3, dtype=torch.float32, device=audio[0].device)
+        pieces = []
+        for i, a in enumerate(audio):
+            pieces.append(a)
+            gap = self.offsets[i + 1] - self.offsets[i] - a.numel()
+            if gap:
+                pieces.append(pad[:gap])
+        return torch.cat(pieces)
+
+
+_ragged_plan_cache: "OrderedDict[tuple, _MfccRaggedPlan]" = OrderedDict()
+
+
+def mfcc_ragged_plan(lengths: Sequence[int], sample_rate: int, n_mfcc: int, rows: np.ndarray) -> _MfccRaggedPlan:
+    """Ragged K1 plan, from a cache of the few most recent ones (a training loop repeats its batches every epoch)."""
+    N.device_check()
+    rows = np.ascontiguousarray(rows, dtype=np.int32)
+    key = (torch.cuda.current_device(), tuple(int(n) for n in lengths), int(sample_rate), int(n_mfcc), rows.shape,
+           rows.tobytes())
+    p = _ragged_plan_cache.get(key)
+    if p is None:
+        p = _MfccRaggedPlan(lengths, sample_rate, n_mfcc, rows)
+        _ragged_plan_cache[key] = p
+        while len(_ragged_plan_cache) > 4:
+            _ragged_plan_cache.popitem(last=False)
+    else:
+        _ragged_plan_cache.move_to_end(key)
+    return p
+
+
+def _ragged_audio(audio: Sequence[torch.Tensor], n_clips: int):
+    if len(audio) != n_clips:
+        raise RuntimeError(f"expected {n_clips} audio tensors, got {len(audio)}")
+    out = []
+    for i, a in enumerate(audio):
+        N.require_cuda(a, f"audio[{i}]")
+        if a.dim() != 1 or a.numel() == 0:
+            raise RuntimeError(f"audio[{i}] must be a non-empty 1-D tensor, got shape {tuple(a.shape)}")
+        out.append(N.f32c(a))
+    return out
+
+
+def audio_stats_sweep_ragged(audio: Sequence[torch.Tensor], shifts_samples, sample_rate: int = 16000,
+                             n_mfcc: int = 20) -> torch.Tensor:
+    """K1 over clips of different lengths: ``audio`` is a list of B 1-D CUDA f32 tensors, ``shifts_samples`` one row of K
+    integer sample delays per clip (``shift_samples(k, fps_i, sample_rate)``).  Returns [B, K, 2*n_mfcc]; row i is
+    bit for bit ``audio_stats_sweep(audio[i][None], shifts_samples[i])[0]``."""
+    rows = np.asarray(shifts_samples, dtype=np.int64)
+    if rows.ndim != 2 or rows.shape[0] != len(audio):
+        raise RuntimeError(f"shifts_samples must have one row per clip ({len(audio)}), got shape {rows.shape}")
+    audio = _ragged_audio(audio, rows.shape[0])
+    plan = mfcc_ragged_plan([a.numel() for a in audio], sample_rate, n_mfcc, rows)
+    packed = plan.pack(audio)
+    L = N.lib()
+    out = torch.empty((plan.n_clips, plan.n_shifts, 2 * n_mfcc), dtype=torch.float32, device=packed.device)
+    ws = N.workspace(L.avs_mfcc_ragged_workspace_bytes(plan.handle.h), packed.device)
+    N.check(L.avs_mfcc_ragged_stats_sweep(plan.handle.h, N.ptr(packed), N.ptr(out), N.ptr(ws), ws.numel(),
+                                          N.stream_ptr()), "mfcc_ragged_stats_sweep")
+    return out
+
+
 def compute_audio_stats(audio: np.ndarray, sample_rate: int, n_mfcc: int) -> torch.Tensor:
     """Reference contract (:117-127): 1-D float audio -> CPU tensor [2*n_mfcc] = cat(mean, std)
     of ``librosa.feature.mfcc(y, sr, n_mfcc, hop_length=sr//40)`` over frames."""
@@ -220,7 +306,8 @@ class SyncSweeper:
     """All clips x all shifts of the +-``max_shift_frames`` sweep in one pipeline (K2 | K1 -> K4).
 
     ``run(frames, audio)`` takes device tensors; ``run_host(frames, audio)`` takes host arrays and
-    pipelines the H2D/D2H copies against compute chunk by chunk.  Both return
+    pipelines the H2D/D2H copies against compute chunk by chunk; ``run_ragged(frames, audio, fps)`` takes one audio
+    tensor per clip, each of its own length and frame rate.  All return
     ``(scores [B, 2S+1], best_shift_frames [B])`` where ``best_shift_frames = argmax_k - S``.
     ``frames`` is the reference's f32 tensor ``[B,1,75,50,100]`` or the uint8 pixels it is made from
     (``float32(u8 / 255.0)``, dataset.py:226-231): same scores bit for bit, a quarter of the bytes.
@@ -234,6 +321,7 @@ class SyncSweeper:
         self.shift_frames = list(range(-self.S, self.S + 1))
         self.shifts = [shift_samples(k, fps, sample_rate) for k in self.shift_frames]
         self.n_samples, self.n_mfcc = n_samples, n_mfcc
+        self.fps, self.sample_rate = fps, sample_rate
         self.lipnet, self.detector = lipnet, detector
         self.plan = mfcc_plan(n_samples, sample_rate, n_mfcc, self.shifts)
         self.net = lipnet._stcnn()
@@ -262,6 +350,33 @@ class SyncSweeper:
         best = torch.empty((B,), dtype=torch.int32, device=frames.device)
         fn = N.lib().avs_sweep_run_u8 if frames.dtype == torch.uint8 else N.lib().avs_sweep_run
         N.check(fn(self.handle.h, N.ptr(frames), N.ptr(audio), B, N.ptr(scores), N.ptr(best), N.stream_ptr()), "sweep_run")
+        return scores, best - self.S
+
+    def run_ragged(self, frames: torch.Tensor, audio: Sequence[torch.Tensor], fps=None):
+        """Clips whose audio differs in length and frame rate: ``audio`` is a list of B 1-D CUDA f32 tensors at the
+        sweeper's sample rate, ``fps`` one frame rate for all clips or one per clip (default: the sweeper's).  Every clip
+        is scored at its own length and with its own shifts, bit for bit as a one-clip ``SyncSweeper(n_samples=len_i,
+        fps=fps_i).run`` would; same outputs as ``run``."""
+        N.require_cuda(frames, "frames")
+        frames = self.lipnet._check_frames(frames)
+        B = frames.shape[0]
+        audio = _ragged_audio(audio, B)
+        if fps is None:
+            fps = self.fps
+        fps = [float(fps)] * B if np.isscalar(fps) else [float(f) for f in fps]
+        if len(fps) != B:
+            raise RuntimeError(f"expected one frame rate per clip ({B}), got {len(fps)}")
+        scores = torch.empty((B, self.K), dtype=torch.float32, device=frames.device)
+        best = torch.empty((B,), dtype=torch.int32, device=frames.device)
+        if B == 0:
+            return scores, best
+        row_of = {f: [shift_samples(k, f, self.sample_rate) for k in self.shift_frames] for f in set(fps)}
+        plan = mfcc_ragged_plan([a.numel() for a in audio], self.sample_rate, self.n_mfcc,
+                                np.array([row_of[f] for f in fps], dtype=np.int32))
+        packed = plan.pack(audio)
+        fn = N.lib().avs_sweep_run_ragged_u8 if frames.dtype == torch.uint8 else N.lib().avs_sweep_run_ragged
+        N.check(fn(self.handle.h, plan.handle.h, N.ptr(frames), N.ptr(packed), B, N.ptr(scores), N.ptr(best),
+                   N.stream_ptr()), "sweep_run_ragged")
         return scores, best - self.S
 
     def run_host(self, frames: np.ndarray, audio: np.ndarray):
@@ -346,12 +461,15 @@ class FeatureExtractor:
         if video_path in self.visual_cache:
             return self.visual_cache[video_path], self.fps_cache[video_path]
         frames = self.grid.process_video(video_path)
-        getter = getattr(self.grid, "get_video_fps", None)     # a dataset may know better (synthetic clips)
-        fps = (getter(video_path) if getter is not None else None) or get_video_fps(video_path, self.cfg.default_fps)
+        fps = self._video_fps(video_path)
         stats = visual_stats(self.lipnet, frames.unsqueeze(0).to(self.device))[0].cpu()
         self.visual_cache[video_path] = stats
         self.fps_cache[video_path] = fps
         return stats, fps
+
+    def _video_fps(self, video_path: str) -> float:
+        getter = getattr(self.grid, "get_video_fps", None)     # a dataset may know better (synthetic clips)
+        return (getter(video_path) if getter is not None else None) or get_video_fps(video_path, self.cfg.default_fps)
 
     def _load_audio(self, video_path: str) -> Tuple[np.ndarray, int]:
         if video_path in self.audio_cache:
@@ -407,6 +525,26 @@ class FeatureExtractor:
         shifts = [shift_samples(k, fps, sr) for k in range(-max_shift_frames, max_shift_frames + 1)]
         ast = audio_stats_sweep(a, shifts, sr, self.cfg.n_mfcc)[0].cpu()
         return torch.cat([visual_stats_.unsqueeze(0).expand(len(shifts), -1), ast], dim=1)
+
+    def build_features_sweep_batch(self, paths: Sequence[str], max_shift_frames: int) -> torch.Tensor:
+        """``build_features_sweep`` of many clips at once: [n, 2S+1, 13864], the same bits as stacking the per-clip
+        calls.  The visual statistics of the clips not yet cached come from one STCNN call, the audio statistics of all
+        clips, each at its own length and frame rate, from one ragged K1 launch; the same caches are filled."""
+        S, sr = int(max_shift_frames), self.cfg.sample_rate
+        todo = [p for p in dict.fromkeys(paths) if p not in self.visual_cache]
+        if todo:
+            frames = torch.stack([self.grid.process_video(p) for p in todo]).to(self.device)
+            vst = visual_stats(self.lipnet, frames).cpu()
+            for i, p in enumerate(todo):
+                self.visual_cache[p] = vst[i].clone()
+                self.fps_cache[p] = self._video_fps(p)
+        if not paths:
+            return torch.empty((0, 2 * S + 1, 2 * self.lipnet.conv_output_dim + 2 * self.cfg.n_mfcc))
+        audio = [self._audio_on_device(p)[0] for p in paths]
+        rows = [[shift_samples(k, self.fps_cache[p], sr) for k in range(-S, S + 1)] for p in paths]
+        ast = audio_stats_sweep_ragged(audio, rows, sr, self.cfg.n_mfcc).cpu()
+        return torch.stack([torch.cat([self.visual_cache[p].unsqueeze(0).expand(2 * S + 1, -1), ast[i]], dim=1)
+                            for i, p in enumerate(paths)])
 
 
 # ---------------------------------------------------------------------------------- dataset / epoch

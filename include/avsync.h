@@ -95,6 +95,32 @@ AVS_API int avs_mfcc_sweep_debug(const avs_mfcc_plan* plan, const float* audio, 
                          float* out_stats, float* out_mfcc, void* workspace, size_t workspace_bytes,
                          void* stream);
 
+/* Ragged K1: a batch of n_clips clips, clip i with lengths[i] samples and its own row of n_shifts signed delays
+ * shift_samples[i][k] (the row follows from the clip's frame rate), one sample_rate and n_mfcc.  Clip i's statistics
+ * are those of a uniform plan of that clip alone, bit for bit.  The clips' audio is packed into one device buffer:
+ * clip i starts at audio_offsets[i] (a multiple of 4 samples); the bytes between clips are never read, and
+ * audio_offsets[n_clips] is the buffer's length.  n_mfcc in [1, 40]; a clip may have at most 2777 STFT frames
+ * (n_mfcc <= 20; 1324 for n_mfcc up to 40: about 69 s / 33 s at 16 kHz), the statistics kernel's shared-memory limit.
+ * All arguments are checked before any CUDA call.  Creation copies the plan to the device with stream-ordered
+ * allocations and copies on `stream` that wait for no other work; destroy waits for the device. */
+typedef struct avs_mfcc_ragged_plan avs_mfcc_ragged_plan;
+AVS_API int avs_mfcc_ragged_plan_create(int n_clips, const int32_t* lengths, int sample_rate, int n_mfcc,
+                                const int32_t* shift_samples, int n_shifts, void* stream,
+                                avs_mfcc_ragged_plan** out);
+AVS_API void avs_mfcc_ragged_plan_destroy(avs_mfcc_ragged_plan* plan);
+/* Host-only (no device needed): audio_offsets [n_clips+1], n_frames / n_unique [n_clips] per clip; frames_out (may be
+ * NULL) receives sum(n_unique) triples (start, lo, hi), clip after clip, and map_out (may be NULL) the clips'
+ * [n_shifts][n_frames[i]] -> clip-local unique-frame-id tables one after the other.  The same per clip as
+ * avs_mfcc_plan_describe for that clip alone, up to the numbering of its unique frames. */
+AVS_API int avs_mfcc_ragged_plan_describe(int n_clips, const int32_t* lengths, int sample_rate,
+                                  const int32_t* shift_samples, int n_shifts, int64_t* audio_offsets,
+                                  int32_t* n_frames, int32_t* n_unique, int32_t* frames_out, int32_t* map_out);
+AVS_API int avs_mfcc_ragged_plan_audio_offsets(const avs_mfcc_ragged_plan* plan, int64_t* audio_offsets);
+AVS_API size_t avs_mfcc_ragged_workspace_bytes(const avs_mfcc_ragged_plan* plan);
+/* audio: device f32, packed at the plan's offsets; out_stats: device f32 [n_clips, n_shifts, 2*n_mfcc]. */
+AVS_API int avs_mfcc_ragged_stats_sweep(const avs_mfcc_ragged_plan* plan, const float* audio, float* out_stats,
+                                void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------- K2: STCNN
  * Replaces extract_visual_embeddings (misalignment_detection_train.py:130-144) == the
  * conv half of LipNet.forward (model.py:67-82), eval mode, plus the visual statistics of
@@ -189,6 +215,16 @@ AVS_API int avs_sweep_run_u8(avs_sweep* sw, const uint8_t* frames, const float* 
                      float* out_scores, int32_t* out_best, void* stream);
 AVS_API int avs_sweep_run_host_u8(avs_sweep* sw, const uint8_t* frames_host, const float* audio_host,
                           int n_clips, float* out_scores_host, int32_t* out_best_host);
+/* Clips of different audio lengths and frame rates: the audio statistics come from a ragged plan (n_clips must be the
+ * plan's, its n_shifts and n_mfcc the handle's) instead of the handle's uniform plan; audio_packed is laid out at the
+ * plan's offsets.  Frames, outputs, chunking and ordering as avs_sweep_run; each clip's scores equal a one-clip sweep
+ * over a uniform plan of its own length and shifts, bit for bit. */
+AVS_API int avs_sweep_run_ragged(avs_sweep* sw, const avs_mfcc_ragged_plan* plan, const float* frames,
+                         const float* audio_packed, int n_clips, float* out_scores, int32_t* out_best,
+                         void* stream);
+AVS_API int avs_sweep_run_ragged_u8(avs_sweep* sw, const avs_mfcc_ragged_plan* plan, const uint8_t* frames,
+                            const float* audio_packed, int n_clips, float* out_scores, int32_t* out_best,
+                            void* stream);
 /* ---------------------------------------------------------------- decode metrics (SURVEY 8f-3)
  * Edit distances behind calculate_cer / calculate_wer (train.py:945-993) and the positional character
  * matches of evaluate_model (utils.py:83-86) for a batch of id sequences that are already on the device
