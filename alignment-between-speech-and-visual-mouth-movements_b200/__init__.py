@@ -8,7 +8,8 @@ error behaviour) over the C-ABI library ``libavsync_b200.so`` (``include/avsync.
     misalignment_detection_train.{DetectorConfig, shift_audio, compute_audio_stats,
         extract_visual_embeddings, FeatureExtractor, MisalignmentDataset, MisalignmentDetector, run_epoch,
         load_lipnet, save_detector}                  utils.evaluate_model
-    misalignment_detection_train.{SyncSweeper, sync_sweep, audio_stats_sweep_ragged}, utils.ctc_greedy_decode   (new, batched)
+    misalignment_detection_train.{SyncSweeper, sync_sweep, audio_stats_sweep_ragged, audio_stats_sweep_windows,
+        window_bounds}, utils.ctc_greedy_decode   (new, batched)
     distributed.{shard_range, sweep_sharded, gather_scores, ddp_detector_step, GraphedDetectorStep}        (new, multi-GPU)
 
 Import as ``avsync_b200`` (the directory name is not a valid identifier; ``avsync_b200.py`` at the
@@ -19,7 +20,8 @@ from .model import LipNet
 from .utils import ctc_greedy_decode, decode_batch, decode_metrics, decode_prediction, evaluate_model
 from .misalignment_detection_train import (DetectorConfig, FeatureExtractor, MisalignmentDataset, MisalignmentDetector,
                                            SyncSweeper, run_epoch,
-                                           audio_stats_sweep, audio_stats_sweep_ragged, compute_audio_stats, extract_visual_embeddings,
+                                           audio_stats_sweep, audio_stats_sweep_ragged, audio_stats_sweep_windows, compute_audio_stats,
+                                           extract_visual_embeddings, window_bounds,
                                            load_detector, load_lipnet, save_detector, shift_audio, shift_samples, get_video_fps,
                                            resample_audio, default_audio_loader,
                                            sweep_score, sync_sweep, visual_stats)
@@ -27,6 +29,6 @@ from .dataset import GridPreprocessor
 from . import distributed
 
 __all__ = ["LipNet", "ctc_greedy_decode", "decode_batch", "decode_prediction", "DetectorConfig", "FeatureExtractor",
-           "MisalignmentDataset", "MisalignmentDetector", "SyncSweeper", "run_epoch", "evaluate_model", "decode_metrics", "audio_stats_sweep", "audio_stats_sweep_ragged", "compute_audio_stats",
+           "MisalignmentDataset", "MisalignmentDetector", "SyncSweeper", "run_epoch", "evaluate_model", "decode_metrics", "audio_stats_sweep", "audio_stats_sweep_ragged", "audio_stats_sweep_windows", "window_bounds", "compute_audio_stats",
            "extract_visual_embeddings", "load_detector", "load_lipnet", "save_detector", "shift_audio",
            "shift_samples", "get_video_fps", "resample_audio", "default_audio_loader", "sweep_score", "sync_sweep", "visual_stats", "GridPreprocessor", "distributed"]

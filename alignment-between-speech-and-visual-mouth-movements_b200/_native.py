@@ -49,6 +49,11 @@ SIGNATURES = {
     "avs_mfcc_ragged_plan_audio_offsets": (c_int, [_P, POINTER(ctypes.c_int64)]),
     "avs_mfcc_ragged_workspace_bytes": (c_size_t, [_P]),
     "avs_mfcc_ragged_stats_sweep": (c_int, [_P, _P, _P, _P, c_size_t, _P]),
+    "avs_mfcc_ragged_plan_create_windows": (c_int, [c_int, ctypes.c_int64, POINTER(ctypes.c_int64), POINTER(c_int32), c_int, c_int,
+                                                    c_int, POINTER(c_int32), c_int, _P, POINTER(_P)]),
+    "avs_mfcc_ragged_plan_describe_windows": (c_int, [c_int, ctypes.c_int64, POINTER(ctypes.c_int64), POINTER(c_int32), c_int,
+                                                      c_int, POINTER(c_int32), c_int, POINTER(c_int32), POINTER(c_int32),
+                                                      POINTER(c_int32), POINTER(c_int32)]),
     "avs_stcnn_create": (c_int, [_P, _P, _P, _P, _P, _P, c_int, _P, POINTER(_P)]),
     "avs_stcnn_destroy": (None, [_P]),
     "avs_stcnn_workspace_bytes": (c_size_t, [_P, c_int]),
@@ -81,6 +86,8 @@ SIGNATURES = {
     "avs_sweep_run_host_u8": (c_int, [_P, _P, _P, c_int, _P, _P]),
     "avs_sweep_run_ragged": (c_int, [_P, _P, _P, _P, c_int, _P, _P, _P]),
     "avs_sweep_run_ragged_u8": (c_int, [_P, _P, _P, _P, c_int, _P, _P, _P]),
+    "avs_sweep_run_windows": (c_int, [_P, _P, _P, c_int, _P, c_int, _P, _P, _P]),
+    "avs_sweep_run_windows_u8": (c_int, [_P, _P, _P, c_int, _P, c_int, _P, _P, _P]),
 }
 # tools build only (make EXPERIMENTS=1 -> libavsync_b200_exp.so, loaded by tools/ through use_experiments_build())
 EXPERIMENT_SIGNATURES = {

@@ -2,7 +2,8 @@
 // + bias + ReLU + MaxPool3d((1,2,2)) fused (model.py:67-76).  This is the bring-up / cross-check
 // path and the fp32-exact arithmetic mode; the throughput path is conv_umma.cu.
 //
-// One CTA computes, for one (clip, t), a 16 x 16 tile of POOLED outputs (32 x 32 conv outputs) for
+// Input clip b starts at in + b * i_sb (the layer-1 input of overlapping windows of one recording sits in the recording's
+// own buffer, i_sb = stride * H * W).  One CTA computes, for one (clip, t), a 16 x 16 tile of POOLED outputs (32 x 32 conv outputs) for
 // CO_T = 8 output channels: each thread owns one pooled position = a 2 x 2 conv quad x 8 channels.
 // Input patches (3 time planes x (32 + KH - 1) x (32 + KW - 1)) and the weights of the current input
 // channel are staged in shared memory.
@@ -14,7 +15,7 @@ template <int KH, int KW>
 __global__ void __launch_bounds__(256)
 conv_pool_ffma_kernel(const float* __restrict__ in, const float* __restrict__ wgt, const float* __restrict__ bias,
                       float* __restrict__ out, int Cin, int Cout, int T, int H, int W,
-                      long long o_sb, long long o_sc, long long o_st) {
+                      long long i_sb, long long o_sb, long long o_sc, long long o_st) {
   constexpr int CO_T = 8, PT = 16, CT = 32;
   constexpr int PH = CT + KH - 1, PW = CT + KW - 1, PWP = PW + 1;
   constexpr int PADH = KH / 2, PADW = KW / 2;
@@ -43,7 +44,7 @@ conv_pool_ffma_kernel(const float* __restrict__ in, const float* __restrict__ wg
       const int tt = t + kd - 1, hh = h0 + r - PADH, ww = w0 + c - PADW;
       float v = 0.f;
       if (tt >= 0 && tt < T && hh >= 0 && hh < H && ww >= 0 && ww < W)
-        v = in[(((static_cast<size_t>(b) * Cin + ci) * T + tt) * H + hh) * W + ww];
+        v = in[b * i_sb + ((static_cast<long long>(ci) * T + tt) * H + hh) * W + ww];
       s_in[kd][r][c] = v;
     }
     for (int i = tid; i < 3 * KH * KW * CO_T; i += 256) {
@@ -88,15 +89,15 @@ conv_pool_ffma_kernel(const float* __restrict__ in, const float* __restrict__ wg
 }
 
 int conv_pool_ffma(const float* in, const float* w, const float* bias, float* out, int B, int Cin, int Cout, int T,
-                   int H, int W, int KH, int KW, long long o_sb, long long o_sc, long long o_st, cudaStream_t st) {
+                   int H, int W, int KH, int KW, long long i_sb, long long o_sb, long long o_sc, long long o_st, cudaStream_t st) {
   const int Ho = H / 2, Wo = W / 2;
   dim3 grid(cdiv(Ho, 16) * cdiv(Wo, 16), B * T, cdiv(Cout, 8));
   ProfScope ps(Cin == 1 ? PROF_CONV1 : (Cout == 64 ? PROF_CONV2 : PROF_CONV3), st);
   AVS_REQUIRE(static_cast<long long>(B) * T <= 65535, "FFMA conv path: n_clips * T must be <= 65535 per call");
   if (KH == 5 && KW == 5)
-    conv_pool_ffma_kernel<5, 5><<<grid, 256, 0, st>>>(in, w, bias, out, Cin, Cout, T, H, W, o_sb, o_sc, o_st);
+    conv_pool_ffma_kernel<5, 5><<<grid, 256, 0, st>>>(in, w, bias, out, Cin, Cout, T, H, W, i_sb, o_sb, o_sc, o_st);
   else if (KH == 3 && KW == 3)
-    conv_pool_ffma_kernel<3, 3><<<grid, 256, 0, st>>>(in, w, bias, out, Cin, Cout, T, H, W, o_sb, o_sc, o_st);
+    conv_pool_ffma_kernel<3, 3><<<grid, 256, 0, st>>>(in, w, bias, out, Cin, Cout, T, H, W, i_sb, o_sb, o_sc, o_st);
   else {
     set_error("unsupported kernel size %dx%d", KH, KW);
     return AVS_EINVAL;

@@ -955,7 +955,8 @@ static void kind_traits_for(int kind, int* NT, int* acc, int* spu, int* pairs, i
 
 // ------------------------------------------------------------------------------------------------ layout kernels
 // frames [B,1,T,H,W] (f32 as the reference passes them, or the u8 pixels they were made from: dataset.py:226-231,
-// value = float32(u8 / 255.0)) -> layer-1 input: X8 layout, position p holds the 8 consecutive padded-row values
+// value = float32(u8 / 255.0); clip b starts pitch * H * W values after clip b - 1: pitch = T for a batch of clips, the
+// window stride for overlapping windows of one recording) -> layer-1 input: X8 layout, position p holds the 8 consecutive padded-row values
 // val(p) .. val(p+7) (so the kw taps are the K index of the MMA).  One CTA per (clip, tp, parity): the
 // flattened padded parity array is staged in shared memory as bf16 (hi and lo residual) with coalesced
 // row loads, then every thread emits 16-byte X8 entries for consecutive positions.  The u8 variant converts through
@@ -963,7 +964,8 @@ static void kind_traits_for(int kind, int* NT, int* acc, int* spu, int* pairs, i
 // for frames that came from 8-bit pixels.
 template <typename TIn>
 __global__ void __launch_bounds__(256)
-pack_frames_kernel(const TIn* __restrict__ frames, __nv_bfloat16* __restrict__ act, int PP, int split, int T, int n_items) {
+pack_frames_kernel(const TIn* __restrict__ frames, __nv_bfloat16* __restrict__ act, int PP, int split, int T, int n_items,
+                   int pitch) {
   extern __shared__ __align__(16) uint16_t s_val[];  // [2][NV]: hi, lo (NV = PP + 8 rounded up to 8 values)
   __shared__ uint32_t s_lut[256];                    // u8 variant: bf16 hi | bf16 lo << 16 of float32(v / 255.0)
   constexpr bool kU8 = sizeof(TIn) == 1;
@@ -989,7 +991,7 @@ pack_frames_kernel(const TIn* __restrict__ frames, __nv_bfloat16* __restrict__ a
     if (tp >= 1 && tp <= T) {
       // a work unit is four consecutive pixels of one row (the row pitch, the padding and 4-pixel groups are all even,
       // so a group is two aligned 32-bit stores of bf16 pairs)
-      const TIn* f = frames + (b * T + (tp - 1)) * static_cast<long long>(H * W);
+      const TIn* f = frames + (b * pitch + (tp - 1)) * static_cast<long long>(H * W);
       for (int i = threadIdx.x; i < HH * QW; i += 256) {
         const int row = i / QW, wq = (i - row * QW) * 4;
         const int h = 2 * row + par - PH;
@@ -1042,7 +1044,7 @@ pack_frames_kernel(const TIn* __restrict__ frames, __nv_bfloat16* __restrict__ a
 // padded parity rows go to shared memory as bf16, then every thread emits 16-byte entries.
 template <typename TIn>
 __global__ void __launch_bounds__(256)
-pack_frames_pooled_kernel(const TIn* __restrict__ frames, __nv_bfloat16* __restrict__ act, int PP, int T, int n_items) {
+pack_frames_pooled_kernel(const TIn* __restrict__ frames, __nv_bfloat16* __restrict__ act, int PP, int T, int n_items, int pitch) {
   constexpr bool kU8 = sizeof(TIn) == 1;
   using K1 = LayerKind<KIND_L1>;
   constexpr int H = K1::H, W = K1::W, PH = K1::KH / 2, PW = K1::KW / 2, HH = H / 2 + PH, QW = W / 4, WO = W / 2;
@@ -1058,7 +1060,7 @@ pack_frames_pooled_kernel(const TIn* __restrict__ frames, __nv_bfloat16* __restr
     for (int i = threadIdx.x; i < HH * SP / 8; i += 256) reinterpret_cast<uint4*>(s_hi)[i] = make_uint4(0, 0, 0, 0);
     __syncthreads();
     if (tp >= 1 && tp <= T) {
-      const TIn* f = frames + (b * T + (tp - 1)) * static_cast<long long>(H * W);
+      const TIn* f = frames + (b * pitch + (tp - 1)) * static_cast<long long>(H * W);
       for (int i = threadIdx.x; i < HH * QW; i += 256) {  // four consecutive pixels of one row per step
         const int row = i / QW, wq = (i - row * QW) * 4;
         const int h = 2 * row + par - PH;
@@ -1366,7 +1368,8 @@ void umma_layer_free(UmmaLayer* L) {
   L->d_w = nullptr; L->d_bias = nullptr;
 }
 
-int umma_pack_frames(const void* frames, bool frames_u8, __nv_bfloat16* act, const LayerGeom& g, int split, int B, int n_sms, cudaStream_t st) {
+int umma_pack_frames(const void* frames, bool frames_u8, int pitch, __nv_bfloat16* act, const LayerGeom& g, int split, int B, int n_sms,
+                     cudaStream_t st) {
   ProfScope ps(PROF_PACK, st);
   AVS_REQUIRE(g.H == AVS_H && g.W == AVS_W && g.KH == 5 && g.KW == 5 && g.Cin == 1, "pack_frames: LipNet layer-1 geometry only");
   const size_t sm = static_cast<size_t>(2) * ((g.PP + 8 + 7) & ~7) * sizeof(uint16_t);
@@ -1374,10 +1377,10 @@ int umma_pack_frames(const void* frames, bool frames_u8, __nv_bfloat16* act, con
   const int n_items = B * (AVS_T + 2) * 2;
   const unsigned grid = static_cast<unsigned>(std::min(n_items, n_sms * 8));
   if (!split) {  // bf16 kind: one X8 entry per pooled column
-    if (frames_u8) pack_frames_pooled_kernel<uint8_t><<<grid, 256, 0, st>>>(static_cast<const uint8_t*>(frames), act, g.PP, AVS_T, n_items);
-    else pack_frames_pooled_kernel<float><<<grid, 256, 0, st>>>(static_cast<const float*>(frames), act, g.PP, AVS_T, n_items);
-  } else if (frames_u8) pack_frames_kernel<uint8_t><<<grid, 256, sm, st>>>(static_cast<const uint8_t*>(frames), act, g.PP, split, AVS_T, n_items);
-  else pack_frames_kernel<float><<<grid, 256, sm, st>>>(static_cast<const float*>(frames), act, g.PP, split, AVS_T, n_items);
+    if (frames_u8) pack_frames_pooled_kernel<uint8_t><<<grid, 256, 0, st>>>(static_cast<const uint8_t*>(frames), act, g.PP, AVS_T, n_items, pitch);
+    else pack_frames_pooled_kernel<float><<<grid, 256, 0, st>>>(static_cast<const float*>(frames), act, g.PP, AVS_T, n_items, pitch);
+  } else if (frames_u8) pack_frames_kernel<uint8_t><<<grid, 256, sm, st>>>(static_cast<const uint8_t*>(frames), act, g.PP, split, AVS_T, n_items, pitch);
+  else pack_frames_kernel<float><<<grid, 256, sm, st>>>(static_cast<const float*>(frames), act, g.PP, split, AVS_T, n_items, pitch);
   AVS_LAUNCHED();
   return AVS_OK;
 }

@@ -819,8 +819,16 @@ extern "C" __attribute__((visibility("hidden"))) int avs_mfcc_plan_nshifts_inter
 // [ubase[i], ubase[i+1]) of one flat frame list, each frame carrying its clip in the 4th int; its [K][F_i] map holds
 // clip-local ids.  Per clip the frames and the map are exactly those of a uniform plan of that clip alone (same keys,
 // same map resolved to keys), so the kernels compute the same values and sum them in the same order.
+//
+// A windowed plan (avs_mfcc_ragged_plan_create_windows) is the same type with group > 0: its clips are overlapping windows
+// of one recording, clip i's audio starts at audio_off[i] of the recording itself (nothing is packed, the offsets may
+// overlap and need not be aligned), and its frames are keyed in recording coordinates within a de-duplication group of
+// `group` consecutive windows: a key shared by windows of a group is one unique frame, every such window's map points to
+// it, and each frame's 4th int is a window whose descriptor has audio_off 0.  ubase[i] is then the first frame of window
+// i's group, and a window's map holds ids relative to that.
 struct avs_mfcc_ragged_plan {
   int n_clips, sr, hop, n_mfcc, n_shifts, max_frames;
+  int group = 0;                     // windows per de-duplication group (windowed plans); 0: a ragged plan
   std::vector<long long> audio_off;  // [n_clips + 1] packed-audio offsets in samples; the last one is the buffer's size
   std::vector<int> ubase;            // [n_clips + 1] first unique frame of each clip in the flat frame list
   int4* d_frames = nullptr;          // [U] (start, lo, hi, clip)
@@ -1067,6 +1075,136 @@ void build_ragged(int n_clips, const int32_t* lengths, int sample_rate, const in
   h.ubase[n_clips] = static_cast<int>(h.frames.size());
 }
 
+// ------------------------------------------------------------------------------------------------ windowed plans
+constexpr long long kMaxWindowAudio = (1LL << 31) - 4096;  // recording coordinates (+ one FFT frame) stay inside int32
+
+int validate_windows(int n_windows, long long n_audio, const int64_t* starts, const int32_t* lengths, int group,
+                     int sample_rate, const int32_t* row, int n_shifts, int max_frames, int n_mfcc) {
+  AVS_REQUIRE(starts != nullptr && lengths != nullptr && row != nullptr, "null argument");
+  AVS_REQUIRE(n_windows > 0, "a windowed plan needs at least one window");
+  AVS_REQUIRE(sample_rate > 0 && n_shifts > 0, "empty problem");
+  if (group < 1) {
+    set_error("windowed plan: group_clips is %d; a de-duplication group holds at least one window", group);
+    return AVS_EINVAL;
+  }
+  if (n_audio < 1 || n_audio >= kMaxWindowAudio) {
+    set_error("windowed plan: the recording has %lld samples; it must have at least one and fewer than 2^31 - 4096", n_audio);
+    return AVS_EINVAL;
+  }
+  for (int i = 0; i < n_windows; ++i) {
+    if (starts[i] < 0 || starts[i] >= n_audio) {
+      set_error("windowed plan: window %d starts at sample %lld, outside the recording's %lld samples", i,
+                static_cast<long long>(starts[i]), n_audio);
+      return AVS_EINVAL;
+    }
+    if (lengths[i] > 0 && starts[i] + lengths[i] > n_audio) {
+      set_error("windowed plan: window %d ends at sample %lld, after the recording's %lld samples", i,
+                static_cast<long long>(starts[i]) + lengths[i], n_audio);
+      return AVS_EINVAL;
+    }
+  }
+  // lengths, frame limits and the map size: exactly the checks of a ragged batch of the cut windows (one shift row)
+  const int hop = std::max(1, sample_rate / 40);
+  long long map_total = 0;
+  for (int i = 0; i < n_windows; ++i) {
+    if (lengths[i] <= 0) {
+      set_error("windowed plan: window %d has %d samples; every window needs at least one", i, lengths[i]);
+      return AVS_EINVAL;
+    }
+    const int F = 1 + lengths[i] / hop;
+    if (max_frames > 0 && F > max_frames) {
+      set_error("windowed plan: window %d has %d samples = %d STFT frames; at n_mfcc = %d the statistics kernel holds at "
+                "most %d frames (%d KB of shared memory)", i, lengths[i], F, n_mfcc, max_frames, kStatsSmemLimit / 1024);
+      return AVS_EINVAL;
+    }
+    map_total += static_cast<long long>(n_shifts) * F;
+  }
+  AVS_REQUIRE(map_total < (1LL << 31), "windowed plan: more than 2^31 (shift, frame) pairs in one recording");
+  return AVS_OK;
+}
+
+struct WindowHostPlan {
+  std::vector<int> n_frames;      // [W]
+  std::vector<int> gbase;         // [n_groups + 1] first unique frame of each group
+  std::vector<long long> mbase;   // [W + 1]
+  std::vector<int4> frames;       // flat (start, lo, hi, first window of the group), recording coordinates
+  std::vector<int> map;           // per window [K][F_w], group-relative ids
+};
+
+// Host plan of validated windows.  A window of length n is planned as a cut clip of that length (build_ragged over the
+// distinct lengths: every window shares the one shift row, so the row's stable keys are built once and only the frames
+// touching a window's end are keyed per length); its keys are then moved to recording coordinates, (start + a0, lo + a0,
+// hi + a0), and numbered within the group — the all-zero key stays (0, 0, 0), once per group.  The window-relative range
+// [lo, hi) lies inside [0, n), so the moved key reads exactly the samples of the cut clip, and equal moved keys read the
+// same samples with the same zero fill.
+void build_windows(int n_windows, const int64_t* starts, const int32_t* lengths, int group, int sample_rate, const int32_t* row,
+                   int K, WindowHostPlan& h) {
+  std::vector<int32_t> distinct(lengths, lengths + n_windows);
+  std::sort(distinct.begin(), distinct.end());
+  distinct.erase(std::unique(distinct.begin(), distinct.end()), distinct.end());
+  const int nd = static_cast<int>(distinct.size());
+  std::vector<int32_t> rows(static_cast<size_t>(nd) * K);
+  for (int d = 0; d < nd; ++d) std::copy(row, row + K, rows.begin() + static_cast<size_t>(d) * K);
+  RaggedHostPlan rel;
+  build_ragged(nd, distinct.data(), sample_rate, rows.data(), K, rel);
+
+  const int n_groups = (n_windows + group - 1) / group;
+  h.n_frames.resize(n_windows);
+  h.mbase.resize(n_windows + 1);
+  h.mbase[0] = 0;
+  for (int i = 0; i < n_windows; ++i) {
+    const int d = static_cast<int>(std::lower_bound(distinct.begin(), distinct.end(), lengths[i]) - distinct.begin());
+    h.n_frames[i] = rel.n_frames[d];
+    h.mbase[i + 1] = h.mbase[i] + static_cast<long long>(K) * h.n_frames[i];
+  }
+  h.map.resize(h.mbase[n_windows]);
+  h.gbase.assign(n_groups + 1, 0);
+  h.frames.clear();
+  TailKeys keys;
+  std::vector<int> gid;
+  for (int g = 0; g < n_groups; ++g) {
+    const int w0 = g * group, w1 = std::min(n_windows, w0 + group);
+    const int fbase = static_cast<int>(h.frames.size());
+    h.gbase[g] = fbase;
+    size_t expect = 0;
+    for (int i = w0; i < w1; ++i) {
+      const int d = static_cast<int>(std::lower_bound(distinct.begin(), distinct.end(), lengths[i]) - distinct.begin());
+      expect += rel.ubase[d + 1] - rel.ubase[d];
+    }
+    keys.reset(expect);
+    int zero = -1;
+    for (int i = w0; i < w1; ++i) {
+      const int d = static_cast<int>(std::lower_bound(distinct.begin(), distinct.end(), lengths[i]) - distinct.begin());
+      const int a0 = static_cast<int>(starts[i]);
+      const int nu = rel.ubase[d + 1] - rel.ubase[d];
+      gid.resize(nu);
+      for (int u = 0; u < nu; ++u) {
+        const int4 k = rel.frames[rel.ubase[d] + u];
+        const int next = static_cast<int>(h.frames.size()) - fbase;
+        if (k.x == 0 && k.y == 0 && k.z == 0) {  // the all-zero frame (a non-zero key has lo < hi)
+          if (zero < 0) {
+            zero = next;
+            h.frames.push_back(make_int4(0, 0, 0, w0));
+          }
+          gid[u] = zero;
+          continue;
+        }
+        const int id = keys.find_or_insert(k.x + a0, k.y + a0, k.z + a0, next);
+        if (id >= 0) {
+          gid[u] = id;
+        } else {
+          gid[u] = next;
+          h.frames.push_back(make_int4(k.x + a0, k.y + a0, k.z + a0, w0));
+        }
+      }
+      const int* src = rel.map.data() + rel.mbase[d];
+      int* dst = h.map.data() + h.mbase[i];
+      for (long long e = 0, ne = h.mbase[i + 1] - h.mbase[i]; e < ne; ++e) dst[e] = gid[src[e]];
+    }
+  }
+  h.gbase[n_groups] = static_cast<int>(h.frames.size());
+}
+
 }  // namespace
 }  // namespace avs
 
@@ -1124,6 +1262,67 @@ extern "C" int avs_mfcc_ragged_plan_create(int n_clips, const int32_t* lengths, 
   return AVS_OK;
 }
 
+extern "C" int avs_mfcc_ragged_plan_describe_windows(int n_windows, int64_t n_audio, const int64_t* audio_starts,
+                                                     const int32_t* lengths, int group_clips, int sample_rate,
+                                                     const int32_t* shift_row, int n_shifts, int32_t* n_frames,
+                                                     int32_t* group_unique, int32_t* frames_out, int32_t* map_out) {
+  AVS_REQUIRE(n_frames && group_unique, "null argument");
+  int rc;
+  if ((rc = validate_windows(n_windows, n_audio, audio_starts, lengths, group_clips, sample_rate, shift_row, n_shifts, 0, 0)))
+    return rc;
+  WindowHostPlan h;
+  build_windows(n_windows, audio_starts, lengths, group_clips, sample_rate, shift_row, n_shifts, h);
+  std::copy(h.n_frames.begin(), h.n_frames.end(), n_frames);
+  for (size_t g = 0; g + 1 < h.gbase.size(); ++g) group_unique[g] = h.gbase[g + 1] - h.gbase[g];
+  if (frames_out)
+    for (size_t u = 0; u < h.frames.size(); ++u) {
+      frames_out[3 * u] = h.frames[u].x; frames_out[3 * u + 1] = h.frames[u].y; frames_out[3 * u + 2] = h.frames[u].z;
+    }
+  if (map_out) std::copy(h.map.begin(), h.map.end(), map_out);
+  return AVS_OK;
+}
+
+extern "C" int avs_mfcc_ragged_plan_create_windows(int n_windows, int64_t n_audio, const int64_t* audio_starts,
+                                                   const int32_t* lengths, int group_clips, int sample_rate, int n_mfcc,
+                                                   const int32_t* shift_row, int n_shifts, void* stream,
+                                                   avs_mfcc_ragged_plan** out) {
+  AVS_REQUIRE(out != nullptr, "null argument");
+  AVS_REQUIRE(n_mfcc >= 1 && n_mfcc <= kMaxQ, "n_mfcc must be in [1, 40]");
+  int rc;
+  if ((rc = validate_windows(n_windows, n_audio, audio_starts, lengths, group_clips, sample_rate, shift_row, n_shifts,
+                             max_frames_for(n_mfcc), n_mfcc)))
+    return rc;
+  WindowHostPlan h;
+  build_windows(n_windows, audio_starts, lengths, group_clips, sample_rate, shift_row, n_shifts, h);
+  avs_mfcc_ragged_plan* p = new avs_mfcc_ragged_plan();
+  p->n_clips = n_windows;
+  p->sr = sample_rate;
+  p->hop = std::max(1, sample_rate / 40);
+  p->n_mfcc = n_mfcc;
+  p->n_shifts = n_shifts;
+  p->group = group_clips;
+  p->max_frames = *std::max_element(h.n_frames.begin(), h.n_frames.end());
+  p->audio_off.assign(audio_starts, audio_starts + n_windows);
+  p->audio_off.push_back(n_audio);
+  p->ubase.resize(n_windows + 1);
+  std::vector<RaggedClip> clips(n_windows);
+  for (int i = 0; i < n_windows; ++i) {
+    p->ubase[i] = h.gbase[i / group_clips];
+    clips[i] = RaggedClip{0, p->ubase[i], static_cast<int>(h.mbase[i]), h.n_frames[i], 0};
+  }
+  p->ubase[n_windows] = h.gbase.back();
+  HostTables tabs;
+  build_tables(sample_rate, n_mfcc, tabs);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if ((rc = upload_async(&p->d_frames, h.frames, st)) || (rc = upload_async(&p->d_map, h.map, st)) ||
+      (rc = upload_async(&p->d_clips, clips, st)) || (rc = upload_tables(p->tab, tabs, st, true))) {
+    avs_mfcc_ragged_plan_destroy(p);
+    return rc;
+  }
+  *out = p;
+  return AVS_OK;
+}
+
 extern "C" void avs_mfcc_ragged_plan_destroy(avs_mfcc_ragged_plan* p) {
   if (!p) return;
   // the buffers come from the stream-ordered allocator, which cudaFree does not wait for: kernels still queued may use them
@@ -1146,6 +1345,7 @@ extern "C" size_t avs_mfcc_ragged_workspace_bytes(const avs_mfcc_ragged_plan* p)
 size_t avs::mfcc_ragged_frames(const avs_mfcc_ragged_plan* p, int c0, int n) {
   return static_cast<size_t>(p->ubase[c0 + n] - p->ubase[c0]);
 }
+int avs::mfcc_ragged_group(const avs_mfcc_ragged_plan* p) { return p->group; }
 void avs::mfcc_ragged_shape(const avs_mfcc_ragged_plan* p, int* n_clips, int* n_shifts, int* n_mfcc) {
   *n_clips = p->n_clips;
   *n_shifts = p->n_shifts;

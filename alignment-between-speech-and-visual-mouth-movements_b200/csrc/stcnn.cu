@@ -50,10 +50,13 @@ static StcnnWs carve(const avs_stcnn* net, int B, void* ws, bool need_emb) {
   return r;
 }
 
-// u8 pixels -> float32(v / 255.0), the frames tensor the reference builds (dataset.py:226-231)
-__global__ void __launch_bounds__(256) u8_to_unit_f32_kernel(const uint8_t* __restrict__ in, float* __restrict__ out, long long n) {
+// u8 pixels -> float32(v / 255.0), the frames tensor the reference builds (dataset.py:226-231).  The n outputs are clips of
+// clip_elems values back to back; input clip b starts at in + b * in_pitch (in_pitch > clip_elems: the windows of a
+// recording are converted, not its first frames)
+__global__ void __launch_bounds__(256) u8_to_unit_f32_kernel(const uint8_t* __restrict__ in, float* __restrict__ out, long long n,
+                                                             long long clip_elems, long long in_pitch) {
   const long long i = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x;
-  if (i < n) out[i] = static_cast<float>(static_cast<double>(in[i]) / 255.0);
+  if (i < n) out[i] = static_cast<float>(static_cast<double>(in[i / clip_elems * in_pitch + i % clip_elems]) / 255.0);
 }
 
 }  // namespace avs
@@ -129,12 +132,13 @@ extern "C" size_t avs_stcnn_workspace_bytes(const avs_stcnn* net, int n_clips) {
 // cap_clips: the workspace is carved for this many clips (>= B), so that repeated calls with different
 // B see the same buffer placement; pads_clean: the caller guarantees that the padding positions of the
 // parity-plane buffers are still zero (zeroed once, and kernels only ever write data positions).
-int avs::stcnn_forward_impl(const avs_stcnn* net, const void* frames_any, bool frames_u8, int B, int cap_clips, bool pads_clean,
+int avs::stcnn_forward_impl(const avs_stcnn* net, const void* frames_any, bool frames_u8, int pitch, int B, int cap_clips, bool pads_clean,
                             const StcnnHooks& hooks, float* out_emb, float* out_vstats, float* out_pool1, float* out_pool2, void* workspace,
                             size_t workspace_bytes, void* stream) {
   AVS_REQUIRE(net && frames_any && workspace, "null argument");
   AVS_REQUIRE(out_emb || out_vstats, "nothing to compute");
   AVS_REQUIRE(cap_clips >= B, "workspace capacity below batch");
+  AVS_REQUIRE(pitch >= 1, "clip pitch must be at least one frame");
   if (B <= 0) return AVS_OK;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   StcnnWs w = carve(net, cap_clips, workspace, out_emb == nullptr);
@@ -153,31 +157,34 @@ int avs::stcnn_forward_impl(const avs_stcnn* net, const void* frames_any, bool f
   auto after_l2 = [&]() -> int { return hooks.on_layer1 ? hooks.on_layer1(hooks.on_layer1_arg) : AVS_OK; };
   if (net->precision == AVS_PREC_FP32) {
     const float* frames = static_cast<const float*>(frames_any);
+    long long fpitch = static_cast<long long>(pitch) * AVS_H * AVS_W;  // values from one clip's first frame to the next's
     if (frames_u8) {
-      const long long n = static_cast<long long>(B) * AVS_T * AVS_H * AVS_W;
-      u8_to_unit_f32_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(static_cast<const uint8_t*>(frames_any), w.f32frames, n);
+      const long long clip = static_cast<long long>(AVS_T) * AVS_H * AVS_W, n = B * clip;
+      u8_to_unit_f32_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(static_cast<const uint8_t*>(frames_any), w.f32frames, n,
+                                                                                   clip, fpitch);
       AVS_LAUNCHED();
       frames = w.f32frames;
+      fpitch = clip;
     }
     // gridDim.y = clips * T is capped at 65535: run in slabs of 512 clips
     for (int b0 = 0; b0 < B; b0 += 512) {
       const int nb = std::min(512, B - b0);
-      const float* f = frames + static_cast<size_t>(b0) * AVS_T * AVS_H * AVS_W;
+      const float* f = frames + b0 * fpitch;
       float* p1 = w.p1 + static_cast<size_t>(b0) * 32 * AVS_T * 25 * 50;
       float* p2 = w.p2 + static_cast<size_t>(b0) * 64 * AVS_T * 12 * 25;
       if (b0 == 0 && hooks.before_layer1) AVS_CUDA(cudaStreamWaitEvent(st, hooks.before_layer1, 0));
-      if ((rc = conv_pool_ffma(f, net->w[0], net->b[0], p1, nb, 1, 32, AVS_T, 50, 100, 5, 5, 32LL * AVS_T * 1250,
+      if ((rc = conv_pool_ffma(f, net->w[0], net->b[0], p1, nb, 1, 32, AVS_T, 50, 100, 5, 5, fpitch, 32LL * AVS_T * 1250,
                                AVS_T * 1250LL, 1250, st)))
         return rc;
       if (b0 == 0 && (rc = after_l1())) return rc;
-      if ((rc = conv_pool_ffma(p1, net->w[1], net->b[1], p2, nb, 32, 64, AVS_T, 25, 50, 5, 5, 64LL * AVS_T * 300,
-                               AVS_T * 300LL, 300, st)))
+      if ((rc = conv_pool_ffma(p1, net->w[1], net->b[1], p2, nb, 32, 64, AVS_T, 25, 50, 5, 5, 32LL * AVS_T * 1250,
+                               64LL * AVS_T * 300, AVS_T * 300LL, 300, st)))
         return rc;
       if (b0 == 0 && (rc = after_l2())) return rc;
       if (b0 == 0 && hooks.before_layer3) AVS_CUDA(cudaStreamWaitEvent(st, hooks.before_layer3, 0));
       // layer 3 writes the permuted (B, T, C*72) embedding directly (model.py:81-82)
       if ((rc = conv_pool_ffma(p2, net->w[2], net->b[2], emb + static_cast<size_t>(b0) * AVS_T * AVS_EMB, nb, 64, 96,
-                               AVS_T, 12, 25, 3, 3, static_cast<long long>(AVS_T) * AVS_EMB, 72, AVS_EMB, st)))
+                               AVS_T, 12, 25, 3, 3, 64LL * AVS_T * 300, static_cast<long long>(AVS_T) * AVS_EMB, 72, AVS_EMB, st)))
         return rc;
     }
     if (out_pool1) AVS_CUDA(cudaMemcpyAsync(out_pool1, w.p1, static_cast<size_t>(B) * 32 * AVS_T * 1250 * 4, cudaMemcpyDeviceToDevice, st));
@@ -189,7 +196,7 @@ int avs::stcnn_forward_impl(const avs_stcnn* net, const void* frames_any, bool f
       AVS_CUDA(cudaMemsetAsync(w.act[1], 0, umma_act_bytes(net->L[1].g, split, B), st));
       AVS_CUDA(cudaMemsetAsync(w.act[2], 0, umma_act_bytes(net->L[2].g, split, B), st));
     }
-    if ((rc = umma_pack_frames(frames_any, frames_u8, w.act[0], net->L[0].g, split, B, net->n_sms, st))) return rc;
+    if ((rc = umma_pack_frames(frames_any, frames_u8, pitch, w.act[0], net->L[0].g, split, B, net->n_sms, st))) return rc;
     for (int l = 0; l < 3; ++l) {
       EpiOut eo{};
       if (l < 2) {
@@ -218,13 +225,13 @@ int avs::stcnn_forward_impl(const avs_stcnn* net, const void* frames_any, bool f
 extern "C" int avs_stcnn_forward_debug(const avs_stcnn* net, const float* frames, int B, float* out_emb,
                                        float* out_vstats, float* out_pool1, float* out_pool2, void* workspace,
                                        size_t workspace_bytes, void* stream) {
-  return stcnn_forward_impl(net, frames, false, B, B, false, StcnnHooks{}, out_emb, out_vstats, out_pool1, out_pool2, workspace,
+  return stcnn_forward_impl(net, frames, false, AVS_T, B, B, false, StcnnHooks{}, out_emb, out_vstats, out_pool1, out_pool2, workspace,
                             workspace_bytes, stream);
 }
 
 extern "C" int avs_stcnn_forward_u8(const avs_stcnn* net, const uint8_t* frames, int n_clips, float* out_emb, float* out_vstats,
                                     void* workspace, size_t workspace_bytes, void* stream) {
-  return stcnn_forward_impl(net, frames, true, n_clips, n_clips, false, StcnnHooks{}, out_emb, out_vstats, nullptr, nullptr, workspace,
+  return stcnn_forward_impl(net, frames, true, AVS_T, n_clips, n_clips, false, StcnnHooks{}, out_emb, out_vstats, nullptr, nullptr, workspace,
                             workspace_bytes, stream);
 }
 

@@ -25,10 +25,13 @@ int mfcc_ragged_stats_part(const avs_mfcc_ragged_plan* p, int c0, int n, float* 
 // unique frames of clips [c0, c0 + n) of a ragged plan
 size_t mfcc_ragged_frames(const avs_mfcc_ragged_plan* p, int c0, int n);
 void mfcc_ragged_shape(const avs_mfcc_ragged_plan* p, int* n_clips, int* n_shifts, int* n_mfcc);
+// windows per de-duplication group of a windowed plan (avs_mfcc_ragged_plan_create_windows); 0 for a ragged plan
+int mfcc_ragged_group(const avs_mfcc_ragged_plan* p);
 
-// fp32 CUDA-core layer: in NCDHW f32, w OIDHW f32, out addressed as b*o_sb + c*o_sc + t*o_st + ho*Wo + wo
+// fp32 CUDA-core layer: in NCDHW f32 with clip b at in + b*i_sb, w OIDHW f32, out addressed as
+// b*o_sb + c*o_sc + t*o_st + ho*Wo + wo
 int conv_pool_ffma(const float* in, const float* w, const float* bias, float* out, int B, int Cin, int Cout, int T,
-                   int H, int W, int KH, int KW, long long o_sb, long long o_sc, long long o_st, cudaStream_t st);
+                   int H, int W, int KH, int KW, long long i_sb, long long o_sb, long long o_sc, long long o_st, cudaStream_t st);
 int vstats(const float* emb, float* out, int B, int F, cudaStream_t st);
 int stcnn_precision(const avs_stcnn* net);
 
@@ -89,7 +92,9 @@ int umma_layer_build(UmmaLayer* L, const LayerGeom& g, int split, const float* w
 void umma_layer_free(UmmaLayer* L);
 void conv_item_span(int n_clips, int T, int n_tiles, int NT, int grid, int cta, int* first, int* last);
 size_t umma_act_bytes(const LayerGeom& g, int split, int B);   // bytes of the input activation buffer of a layer
-int umma_pack_frames(const void* frames, bool frames_u8, __nv_bfloat16* act, const LayerGeom& g1, int split, int B, int n_sms, cudaStream_t st);
+// frames: clip b starts pitch frames of [H, W] after clip b - 1 (pitch = T: a batch of clips; < T: overlapping windows)
+int umma_pack_frames(const void* frames, bool frames_u8, int pitch, __nv_bfloat16* act, const LayerGeom& g1, int split, int B,
+                     int n_sms, cudaStream_t st);
 int umma_conv_forward(const UmmaLayer& L, const __nv_bfloat16* act_in, const EpiOut& eo, int B, int n_sms, cudaStream_t st);
 int umma_unpack_act(const __nv_bfloat16* act, float* out_ncdhw, const LayerGeom& g_next, int split, int C, int B, cudaStream_t st);
 
@@ -105,7 +110,8 @@ struct StcnnHooks {
   void* on_layer1_arg = nullptr;
   cudaEvent_t before_layer3 = nullptr;
 };
-int stcnn_forward_impl(const avs_stcnn* net, const void* frames, bool frames_u8, int B, int cap_clips, bool pads_clean,
+// pitch: frames between the starts of consecutive clips (AVS_T for a batch of clips, the stride for windows of a recording)
+int stcnn_forward_impl(const avs_stcnn* net, const void* frames, bool frames_u8, int pitch, int B, int cap_clips, bool pads_clean,
                        const StcnnHooks& hooks, float* out_emb,
                        float* out_vstats, float* out_pool1, float* out_pool2, void* workspace, size_t workspace_bytes,
                        void* stream);

@@ -186,8 +186,9 @@ static int enqueue_audio_branch(void* arg) {
   return rc;
 }
 
+// frames: the chunk's first clip; clip b of the chunk starts `pitch` frames after clip b - 1 (AVS_T, or the window stride)
 static int run_chunk(avs_sweep* s, const void* frames, bool frames_u8, const float* audio, int c0, int n, cudaStream_t st,
-                     const avs_mfcc_ragged_plan* rp = nullptr) {
+                     const avs_mfcc_ragged_plan* rp = nullptr, int pitch = AVS_T) {
   int rc;
   float* vst = s->vstats + static_cast<size_t>(c0) * AVS_VSTATS;
   float* ast = s->astats + static_cast<size_t>(c0) * s->K * 2 * s->n_mfcc;
@@ -215,7 +216,7 @@ static int run_chunk(avs_sweep* s, const void* frames, bool frames_u8, const flo
 #ifdef AVS_EXPERIMENTS
   static const int audio_mode = env_knob("AVS_AUDIO_MODE", 0);  // 1 serial, 2 conv3 does not wait for the FFT kernel
   if (audio_mode == 1 && !rp) {
-    if ((rc = stcnn_forward_impl(s->net, frames, frames_u8, n, s->chunk, true, StcnnHooks{}, nullptr, vst, nullptr, nullptr, s->ws_stcnn, s->ws_stcnn_bytes, st)))
+    if ((rc = stcnn_forward_impl(s->net, frames, frames_u8, pitch, n, s->chunk, true, StcnnHooks{}, nullptr, vst, nullptr, nullptr, s->ws_stcnn, s->ws_stcnn_bytes, st)))
       return rc;
     return avs_mfcc_stats_sweep(s->plan, audio, n, ast, s->ws_mfcc, s->ws_mfcc_bytes, st);
   }
@@ -228,7 +229,7 @@ static int run_chunk(avs_sweep* s, const void* frames, bool frames_u8, const flo
     AVS_CUDA(cudaEventRecord(s->ev_head, s->side));
     hooks.before_layer1 = s->ev_head;
   }
-  if ((rc = stcnn_forward_impl(s->net, frames, frames_u8, n, s->chunk, true, hooks, nullptr, vst, nullptr, nullptr,
+  if ((rc = stcnn_forward_impl(s->net, frames, frames_u8, pitch, n, s->chunk, true, hooks, nullptr, vst, nullptr, nullptr,
                                s->ws_stcnn, s->ws_stcnn_bytes, st)))
     return rc;
   AVS_CUDA(cudaStreamWaitEvent(st, s->ev_join, 0));
@@ -293,6 +294,7 @@ static int sweep_run_ragged(avs_sweep* s, const avs_mfcc_ragged_plan* rp, const 
   AVS_REQUIRE(n_clips == rn, "n_clips differs from the ragged plan's");
   AVS_REQUIRE(rk == s->K, "the ragged plan's shift count differs from the sweep's");
   AVS_REQUIRE(rq == s->n_mfcc, "the ragged plan's n_mfcc differs from the sweep's");
+  AVS_REQUIRE(mfcc_ragged_group(rp) == 0, "a windowed plan goes to avs_sweep_run_windows, not avs_sweep_run_ragged");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   int rc;
   if ((rc = begin_call(s, st)) || (rc = ensure_capacity(s, n_clips, st)) || (rc = ensure_ragged_ws(s, rp, n_clips, st))) return rc;
@@ -315,6 +317,46 @@ extern "C" int avs_sweep_run_ragged_u8(avs_sweep* s, const avs_mfcc_ragged_plan*
                                        const float* audio_packed, int n_clips, float* out_scores, int32_t* out_best,
                                        void* stream) {
   return sweep_run_ragged(s, plan, frames, true, audio_packed, n_clips, out_scores, out_best, stream);
+}
+
+// Overlapping windows of one recording: window w is frames [w * stride, w * stride + 75) of `frames` and the audio the
+// windowed plan gives it inside `audio` (the recording).  The same chunks, streams, hooks and ordering as the ragged sweep;
+// a chunk's STCNN reads its windows in place (pitch = stride) and its K1 covers whole de-duplication groups of the plan.
+static int sweep_run_windows(avs_sweep* s, const avs_mfcc_ragged_plan* rp, const void* frames, bool frames_u8, int stride,
+                             const float* audio, int n_windows, float* out_scores, int32_t* out_best, void* stream) {
+  AVS_REQUIRE(s && rp && frames && audio && out_scores && out_best, "null argument");
+  int rn, rk, rq;
+  mfcc_ragged_shape(rp, &rn, &rk, &rq);
+  const int group = mfcc_ragged_group(rp);
+  AVS_REQUIRE(group > 0, "avs_sweep_run_windows needs a windowed plan (avs_mfcc_ragged_plan_create_windows)");
+  AVS_REQUIRE(stride >= 1, "stride_frames must be at least 1");
+  AVS_REQUIRE(n_windows == rn, "n_windows differs from the windowed plan's");
+  AVS_REQUIRE(rk == s->K, "the windowed plan's shift count differs from the sweep's");
+  AVS_REQUIRE(rq == s->n_mfcc, "the windowed plan's n_mfcc differs from the sweep's");
+  if (s->chunk % group != 0) {
+    set_error("the windowed plan's de-duplication groups of %d windows do not divide the sweep's chunks of %d", group, s->chunk);
+    return AVS_EINVAL;
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  int rc;
+  if ((rc = begin_call(s, st)) || (rc = ensure_capacity(s, n_windows, st)) || (rc = ensure_ragged_ws(s, rp, n_windows, st))) return rc;
+  const size_t fstride = static_cast<size_t>(stride) * AVS_H * AVS_W * (frames_u8 ? 1 : sizeof(float));
+  for (int c0 = 0; c0 < n_windows; c0 += s->chunk) {
+    const int n = std::min(s->chunk, n_windows - c0);
+    if ((rc = run_chunk(s, static_cast<const uint8_t*>(frames) + c0 * fstride, frames_u8, audio, c0, n, st, rp, stride))) break;
+  }
+  if (!rc) rc = score_all(s, n_windows, out_scores, out_best, st);
+  const int rc2 = end_call(s, st);
+  return rc ? rc : rc2;
+}
+
+extern "C" int avs_sweep_run_windows(avs_sweep* s, const avs_mfcc_ragged_plan* plan, const float* frames, int stride_frames,
+                                     const float* audio, int n_windows, float* out_scores, int32_t* out_best, void* stream) {
+  return sweep_run_windows(s, plan, frames, false, stride_frames, audio, n_windows, out_scores, out_best, stream);
+}
+extern "C" int avs_sweep_run_windows_u8(avs_sweep* s, const avs_mfcc_ragged_plan* plan, const uint8_t* frames, int stride_frames,
+                                        const float* audio, int n_windows, float* out_scores, int32_t* out_best, void* stream) {
+  return sweep_run_windows(s, plan, frames, true, stride_frames, audio, n_windows, out_scores, out_best, stream);
 }
 
 static bool is_pinned(const void* p) {

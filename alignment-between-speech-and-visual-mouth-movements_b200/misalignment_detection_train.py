@@ -206,6 +206,103 @@ def audio_stats_sweep_ragged(audio: Sequence[torch.Tensor], shifts_samples, samp
     return out
 
 
+WINDOW_FRAMES = 75                         # frames per scored window: the clip length the detector was trained on
+
+
+def window_bounds(n_frames: int, n_audio: int, fps: float, sample_rate: int, stride_frames: int):
+    """Windows of a long recording, the one place their semantics are defined (include/avsync.h: windowed K1).
+
+    Window ``w`` covers video frames ``[t_w, t_w + 75)`` with ``t_w = w * stride_frames``, for every ``w`` with
+    ``t_w + 75 <= n_frames``; frames after the last full window are not scored.  Its audio is ``[a0_w, a1_w)`` with
+    ``a0_w = int(t_w / max(fps, 1e-5) * sample_rate)`` (the truncation of ``shift_samples``) and
+    ``a1_w = min(n_audio, int((t_w + 75) / max(fps, 1e-5) * sample_rate))``.  Each window is scored as that cut clip
+    would be.  Returns int64 arrays ``(start_frames, a0, a1)`` of length ``(n_frames - 75) // stride_frames + 1``.
+    Raises ``RuntimeError`` for ``n_frames < 75``, ``stride_frames < 1`` and a window whose audio slice is empty."""
+    n_frames, n_audio, stride_frames = int(n_frames), int(n_audio), int(stride_frames)
+    if stride_frames < 1:
+        raise RuntimeError(f"stride_frames must be at least 1, got {stride_frames}")
+    if n_frames < WINDOW_FRAMES:
+        raise RuntimeError(f"a recording needs at least {WINDOW_FRAMES} frames to be scored, got {n_frames}")
+    W = (n_frames - WINDOW_FRAMES) // stride_frames + 1
+    t = np.arange(W, dtype=np.int64) * stride_frames
+    f = max(float(fps), 1e-5)
+    a0 = np.trunc(t.astype(np.float64) / f * sample_rate).astype(np.int64)
+    a1 = np.minimum(n_audio, np.trunc((t + WINDOW_FRAMES).astype(np.float64) / f * sample_rate).astype(np.int64))
+    empty = np.nonzero(a1 <= a0)[0]
+    if empty.size:
+        w = int(empty[0])
+        raise RuntimeError(f"window {w} (frames {int(t[w])}..{int(t[w]) + WINDOW_FRAMES - 1}) has no audio: it starts at "
+                           f"sample {int(a0[w])} of {n_audio}")
+    return t, a0, a1
+
+
+class _MfccWindowPlan:
+    """Windowed K1 plan: overlapping windows of one recording, read in place, STFT frames shared within groups of
+    ``group_clips`` consecutive windows (include/avsync.h: avs_mfcc_ragged_plan_create_windows)."""
+
+    def __init__(self, n_audio: int, a0: np.ndarray, lengths: np.ndarray, sample_rate: int, n_mfcc: int,
+                 row: Sequence[int], group_clips: int):
+        a0 = np.ascontiguousarray(a0, dtype=np.int64)
+        ln = np.ascontiguousarray(lengths, dtype=np.int32)
+        row = np.ascontiguousarray(row, dtype=np.int32)
+        L = N.lib()
+        h = N.c_void_p()
+        self.stream = torch.cuda.current_stream()          # the plan's upload is queued here
+        N.check(L.avs_mfcc_ragged_plan_create_windows(len(a0), int(n_audio), a0.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)),
+                                                      ln.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), int(group_clips),
+                                                      int(sample_rate), int(n_mfcc),
+                                                      row.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), len(row),
+                                                      N.stream_ptr(), ctypes.byref(h)), "mfcc_ragged_plan_create_windows")
+        self.handle = N.Handle(h, L.avs_mfcc_ragged_plan_destroy)
+        self.n_clips, self.n_shifts, self.n_mfcc = len(a0), len(row), n_mfcc
+
+
+_window_plan_cache: "OrderedDict[tuple, _MfccWindowPlan]" = OrderedDict()
+
+
+def mfcc_window_plan(n_frames: int, n_audio: int, fps: float, stride_frames: int, sample_rate: int, n_mfcc: int,
+                     row: Sequence[int], group_clips: int):
+    """Windowed K1 plan of a recording and its ``window_bounds``, from a cache of the few most recent plans (the plan
+    depends on the recording's frame count, sample count and frame rate only, not on its content)."""
+    N.device_check()
+    starts, a0, a1 = window_bounds(n_frames, n_audio, fps, sample_rate, stride_frames)
+    key = (torch.cuda.current_device(), int(n_frames), int(n_audio), float(fps), int(stride_frames), int(sample_rate),
+           int(n_mfcc), tuple(int(s) for s in row), int(group_clips))
+    p = _window_plan_cache.get(key)
+    if p is None:
+        p = _MfccWindowPlan(n_audio, a0, a1 - a0, sample_rate, n_mfcc, row, group_clips)
+        _window_plan_cache[key] = p
+        while len(_window_plan_cache) > 4:
+            _window_plan_cache.popitem(last=False)
+    else:
+        _window_plan_cache.move_to_end(key)
+    return p, starts, a0, a1
+
+
+def _recording_audio(audio: torch.Tensor) -> torch.Tensor:
+    N.require_cuda(audio, "audio")
+    if audio.dim() != 1 or audio.numel() == 0:
+        raise RuntimeError(f"audio must be a non-empty 1-D tensor, got shape {tuple(audio.shape)}")
+    return N.f32c(audio)
+
+
+def audio_stats_sweep_windows(audio: torch.Tensor, n_frames: int, fps: float, stride_frames: int, shifts_samples: Sequence[int],
+                              sample_rate: int = 16000, n_mfcc: int = 20, group_clips: int = 64) -> torch.Tensor:
+    """K1 over the ``window_bounds`` windows of one recording (``audio`` 1-D CUDA f32, ``n_frames`` video frames at
+    ``fps``), one row of K sample delays for all windows.  Returns [W, K, 2*n_mfcc]; row w is bit for bit
+    ``audio_stats_sweep_ragged([audio[a0_w:a1_w]], [shifts_samples])[0]``."""
+    audio = _recording_audio(audio)
+    plan, _, _, _ = mfcc_window_plan(n_frames, audio.numel(), fps, stride_frames, sample_rate, n_mfcc, shifts_samples,
+                                     group_clips)
+    torch.cuda.current_stream().wait_stream(plan.stream)
+    L = N.lib()
+    out = torch.empty((plan.n_clips, plan.n_shifts, 2 * n_mfcc), dtype=torch.float32, device=audio.device)
+    ws = N.workspace(L.avs_mfcc_ragged_workspace_bytes(plan.handle.h), audio.device)
+    N.check(L.avs_mfcc_ragged_stats_sweep(plan.handle.h, N.ptr(audio), N.ptr(out), N.ptr(ws), ws.numel(), N.stream_ptr()),
+            "mfcc_ragged_stats_sweep")
+    return out
+
+
 def compute_audio_stats(audio: np.ndarray, sample_rate: int, n_mfcc: int) -> torch.Tensor:
     """Reference contract (:117-127): 1-D float audio -> CPU tensor [2*n_mfcc] = cat(mean, std)
     of ``librosa.feature.mfcc(y, sr, n_mfcc, hop_length=sr//40)`` over frames."""
@@ -309,6 +406,8 @@ class SyncSweeper:
     pipelines the H2D/D2H copies against compute chunk by chunk; ``run_ragged(frames, audio, fps)`` takes one audio
     tensor per clip, each of its own length and frame rate.  All return
     ``(scores [B, 2S+1], best_shift_frames [B])`` where ``best_shift_frames = argmax_k - S``.
+    ``run_windows(frames, audio, fps, stride_frames)`` scores one long recording as overlapping 75-frame windows and
+    also returns each window's first frame.
     ``frames`` is the reference's f32 tensor ``[B,1,75,50,100]`` or the uint8 pixels it is made from
     (``float32(u8 / 255.0)``, dataset.py:226-231): same scores bit for bit, a quarter of the bytes.
     """
@@ -378,6 +477,31 @@ class SyncSweeper:
         N.check(fn(self.handle.h, plan.handle.h, N.ptr(frames), N.ptr(packed), B, N.ptr(scores), N.ptr(best),
                    N.stream_ptr()), "sweep_run_ragged")
         return scores, best - self.S
+
+    def run_windows(self, frames: torch.Tensor, audio: torch.Tensor, fps=None, stride_frames: int = 25):
+        """A long recording scored as overlapping 75-frame windows every ``stride_frames`` frames (``window_bounds``):
+        ``frames`` [T, 50, 100] (uint8 pixels or the reference's f32 values) and ``audio`` 1-D f32 at the sweeper's
+        sample rate, both on the device; ``fps`` the recording's frame rate (default: the sweeper's).  The windows are
+        read in place, and STFT frames shared by neighbouring windows are computed once.  Returns
+        ``(scores [W, 2S+1], best_shift_frames [W], start_frames [W])``; window w's outputs equal, bit for bit,
+        ``run_ragged`` on the cut clip ``frames[t_w:t_w+75]``, ``audio[a0_w:a1_w]``."""
+        N.require_cuda(frames, "frames")
+        audio = _recording_audio(audio)
+        if frames.dim() != 3 or tuple(frames.shape[1:]) != (50, 100):
+            raise RuntimeError(f"expected frames of shape (T, 50, 100), got {tuple(frames.shape)}")
+        frames = frames.detach().contiguous() if frames.dtype == torch.uint8 else N.f32c(frames)
+        fps = self.fps if fps is None else float(fps)
+        row = [shift_samples(k, fps, self.sample_rate) for k in self.shift_frames]
+        plan, starts, _, _ = mfcc_window_plan(frames.shape[0], audio.numel(), fps, stride_frames, self.sample_rate,
+                                              self.n_mfcc, row, self.chunk_clips)
+        W = plan.n_clips
+        torch.cuda.current_stream().wait_stream(plan.stream)
+        scores = torch.empty((W, self.K), dtype=torch.float32, device=frames.device)
+        best = torch.empty((W,), dtype=torch.int32, device=frames.device)
+        fn = N.lib().avs_sweep_run_windows_u8 if frames.dtype == torch.uint8 else N.lib().avs_sweep_run_windows
+        N.check(fn(self.handle.h, plan.handle.h, N.ptr(frames), int(stride_frames), N.ptr(audio), W, N.ptr(scores),
+                   N.ptr(best), N.stream_ptr()), "sweep_run_windows")
+        return scores, best - self.S, torch.from_numpy(starts).to(frames.device)
 
     def run_host(self, frames: np.ndarray, audio: np.ndarray):
         u8 = frames.dtype == np.uint8

@@ -117,9 +117,36 @@ AVS_API int avs_mfcc_ragged_plan_describe(int n_clips, const int32_t* lengths, i
                                   int32_t* n_frames, int32_t* n_unique, int32_t* frames_out, int32_t* map_out);
 AVS_API int avs_mfcc_ragged_plan_audio_offsets(const avs_mfcc_ragged_plan* plan, int64_t* audio_offsets);
 AVS_API size_t avs_mfcc_ragged_workspace_bytes(const avs_mfcc_ragged_plan* plan);
-/* audio: device f32, packed at the plan's offsets; out_stats: device f32 [n_clips, n_shifts, 2*n_mfcc]. */
+/* audio: device f32, packed at the plan's offsets (a windowed plan: the recording itself); out_stats: device f32
+ * [n_clips, n_shifts, 2*n_mfcc]. */
 AVS_API int avs_mfcc_ragged_stats_sweep(const avs_mfcc_ragged_plan* plan, const float* audio, float* out_stats,
                                 void* workspace, size_t workspace_bytes, void* stream);
+
+/* Windowed K1: overlapping windows of ONE recording of n_audio samples (the windowed sync sweep below).
+ * Window semantics (computed in Python by window_bounds, the one place that defines them): for a recording of T video
+ * frames at `fps` and a stride of `stride` frames, window w covers frames [t_w, t_w + 75), t_w = w * stride, for every w
+ * with t_w + 75 <= T (W = (T - 75) / stride + 1 windows; T < 75 is an error; frames after the last full window are not
+ * scored).  Its audio is [a0_w, a1_w) with a0_w = int(t_w / max(fps, 1e-5) * sr) (the float64 truncation of
+ * shift_samples) and a1_w = min(n_audio, int((t_w + 75) / max(fps, 1e-5) * sr)); an empty slice is an error.  Window w's
+ * statistics equal, bit for bit, those of the cut clip audio[a0_w : a1_w] in a ragged plan with the same shift row.
+ * The plan reads the windows in place: audio_starts[w] = a0_w (offsets may overlap and need not be aligned),
+ * lengths[w] = a1_w - a0_w, one shift_row of n_shifts delays for every window.  STFT frames are keyed in recording
+ * coordinates and computed once per de-duplication group of group_clips consecutive windows; a sweep takes the plan only
+ * when group_clips divides its chunk.  Checked before any CUDA call: 1 <= n_audio < 2^31 - 4096, 0 <= a0_w < n_audio,
+ * a0_w + lengths[w] <= n_audio, lengths >= 1, the per-window frame limit of the ragged plan, group_clips >= 1.  The
+ * result is an avs_mfcc_ragged_plan (destroy, workspace_bytes and stats_sweep as above). */
+AVS_API int avs_mfcc_ragged_plan_create_windows(int n_windows, int64_t n_audio, const int64_t* audio_starts,
+                                        const int32_t* lengths, int group_clips, int sample_rate, int n_mfcc,
+                                        const int32_t* shift_row, int n_shifts, void* stream,
+                                        avs_mfcc_ragged_plan** out);
+/* Host-only (no device needed): n_frames [n_windows] STFT frames per window, group_unique [ceil(n_windows /
+ * group_clips)] unique frames per group; frames_out (may be NULL) receives sum(group_unique) triples (start, lo, hi) in
+ * recording coordinates, group after group, and map_out (may be NULL) the windows' [n_shifts][n_frames[w]] tables of
+ * group-relative unique-frame ids one after the other. */
+AVS_API int avs_mfcc_ragged_plan_describe_windows(int n_windows, int64_t n_audio, const int64_t* audio_starts,
+                                          const int32_t* lengths, int group_clips, int sample_rate,
+                                          const int32_t* shift_row, int n_shifts, int32_t* n_frames,
+                                          int32_t* group_unique, int32_t* frames_out, int32_t* map_out);
 
 /* ---------------------------------------------------------------- K2: STCNN
  * Replaces extract_visual_embeddings (misalignment_detection_train.py:130-144) == the
@@ -225,6 +252,18 @@ AVS_API int avs_sweep_run_ragged(avs_sweep* sw, const avs_mfcc_ragged_plan* plan
 AVS_API int avs_sweep_run_ragged_u8(avs_sweep* sw, const avs_mfcc_ragged_plan* plan, const uint8_t* frames,
                             const float* audio_packed, int n_clips, float* out_scores, int32_t* out_best,
                             void* stream);
+/* Overlapping windows of one recording (semantics at avs_mfcc_ragged_plan_create_windows): frames device f32 or u8
+ * [T, 50, 100], contiguous; window w is frames [w * stride_frames, w * stride_frames + 75), read in place; audio is the
+ * recording at the windowed plan's sample rate.  n_windows must be the plan's, its n_shifts and n_mfcc the handle's, and
+ * its group_clips must divide the handle's chunk_clips.  Outputs [n_windows] as avs_sweep_run; chunking, streams and
+ * ordering as avs_sweep_run_ragged.  Window w's scores equal, bit for bit, avs_sweep_run_ragged on the cut clip (frames
+ * [t_w, t_w + 75) and audio [a0_w, a1_w)).  A windowed plan is refused by avs_sweep_run_ragged and a ragged one here. */
+AVS_API int avs_sweep_run_windows(avs_sweep* sw, const avs_mfcc_ragged_plan* plan, const float* frames,
+                          int stride_frames, const float* audio, int n_windows, float* out_scores,
+                          int32_t* out_best, void* stream);
+AVS_API int avs_sweep_run_windows_u8(avs_sweep* sw, const avs_mfcc_ragged_plan* plan, const uint8_t* frames,
+                             int stride_frames, const float* audio, int n_windows, float* out_scores,
+                             int32_t* out_best, void* stream);
 /* ---------------------------------------------------------------- decode metrics (SURVEY 8f-3)
  * Edit distances behind calculate_cer / calculate_wer (train.py:945-993) and the positional character
  * matches of evaluate_model (utils.py:83-86) for a batch of id sequences that are already on the device
