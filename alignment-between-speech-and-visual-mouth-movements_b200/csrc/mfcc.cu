@@ -29,6 +29,15 @@ constexpr int kBins = kHalf + 1;      // 1025
 constexpr int kMels = AVS_NMELS;      // 128
 constexpr int kMaxQ = 40;
 
+namespace {
+constexpr int kStatsSmemLimit = 227 * 1024;  // dynamic shared memory of one block on sm_100
+// mfcc_stats_kernel holds the DCT basis and the coefficients of every frame of one shifted signal: (128 + F) * NQ floats
+int max_frames_for(int n_mfcc) {
+  const int nq = n_mfcc <= 20 ? 20 : kMaxQ;
+  return kStatsSmemLimit / (nq * static_cast<int>(sizeof(float))) - kMels;
+}
+}  // namespace
+
 }  // namespace avs
 
 namespace avs {
@@ -645,13 +654,21 @@ extern "C" int avs_mfcc_plan_create(int n_samples, int sample_rate, int n_mfcc, 
   AVS_REQUIRE(out != nullptr && shift_samples != nullptr, "null argument");
   AVS_REQUIRE(n_samples > 0 && sample_rate > 0 && n_shifts > 0, "empty problem");
   AVS_REQUIRE(n_mfcc >= 1 && n_mfcc <= kMaxQ, "n_mfcc must be in [1, 40]");
+  const int hop = std::max(1, sample_rate / 40);  // misalignment_detection_train.py:120
+  const int n_frames = 1 + n_samples / hop;       // center=True: 1 + (n + 2*(n_fft/2) - n_fft) / hop
+  const int max_frames = max_frames_for(n_mfcc);
+  if (n_frames > max_frames) {
+    set_error("mfcc plan: %d samples = %d STFT frames; at n_mfcc = %d the statistics kernel holds at most %d frames "
+              "(%d KB of shared memory)", n_samples, n_frames, n_mfcc, max_frames, kStatsSmemLimit / 1024);
+    return AVS_EINVAL;
+  }
   avs_mfcc_plan* p = new avs_mfcc_plan();
   p->n_samples = n_samples;
   p->sr = sample_rate;
-  p->hop = std::max(1, sample_rate / 40);  // misalignment_detection_train.py:120
+  p->hop = hop;
   p->n_mfcc = n_mfcc;
   p->n_shifts = n_shifts;
-  p->n_frames = 1 + n_samples / p->hop;  // center=True: 1 + (n + 2*(n_fft/2) - n_fft) / hop
+  p->n_frames = n_frames;
 
   std::vector<int4> frames;
   std::vector<int> map;
@@ -839,13 +856,6 @@ struct avs_mfcc_ragged_plan {
 
 namespace avs {
 namespace {
-
-constexpr int kStatsSmemLimit = 227 * 1024;  // dynamic shared memory of one block on sm_100
-// mfcc_stats_kernel holds the DCT basis and the coefficients of every frame of one shifted signal: (128 + F) * NQ floats
-int max_frames_for(int n_mfcc) {
-  const int nq = n_mfcc <= 20 ? 20 : kMaxQ;
-  return kStatsSmemLimit / (nq * static_cast<int>(sizeof(float))) - kMels;
-}
 
 long long floor_div(long long a, long long b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
 

@@ -217,8 +217,8 @@ extern "C" size_t avs_sweep_score_workspace_bytes(int n_clips, int hidden) {
 }
 
 // K slices of the tensor-core form of the hidden-layer GEMM: fixed per K (bit-identical scores whatever the batch), the
-// largest divisor of the k-block count up to 16 — 9 for the detector's 13824 visual dims (432 blocks of 32), i.e. 144
-// CTAs at 1024 clips where the unsplit GEMM has 16 output tiles.
+// largest divisor of the k-block count up to 16 — 16 for the detector's 13824 visual dims (432 blocks of 32, 27 blocks per
+// slice), i.e. 256 CTAs at 1024 clips where the unsplit GEMM has 16 output tiles.
 static int tensor_gemm_splits(int v_dim) {
   const int nk = v_dim / 32;
   int s = 1;

@@ -73,7 +73,10 @@ AVS_API int avs_device_check(int device);
  * Replaces compute_audio_stats(shift_audio(audio, k, fps, sr), sr, n_mfcc)
  * (misalignment_detection_train.py:100-127, librosa.feature.mfcc at :121) for all K shifts
  * of B clips in one call.  shift_samples[k] is the signed integer delay shift_audio applies
- * (:103).  The plan de-duplicates STFT frames shared between shifts on the host. */
+ * (:103).  The plan de-duplicates STFT frames shared between shifts on the host.  n_mfcc in [1, 40]; a clip may have
+ * at most 2777 STFT frames (n_mfcc <= 20; 1324 for n_mfcc up to 40: 1 + n_samples / (sample_rate / 40) frames, about
+ * 69 s / 33 s at 16 kHz), the statistics kernel's shared-memory limit.  A longer clip is rejected with AVS_EINVAL
+ * before any CUDA call. */
 typedef struct avs_mfcc_plan avs_mfcc_plan;
 AVS_API int avs_mfcc_plan_create(int n_samples, int sample_rate, int n_mfcc,
                          const int32_t* shift_samples, int n_shifts, avs_mfcc_plan** out);
