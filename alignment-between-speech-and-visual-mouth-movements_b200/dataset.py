@@ -24,6 +24,20 @@ def create_vocab():
     return char_to_idx, {i: c for c, i in char_to_idx.items()}
 
 
+# The GRID corpus grammar (Cooke et al., 2006): command, colour, preposition, letter (no "w"), digit, adverb.
+GRID_WORDS = (["bin", "lay", "place", "set"] + ["blue", "green", "red", "white"] + ["at", "by", "in", "with"]
+              + [c for c in "abcdefghijklmnopqrstuvxyz"]
+              + ["zero", "one", "two", "three", "four", "five", "six", "seven", "eight", "nine"]
+              + ["again", "now", "please", "soon"])
+
+
+def grid_lexicon():
+    """The 51 GRID words as a ``CtcLexicon`` over ``create_vocab()`` (blank 0, space 37, 39 ids), on the current
+    CUDA device, for ``ctc_beam_decode`` / ``decode_batch`` / ``evaluate_model``."""
+    from .utils import CtcLexicon
+    return CtcLexicon(GRID_WORDS, create_vocab()[0], space=" ")
+
+
 class GridPreprocessor:
     """Decoded uint8 frames -> float32 [B, 1, 75, 50, 100] on the GPU."""
 

@@ -1,8 +1,10 @@
 """`utils.decode_prediction` drop-in (reference: utils.py:8-36) + the batched decode it is built on."""
 from __future__ import annotations
 
-from typing import List, Tuple
+import ctypes
+from typing import Dict, List, Optional, Sequence, Tuple
 
+import numpy as np
 import torch
 
 from . import _native as N
@@ -38,16 +40,83 @@ def decode_prediction(outputs: torch.Tensor, dataset, blank_index: int = 0) -> s
     return ids_to_text(ids[0, :n].tolist(), dataset)
 
 
-def decode_batch(outputs: torch.Tensor, dataset, blank_index: int = 0) -> List[str]:
-    """Decode a whole batch [B,T,V] with one kernel launch and one device->host copy."""
-    ids, lens = ctc_greedy_decode(outputs, blank_index)
+class CtcLexicon:
+    """A word lexicon for ``ctc_beam_decode`` (K5b): the words' character trie, built once and kept on the current CUDA
+    device.  ``words`` are strings over the keys of ``char_to_idx``; ``space`` separates words.  ``vocab`` defaults to
+    the largest id of ``char_to_idx`` plus one; ``blank_index`` must be the blank the log-probs are decoded with."""
+
+    def __init__(self, words: Sequence[str], char_to_idx: Dict[str, int], space: str = " ",
+                 vocab: Optional[int] = None, blank_index: int = 0):
+        ids, offsets = [], [0]
+        for w in words:
+            for ch in w:
+                if ch not in char_to_idx:
+                    raise ValueError(f"lexicon word {w!r} has a character {ch!r} outside char_to_idx")
+                ids.append(char_to_idx[ch])
+            offsets.append(len(ids))
+        self.words = list(words)
+        self.vocab = int(vocab) if vocab is not None else max(char_to_idx.values()) + 1
+        self.blank = int(blank_index)
+        self.space_id = char_to_idx[space]
+        self.device = torch.device("cuda", torch.cuda.current_device())
+        N.device_check()
+        w_ids = np.asarray(ids if ids else [0], dtype=np.int32)
+        w_off = np.asarray(offsets, dtype=np.int32)
+        h = ctypes.c_void_p()
+        N.check(N.lib().avs_ctc_lexicon_create(w_ids.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)),
+                                               w_off.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)), len(self.words),
+                                               self.vocab, self.blank, self.space_id, N.stream_ptr(), ctypes.byref(h)),
+                "ctc_lexicon_create")
+        self._handle = N.Handle(h, N.lib().avs_ctc_lexicon_destroy)
+
+    @property
+    def handle(self) -> ctypes.c_void_p:
+        return self._handle.h
+
+
+def ctc_beam_decode(logp: torch.Tensor, beam_width: int, top_n: int = 1, blank_index: int = 0,
+                    lexicon: Optional[CtcLexicon] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Batched CTC prefix beam search (K5b), optionally constrained to a ``CtcLexicon``.  logp [B,T,V] CUDA log-probs
+    (NaN counts as -inf) -> (ids int32 [B, top_n, T] padded with -1, lengths int32 [B, top_n], scores f32 [B, top_n]),
+    best first, on the device.  A score is the log-probability of its label sequence summed over the alignments the
+    search kept.  With a lexicon only complete texts (words of the lexicon joined by single spaces, or the empty text)
+    are returned; a slot with no hypothesis has score -inf and length 0.  One launch, no host sync.
+    Limits: 1 <= beam_width <= 128, 1 <= top_n <= beam_width, 2 <= V <= 64, 1 <= T <= 1024."""
+    N.require_cuda(logp, "logp")
+    if logp.dim() != 3:
+        raise ValueError("logp must be [B, T, V]")
+    logp = N.f32c(logp)
+    B, T, V = logp.shape
+    if lexicon is not None and lexicon.device != logp.device:
+        raise ValueError(f"the lexicon lives on {lexicon.device}, logp on {logp.device}")
+    ids = torch.empty((B, top_n, T), dtype=torch.int32, device=logp.device)
+    lens = torch.empty((B, top_n), dtype=torch.int32, device=logp.device)
+    scores = torch.empty((B, top_n), dtype=torch.float32, device=logp.device)
+    L = N.lib()
+    ws = N.workspace(L.avs_ctc_beam_workspace_bytes(B, T, int(beam_width)), logp.device)
+    N.check(L.avs_ctc_beam(N.ptr(logp), B, T, V, int(blank_index), int(beam_width), int(top_n),
+                           lexicon.handle if lexicon is not None else None, N.ptr(ids), N.ptr(lens), N.ptr(scores),
+                           N.ptr(ws), ws.numel(), N.stream_ptr()), "ctc_beam")
+    return ids, lens, scores
+
+
+def decode_batch(outputs: torch.Tensor, dataset, blank_index: int = 0, beam_width: Optional[int] = None,
+                 lexicon: Optional[CtcLexicon] = None) -> List[str]:
+    """Decode a whole batch [B,T,V] with one kernel launch and one device->host copy: greedy (K5) by default, the top
+    hypothesis of ``ctc_beam_decode`` (K5b) when ``beam_width`` is given."""
+    if beam_width is None:
+        ids, lens = ctc_greedy_decode(outputs, blank_index)
+    else:
+        ids, lens, _ = ctc_beam_decode(outputs, beam_width, 1, blank_index, lexicon)
+        ids, lens = ids[:, 0], lens[:, 0]
     ids_h, lens_h = ids.cpu().tolist(), lens.cpu().tolist()
     return [ids_to_text(row[:n], dataset) for row, n in zip(ids_h, lens_h)]
 
 
-def evaluate_model(model, test_loader, dataset, device, num_samples=5, verbose=True):
+def evaluate_model(model, test_loader, dataset, device, num_samples=5, verbose=True, beam_width=None, lexicon=None):
     """Reference utils.py:38-86 — forward, decode, naive positional character accuracy for the first
-    ``num_samples`` items.  One batched decode (K5) per batch instead of one device sync per sample.
+    ``num_samples`` items.  One batched decode (K5) per batch instead of one device sync per sample; with
+    ``beam_width`` the decode is ``ctc_beam_decode`` (K5b, optionally with ``lexicon``).
     Prints the reference's lines when ``verbose`` and returns [(true_text, predicted_text, accuracy %)]."""
     model.eval()
     model.to(device)
@@ -60,7 +129,7 @@ def evaluate_model(model, test_loader, dataset, device, num_samples=5, verbose=T
             if i >= num_samples:
                 break
             outputs = model(videos.to(device))
-            texts = decode_batch(outputs, dataset)
+            texts = decode_batch(outputs, dataset, beam_width=beam_width, lexicon=lexicon)
             for j in range(videos.size(0)):
                 n = i * test_loader.batch_size + j
                 if n >= num_samples:

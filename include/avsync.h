@@ -218,6 +218,39 @@ AVS_API int avs_sweep_score(const float* vstats, const float* astats, int n_clip
 AVS_API int avs_ctc_greedy(const float* logp, int n_clips, int n_steps, int vocab, int blank,
                    int32_t* out_ids, int32_t* out_len, void* stream);
 
+/* ---------------------------------------------------------------- K5b: CTC prefix beam search
+ * Prefix beam search in log space, one CTA per clip.  A hypothesis is a label prefix y with lp_b (ending in blank) and
+ * lp_nb (ending in its last label e), score(y) = logaddexp(lp_b, lp_nb); the search starts from the empty prefix
+ * (lp_b = 0, lp_nb = -inf).  Step t: stay  lp_b' = score(y) + lp[t,blank], lp_nb' = lp_nb(y) + lp[t,e] (y non-empty);
+ * extend by c != blank  lp_nb' = (c == e ? lp_b(y) : score(y)) + lp[t,c], lp_b' = -inf.  Candidates of the same prefix
+ * are merged exactly (their lp_b and lp_nb log-added): prefixes are nodes of a per-clip trie in the workspace, found
+ * through an open-addressing table with exact (parent node, label) keys.  Candidate (r, c): r = rank of the source beam,
+ * c = -1 for the stay, then the labels in increasing order; a merged candidate takes the smaller index.  The beam_width
+ * best survive, ordered by (score descending, index ascending); candidates of score -inf are dropped.  A NaN log-prob
+ * counts as -inf.  A clip's outputs do not depend on the rest of the batch.
+ *
+ * Lexicon: a character trie of words (word w = word_ids[word_offsets[w] : word_offsets[w+1]], word_offsets[0] = 0).  An
+ * extension by a non-space label needs that child in the hypothesis' lexicon state; space_id is allowed only at a word
+ * end and returns to the root, so a space can neither start the text nor follow a space.  At the last step only complete
+ * hypotheses (at a word end, or empty) are returned.  Creation checks, before any CUDA call: n_words >= 1, 2 <= vocab
+ * <= 64, 0 <= blank < vocab, space_id < vocab and != blank, every word non-empty with ids < vocab that are neither the
+ * blank nor space_id; it then uploads its table with a stream-ordered allocation and copy on `stream`.  destroy waits
+ * for the device. */
+typedef struct avs_ctc_lexicon avs_ctc_lexicon;
+AVS_API int avs_ctc_lexicon_create(const int32_t* word_ids, const int32_t* word_offsets, int n_words, int vocab,
+                                   int blank, int space_id, void* stream, avs_ctc_lexicon** out);
+AVS_API void avs_ctc_lexicon_destroy(avs_ctc_lexicon* lex);
+/* 0 for arguments outside the limits below */
+AVS_API size_t avs_ctc_beam_workspace_bytes(int n_clips, int n_steps, int beam_width);
+/* logp f32 [n_clips, n_steps, vocab]; out_ids i32 [n_clips, top_n, n_steps] (first out_len entries valid, rest -1);
+ * out_len i32 [n_clips, top_n]; out_score f32 [n_clips, top_n], best first; lexicon may be NULL (it must have been built
+ * for this vocab and blank).  An output slot with no hypothesis gets score -inf and length 0.  Checked before any CUDA
+ * call: 1 <= beam_width <= 128, 1 <= top_n <= beam_width, 2 <= vocab <= 64, 0 <= blank < vocab, 1 <= n_steps <= 1024,
+ * n_clips >= 0.  No host or device synchronisation. */
+AVS_API int avs_ctc_beam(const float* logp, int n_clips, int n_steps, int vocab, int blank, int beam_width, int top_n,
+                         const avs_ctc_lexicon* lexicon, int32_t* out_ids, int32_t* out_len, float* out_score,
+                         void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------- whole sweep (K2 + K1 + K4)
  * The composed +-S sync sweep of SURVEY.md §3.2: for each clip, visual stats once, audio stats
  * per shift, detector score per shift, arg-max.  The handle owns its device workspace, two
