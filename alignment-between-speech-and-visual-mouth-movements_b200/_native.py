@@ -73,6 +73,8 @@ SIGNATURES = {
     "avs_ctc_lexicon_destroy": (None, [_P]),
     "avs_ctc_beam_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "avs_ctc_beam": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P, c_size_t, _P]),
+    "avs_ctc_align_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "avs_ctc_align": (c_int, [_P, c_int, c_int, c_int, c_int, _P, _P, c_int, _P, _P, _P, _P, _P, _P, _P, c_size_t, _P]),
     "avs_edit_metrics": (c_int, [_P, _P, c_int, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P]),
     "avs_preproc_create": (c_int, [c_int, c_int, c_int, POINTER(_P)]),
     "avs_preproc_destroy": (None, [_P]),

@@ -1,11 +1,11 @@
 """GPU pre-processing prologue for the path (SURVEY.md section 8f-2): the per-frame arithmetic of the
 reference's ``GridDataset.process_video`` (dataset.py:176-256) — gray, mouth crop, bilinear resize to
 100x50, /255, pad/truncate to 75 frames — as one kernel, bit-exact with OpenCV's 8-bit paths.
-Directory discovery, ``.align`` parsing and video DECODING stay on the host (file / codec IO)."""
+Directory discovery, ``.align`` parsing (``read_grid_align``) and video DECODING stay on the host (file / codec IO)."""
 from __future__ import annotations
 
 import ctypes
-from typing import Dict, Optional, Sequence
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -36,6 +36,25 @@ def grid_lexicon():
     CUDA device, for ``ctc_beam_decode`` / ``decode_batch`` / ``evaluate_model``."""
     from .utils import CtcLexicon
     return CtcLexicon(GRID_WORDS, create_vocab()[0], space=" ")
+
+
+def read_grid_align(path: str) -> Tuple[str, List[Tuple[str, float, float]]]:
+    """A GRID ``.align`` file -> (text, [(word, start_frame, end_frame)]).  Each line is ``start end word`` with times in
+    units of 1/25 000 s, i.e. 1 000 per video frame at 25 fps; frames are those times / 1000, as LipNet's reader divides
+    them (GRID boundaries need not fall on frame boundaries).  The silence markers ``sil`` and ``sp`` are dropped;
+    ``text`` is the remaining words joined by single spaces, the transcript ``align_words`` takes."""
+    words = []
+    with open(path) as f:
+        for line in f:
+            parts = line.split()
+            if not parts:
+                continue
+            if len(parts) != 3:
+                raise ValueError(f"{path}: expected 'start end word', got {line.strip()!r}")
+            start, end, word = parts
+            if word not in ("sil", "sp"):
+                words.append((word, int(start) / 1000.0, int(end) / 1000.0))
+    return " ".join(w for w, _, _ in words), words
 
 
 class GridPreprocessor:

@@ -1,8 +1,9 @@
-"""`utils.decode_prediction` drop-in (reference: utils.py:8-36) + the batched decode it is built on."""
+"""`utils.decode_prediction` drop-in (reference: utils.py:8-36) + the batched decode it is built on, and CTC forced
+alignment of known transcripts."""
 from __future__ import annotations
 
 import ctypes
-from typing import Dict, List, Optional, Sequence, Tuple
+from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -98,6 +99,107 @@ def ctc_beam_decode(logp: torch.Tensor, beam_width: int, top_n: int = 1, blank_i
                            lexicon.handle if lexicon is not None else None, N.ptr(ids), N.ptr(lens), N.ptr(scores),
                            N.ptr(ws), ws.numel(), N.stream_ptr()), "ctc_beam")
     return ids, lens, scores
+
+
+class CtcAlignment(NamedTuple):
+    """``ctc_forced_align`` outputs, on the device.  Per clip b, along the best (Viterbi) alignment:
+    loglik f32 [B] log p(target | logp) over all alignments (= -ctc_loss); path_score f32 [B] the best alignment's
+    log-probability; frame_token i32 [B, T] the target position each frame emits (-1 blank, -2 at or past input_len);
+    span i32 [B, Lmax, 2] each token's first frame and end frame (exclusive), -1 past the target; token_prob f32
+    [B, Lmax] the mean of exp(logp[t, token]) over the token's frames, NaN past the target.  An invalid clip (an id
+    outside [0, V) or equal to the blank, a length out of range) has NaN scores; a clip without an alignment of
+    non-zero probability has -inf scores; both have frame_token -2, span -1 and token_prob NaN."""
+    loglik: torch.Tensor
+    path_score: torch.Tensor
+    frame_token: torch.Tensor
+    span: torch.Tensor
+    token_prob: torch.Tensor
+
+
+def _i32_on(t: torch.Tensor, device) -> torch.Tensor:
+    return t.to(device=device, dtype=torch.int32).contiguous()
+
+
+def ctc_forced_align(logp: torch.Tensor, targets: torch.Tensor, target_lens: torch.Tensor,
+                     input_lens: Optional[torch.Tensor] = None, blank_index: int = 0) -> CtcAlignment:
+    """Batched CTC forced alignment (K5c) of known targets.  logp [B,T,V] CUDA log-probs (NaN counts as -inf);
+    targets [B, Lmax] padded label ids and target_lens [B], the layout ``ctc_loss`` and the GRID ``collate_fn`` use;
+    input_lens [B] valid frames per clip (default T).  Returns a ``CtcAlignment`` of device tensors.  One launch and no
+    host sync when the index tensors are int32 on logp's device (others are converted first).
+    Limits: 1 <= T <= 1024, 2 <= V <= 64, 0 <= Lmax <= 512."""
+    N.require_cuda(logp, "logp")
+    if logp.dim() != 3:
+        raise ValueError("logp must be [B, T, V]")
+    logp = N.f32c(logp)
+    B, T, V = logp.shape
+    dev = logp.device
+    if targets.dim() != 2 or targets.shape[0] != B:
+        raise ValueError(f"targets must be [B={B}, Lmax], got {tuple(targets.shape)}")
+    if tuple(target_lens.shape) != (B,) or (input_lens is not None and tuple(input_lens.shape) != (B,)):
+        raise ValueError(f"target_lens and input_lens must be [B={B}]")
+    Lmax = targets.shape[1]
+    targets, target_lens = _i32_on(targets, dev), _i32_on(target_lens, dev)
+    input_lens = _i32_on(input_lens, dev) if input_lens is not None else None
+    out = CtcAlignment(torch.empty((B,), dtype=torch.float32, device=dev),
+                       torch.empty((B,), dtype=torch.float32, device=dev),
+                       torch.empty((B, T), dtype=torch.int32, device=dev),
+                       torch.empty((B, Lmax, 2), dtype=torch.int32, device=dev),
+                       torch.empty((B, Lmax), dtype=torch.float32, device=dev))
+    L = N.lib()
+    ws = N.workspace(L.avs_ctc_align_workspace_bytes(B, T, Lmax), dev)
+    N.check(L.avs_ctc_align(N.ptr(logp), B, T, V, int(blank_index), N.ptr(input_lens), N.ptr(targets), Lmax,
+                            N.ptr(target_lens), *(N.ptr(t) for t in out), N.ptr(ws), ws.numel(), N.stream_ptr()),
+            "ctc_align")
+    return out
+
+
+def align_words(logp: torch.Tensor, texts: Sequence[str], char_to_idx: Optional[Dict[str, int]] = None,
+                fps: float = 25.0, space: str = " ", blank_index: int = 0, input_lens: Optional[torch.Tensor] = None
+                ) -> List[Tuple[List[Tuple[str, float, float, float]], float]]:
+    """Word timings of known transcripts in LipNet log-probs [B,T,V]: ``texts[b]`` is aligned to clip b with
+    ``ctc_forced_align`` (one upload of the targets, one copy of the results back).  Returns per clip
+    ``(words, loglik)``; ``words`` lists ``(word, start_s, end_s, score)`` for every maximal run of non-space
+    characters: from its first character's first frame to its last character's end frame, over ``fps``, scored by the
+    mean ``token_prob`` of its characters.  A clip without an alignment (loglik -inf, or NaN for an invalid clip)
+    keeps its words with NaN times and scores.  ``char_to_idx`` defaults to the GRID vocabulary (``create_vocab``); a
+    character outside it raises ``ValueError``."""
+    if char_to_idx is None:
+        from .dataset import create_vocab
+        char_to_idx = create_vocab()[0]
+    if len(texts) != logp.shape[0]:
+        raise ValueError(f"{len(texts)} texts for {logp.shape[0]} clips")
+    B = len(texts)
+    for s in texts:
+        for ch in s:
+            if ch not in char_to_idx:
+                raise ValueError(f"character {ch!r} of {s!r} is outside char_to_idx")
+    Lmax = max((len(s) for s in texts), default=0)
+    host = np.zeros(B * Lmax + B, dtype=np.int32)      # targets [B, Lmax], then target_lens [B]: one upload
+    for b, s in enumerate(texts):
+        host[b * Lmax:b * Lmax + len(s)] = [char_to_idx[ch] for ch in s]
+        host[B * Lmax + b] = len(s)
+    dev = torch.from_numpy(host).to(logp.device)
+    al = ctc_forced_align(logp, dev[:B * Lmax].view(B, Lmax), dev[B * Lmax:], input_lens, blank_index)
+    packed = torch.cat([al.span.view(B, 2 * Lmax), al.token_prob.view(torch.int32),
+                        al.loglik.view(torch.int32).view(B, 1)], dim=1).cpu().numpy()   # one copy back
+    span = packed[:, :2 * Lmax].reshape(B, Lmax, 2)
+    prob = packed[:, 2 * Lmax:3 * Lmax].view(np.float32)
+    loglik = packed[:, 3 * Lmax].view(np.float32)
+    out = []
+    for b, s in enumerate(texts):
+        ok = np.isfinite(loglik[b])
+        words, k = [], 0
+        for w in s.split(space):
+            if w:
+                a, e = k, k + len(w)
+                if ok:
+                    words.append((w, float(span[b, a, 0]) / fps, float(span[b, e - 1, 1]) / fps,
+                                  float(prob[b, a:e].astype(np.float64).mean())))
+                else:
+                    words.append((w, float("nan"), float("nan"), float("nan")))
+            k += len(w) + len(space)
+        out.append((words, float(loglik[b])))
+    return out
 
 
 def decode_batch(outputs: torch.Tensor, dataset, blank_index: int = 0, beam_width: Optional[int] = None,

@@ -251,6 +251,43 @@ AVS_API int avs_ctc_beam(const float* logp, int n_clips, int n_steps, int vocab,
                          const avs_ctc_lexicon* lexicon, int32_t* out_ids, int32_t* out_len, float* out_score,
                          void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---------------------------------------------------------------- K5c: CTC forced alignment
+ * Aligns a known target y (L labels) to a clip's log-probs, one CTA per clip.  The lattice is the extended target
+ * blank, y0, blank, y1, ..., blank: S = 2L + 1 states, state s carries label(s) = y[s/2] when s is odd, the blank when
+ * it is even.  One pass over the clip's first n = input_len frames runs, in fp64:
+ *   forward  a[t][s] = logsumexp(a[t-1][s], a[t-1][s-1], a[t-1][s-2]) + lp[t][label(s)];
+ *   Viterbi  v[t][s] = max(v[t-1][s], v[t-1][s-1], v[t-1][s-2]) + lp[t][label(s)],
+ * from a[0] = v[0] = (lp[0][blank], lp[0][y0], -inf, ...); the s-2 term applies only when label(s) is not the blank and
+ * differs from label(s-2).  loglik = logsumexp(a[n-1][S-1], a[n-1][S-2]) = log p(y | x) over all alignments
+ * (= -ctc_loss, reduction "none"); path_score = max(v[n-1][S-1], v[n-1][S-2]) is the log-probability of the best
+ * alignment.  Viterbi ties go to the stay s, then to s-1, then to s-2; at the end the trailing blank S-1 wins a tie
+ * against the last token S-2.  A NaN log-prob counts as -inf.  The Viterbi adds are correctly rounded fp64 adds in
+ * time order, so a float64 restatement that adds in the same order takes the same decisions and gets the same bits.
+ * Outputs per clip, along the best alignment:
+ *   frame_token[t]  the target position k whose label frame t emits, -1 for a blank frame, -2 for t >= input_len;
+ *   span[k]         {first frame, end frame (exclusive)} of token k; {-1, -1} for k >= L;
+ *   token_prob[k]   the mean of exp(lp[t][y_k]) over the frames of token k (torchaudio's merge_tokens); NaN for k >= L.
+ * Per-clip status; the other clips of the batch are unaffected:
+ *   invalid: an id of y outside [0, vocab) or equal to the blank, target_len outside [0, target_stride], or input_len
+ *            outside [0, n_steps].  loglik and path_score are NaN, frame_token -2, span -1, token_prob NaN.
+ *   no alignment of non-zero probability (input too short for y, or the log-probs it needs are -inf or NaN): loglik and
+ *            path_score are -inf, the rest as for an invalid clip.
+ *   input_len = 0 aligns the empty target only: loglik = path_score = 0 with L = 0. */
+/* Bytes of device workspace avs_ctc_align needs: the Viterbi backpointers, one byte per (frame, state), when a clip's
+ * n_steps * (2 * max_target_len + 1) exceeds 32 KB; below that they live in shared memory and this is 0.  Also 0
+ * outside the limits of avs_ctc_align. */
+AVS_API size_t avs_ctc_align_workspace_bytes(int n_clips, int n_steps, int max_target_len);
+/* logp f32 [n_clips, n_steps, vocab]; input_len i32 [n_clips] (NULL = n_steps for every clip); targets i32 [n_clips,
+ * target_stride], the first target_len[b] entries of row b are its target; target_len i32 [n_clips].  out_loglik,
+ * out_path_score f32 [n_clips]; out_frame_token i32 [n_clips, n_steps]; out_span i32 [n_clips, target_stride, 2];
+ * out_token_prob f32 [n_clips, target_stride] (targets, out_span and out_token_prob may be NULL when target_stride is 0).
+ * Checked before any CUDA call: 1 <= n_steps <= 1024, 2 <= vocab <= 64, 0 <= blank < vocab, 0 <= target_stride <= 512,
+ * n_clips >= 0, the workspace size.  No host or device synchronisation. */
+AVS_API int avs_ctc_align(const float* logp, int n_clips, int n_steps, int vocab, int blank, const int32_t* input_len,
+                          const int32_t* targets, int target_stride, const int32_t* target_len, float* out_loglik,
+                          float* out_path_score, int32_t* out_frame_token, int32_t* out_span, float* out_token_prob,
+                          void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------- whole sweep (K2 + K1 + K4)
  * The composed +-S sync sweep of SURVEY.md §3.2: for each clip, visual stats once, audio stats
  * per shift, detector score per shift, arg-max.  The handle owns its device workspace, two
