@@ -10,7 +10,8 @@ error behaviour) over the C-ABI library ``libavsync_b200.so`` (``include/avsync.
         load_lipnet, save_detector}                  utils.evaluate_model
     misalignment_detection_train.{SyncSweeper, sync_sweep, audio_stats_sweep_ragged, audio_stats_sweep_windows,
         window_bounds}, utils.{ctc_greedy_decode, ctc_beam_decode, CtcLexicon, ctc_forced_align, CtcAlignment,
-        align_words}, dataset.{GRID_WORDS, grid_lexicon, read_grid_align}                        (new, batched)
+        align_words, ctc_grammar_decode, CtcGrammar, CtcGrammarResult}, dataset.{GRID_WORDS, GRID_SLOTS, grid_lexicon,
+        grid_grammar, read_grid_align}                                                             (new, batched)
     distributed.{shard_range, sweep_sharded, gather_scores, ddp_detector_step, GraphedDetectorStep}        (new, multi-GPU)
 
 Import as ``avsync_b200`` (the directory name is not a valid identifier; ``avsync_b200.py`` at the
@@ -18,8 +19,9 @@ repo root aliases it).
 """
 from . import _native
 from .model import LipNet
-from .utils import (CtcAlignment, CtcLexicon, align_words, ctc_beam_decode, ctc_forced_align, ctc_greedy_decode,
-                    decode_batch, decode_metrics, decode_prediction, evaluate_model)
+from .utils import (CtcAlignment, CtcGrammar, CtcGrammarResult, CtcLexicon, align_words, ctc_beam_decode,
+                    ctc_forced_align, ctc_grammar_decode, ctc_greedy_decode, decode_batch, decode_metrics,
+                    decode_prediction, evaluate_model)
 from .misalignment_detection_train import (DetectorConfig, FeatureExtractor, MisalignmentDataset, MisalignmentDetector,
                                            SyncSweeper, run_epoch,
                                            audio_stats_sweep, audio_stats_sweep_ragged, audio_stats_sweep_windows, compute_audio_stats,
@@ -27,7 +29,7 @@ from .misalignment_detection_train import (DetectorConfig, FeatureExtractor, Mis
                                            load_detector, load_lipnet, save_detector, shift_audio, shift_samples, get_video_fps,
                                            resample_audio, default_audio_loader,
                                            sweep_score, sync_sweep, visual_stats)
-from .dataset import GRID_WORDS, GridPreprocessor, grid_lexicon, read_grid_align
+from .dataset import GRID_SLOTS, GRID_WORDS, GridPreprocessor, grid_grammar, grid_lexicon, read_grid_align
 from . import distributed
 
 __all__ = ["LipNet", "ctc_greedy_decode", "decode_batch", "decode_prediction", "DetectorConfig", "FeatureExtractor",
@@ -35,4 +37,5 @@ __all__ = ["LipNet", "ctc_greedy_decode", "decode_batch", "decode_prediction", "
            "extract_visual_embeddings", "load_detector", "load_lipnet", "save_detector", "shift_audio",
            "shift_samples", "get_video_fps", "resample_audio", "default_audio_loader", "sweep_score", "sync_sweep", "visual_stats", "GridPreprocessor", "distributed",
            "CtcLexicon", "ctc_beam_decode", "GRID_WORDS", "grid_lexicon",
-           "CtcAlignment", "ctc_forced_align", "align_words", "read_grid_align"]
+           "CtcAlignment", "ctc_forced_align", "align_words", "read_grid_align",
+           "CtcGrammar", "CtcGrammarResult", "ctc_grammar_decode", "GRID_SLOTS", "grid_grammar"]

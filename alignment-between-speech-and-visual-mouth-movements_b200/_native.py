@@ -75,6 +75,11 @@ SIGNATURES = {
     "avs_ctc_beam": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P, c_size_t, _P]),
     "avs_ctc_align_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "avs_ctc_align": (c_int, [_P, c_int, c_int, c_int, c_int, _P, _P, c_int, _P, _P, _P, _P, _P, _P, _P, c_size_t, _P]),
+    "avs_ctc_grammar_create": (c_int, [POINTER(c_int32), POINTER(c_int32), POINTER(c_int32), c_int, c_int, c_int, c_int,
+                                       _P, POINTER(_P)]),
+    "avs_ctc_grammar_destroy": (None, [_P]),
+    "avs_ctc_grammar_workspace_bytes": (c_size_t, [_P, c_int, c_int]),
+    "avs_ctc_grammar_decode": (c_int, [_P, _P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, _P, c_size_t, _P]),
     "avs_edit_metrics": (c_int, [_P, _P, c_int, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P]),
     "avs_preproc_create": (c_int, [c_int, c_int, c_int, POINTER(_P)]),
     "avs_preproc_destroy": (None, [_P]),

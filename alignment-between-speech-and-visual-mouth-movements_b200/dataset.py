@@ -25,10 +25,11 @@ def create_vocab():
 
 
 # The GRID corpus grammar (Cooke et al., 2006): command, colour, preposition, letter (no "w"), digit, adverb.
-GRID_WORDS = (["bin", "lay", "place", "set"] + ["blue", "green", "red", "white"] + ["at", "by", "in", "with"]
-              + [c for c in "abcdefghijklmnopqrstuvxyz"]
-              + ["zero", "one", "two", "three", "four", "five", "six", "seven", "eight", "nine"]
-              + ["again", "now", "please", "soon"])
+GRID_SLOTS = [["bin", "lay", "place", "set"], ["blue", "green", "red", "white"], ["at", "by", "in", "with"],
+              [c for c in "abcdefghijklmnopqrstuvxyz"],
+              ["zero", "one", "two", "three", "four", "five", "six", "seven", "eight", "nine"],
+              ["again", "now", "please", "soon"]]
+GRID_WORDS = sum(GRID_SLOTS, [])
 
 
 def grid_lexicon():
@@ -36,6 +37,14 @@ def grid_lexicon():
     CUDA device, for ``ctc_beam_decode`` / ``decode_batch`` / ``evaluate_model``."""
     from .utils import CtcLexicon
     return CtcLexicon(GRID_WORDS, create_vocab()[0], space=" ")
+
+
+def grid_grammar():
+    """The GRID grammar, six slots of ``GRID_SLOTS`` (64 000 sentences), as a ``CtcGrammar`` over ``create_vocab()``
+    (blank 0, space 37, 39 ids), on the current CUDA device, for ``ctc_grammar_decode`` / ``decode_batch`` /
+    ``evaluate_model``."""
+    from .utils import CtcGrammar
+    return CtcGrammar(GRID_SLOTS, create_vocab()[0], space=" ")
 
 
 def read_grid_align(path: str) -> Tuple[str, List[Tuple[str, float, float]]]:

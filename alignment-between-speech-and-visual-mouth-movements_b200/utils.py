@@ -1,5 +1,5 @@
-"""`utils.decode_prediction` drop-in (reference: utils.py:8-36) + the batched decode it is built on, and CTC forced
-alignment of known transcripts."""
+"""`utils.decode_prediction` drop-in (reference: utils.py:8-36) + the batched decode it is built on, exact decoding
+under a word-slot grammar, and CTC forced alignment of known transcripts."""
 from __future__ import annotations
 
 import ctypes
@@ -202,10 +202,119 @@ def align_words(logp: torch.Tensor, texts: Sequence[str], char_to_idx: Optional[
     return out
 
 
+class CtcGrammar:
+    """A word-slot grammar for ``ctc_grammar_decode`` (K5d): ``slots[g]`` lists the words of slot g, and a sentence is
+    one word of each slot, in slot order, joined by single spaces.  Its lattice tables are built once and kept on the
+    current CUDA device.  Words are strings over the keys of ``char_to_idx`` (a character outside raises
+    ``ValueError``); ``space`` separates words.  ``vocab`` defaults to the largest id of ``char_to_idx`` plus one;
+    ``blank_index`` must be the blank the log-probs are decoded with.  Limits (checked natively): 1-16 slots, 1-255
+    distinct words per slot, 1-64 characters per word, at most 2 048 lattice states (the sum of 2·len + 1 over the words,
+    plus one per slot boundary)."""
+
+    def __init__(self, slots: Sequence[Sequence[str]], char_to_idx: Dict[str, int], space: str = " ",
+                 vocab: Optional[int] = None, blank_index: int = 0):
+        ids, w_off, s_off = [], [0], [0]
+        for words in slots:
+            for w in words:
+                for ch in w:
+                    if ch not in char_to_idx:
+                        raise ValueError(f"grammar word {w!r} has a character {ch!r} outside char_to_idx")
+                    ids.append(char_to_idx[ch])
+                w_off.append(len(ids))
+            s_off.append(len(w_off) - 1)
+        self.slots = [list(words) for words in slots]
+        self.space = space
+        self.vocab = int(vocab) if vocab is not None else max(char_to_idx.values()) + 1
+        self.blank = int(blank_index)
+        self.space_id = char_to_idx[space]
+        self.device = torch.device("cuda", torch.cuda.current_device())
+        N.device_check()
+        arrs = [np.asarray(a if a else [0], dtype=np.int32) for a in (ids, w_off, s_off)]
+        p = [a.ctypes.data_as(ctypes.POINTER(ctypes.c_int32)) for a in arrs]
+        h = ctypes.c_void_p()
+        N.check(N.lib().avs_ctc_grammar_create(p[0], p[1], p[2], len(self.slots), self.vocab, self.blank,
+                                               self.space_id, N.stream_ptr(), ctypes.byref(h)), "ctc_grammar_create")
+        self._handle = N.Handle(h, N.lib().avs_ctc_grammar_destroy)
+
+    @property
+    def handle(self) -> ctypes.c_void_p:
+        return self._handle.h
+
+    @property
+    def n_words(self) -> int:
+        return sum(len(words) for words in self.slots)
+
+    def texts(self, words) -> List[str]:
+        """Word indices [B, G] (``CtcGrammarResult.words`` or ``mbr_words``, a tensor or an array) -> one sentence per
+        clip; a clip without a decode (indices -1) gives the empty string."""
+        rows = words.tolist() if hasattr(words, "tolist") else list(words)
+        return ["" if any(i < 0 for i in row) else self.space.join(s[i] for s, i in zip(self.slots, row))
+                for row in rows]
+
+
+class CtcGrammarResult(NamedTuple):
+    """``ctc_grammar_decode`` outputs, on the device.  Per clip b: words i32 [B, G] the word index within each slot along
+    the best path; span i32 [B, G, 2] each of those words' first frame and end frame (exclusive), from its first to its
+    last character frame; path_score f32 [B] the best path's log-probability; loglik f32 [B] log of the summed
+    probability of every sentence of the grammar; posterior f32 [B, W] P(slot g = w) for every word, in grammar order;
+    mbr_words i32 [B, G] the per-slot arg-max of posterior (the lowest index on a tie), the decode that minimises the
+    expected number of word errors.  A clip whose input length is out of range has NaN scores; one without a path of
+    non-zero probability has -inf scores; both have words, span and mbr_words -1 and posterior NaN."""
+    words: torch.Tensor
+    span: torch.Tensor
+    path_score: torch.Tensor
+    loglik: torch.Tensor
+    posterior: torch.Tensor
+    mbr_words: torch.Tensor
+
+
+def ctc_grammar_decode(logp: torch.Tensor, grammar: CtcGrammar, input_lens: Optional[torch.Tensor] = None,
+                       blank_index: int = 0) -> CtcGrammarResult:
+    """Exact CTC decoding (K5d) of log-probs [B,T,V] (CUDA; NaN counts as -inf) over every sentence of a ``CtcGrammar``:
+    the best sentence (Viterbi) with its word spans, the grammar's log-likelihood and every word's posterior.
+    input_lens [B] valid frames per clip (default T).  One launch and no host sync when input_lens is int32 on logp's
+    device (otherwise it is converted first).  Limits: 1 <= T <= 1024, V equal to the grammar's vocab."""
+    N.require_cuda(logp, "logp")
+    if logp.dim() != 3:
+        raise ValueError("logp must be [B, T, V]")
+    if int(blank_index) != grammar.blank:
+        raise ValueError(f"the grammar was built for blank {grammar.blank}, not {blank_index}")
+    logp = N.f32c(logp)
+    B, T, V = logp.shape
+    dev = logp.device
+    if grammar.device != dev:
+        raise ValueError(f"the grammar lives on {grammar.device}, logp on {dev}")
+    if input_lens is not None:
+        if tuple(input_lens.shape) != (B,):
+            raise ValueError(f"input_lens must be [B={B}]")
+        input_lens = _i32_on(input_lens, dev)
+    G, W = len(grammar.slots), grammar.n_words
+    out = CtcGrammarResult(torch.empty((B, G), dtype=torch.int32, device=dev),
+                           torch.empty((B, G, 2), dtype=torch.int32, device=dev),
+                           torch.empty((B,), dtype=torch.float32, device=dev),
+                           torch.empty((B,), dtype=torch.float32, device=dev),
+                           torch.empty((B, W), dtype=torch.float32, device=dev),
+                           torch.empty((B, G), dtype=torch.int32, device=dev))
+    L = N.lib()
+    ws = N.workspace(L.avs_ctc_grammar_workspace_bytes(grammar.handle, B, T), dev)
+    N.check(L.avs_ctc_grammar_decode(grammar.handle, N.ptr(logp), B, T, V, N.ptr(input_lens), *(N.ptr(t) for t in out),
+                                     N.ptr(ws), ws.numel(), N.stream_ptr()), "ctc_grammar_decode")
+    return out
+
+
+def _check_decoder(beam_width, lexicon, grammar) -> None:
+    if grammar is not None and (beam_width is not None or lexicon is not None):
+        raise ValueError("grammar decodes exactly: it cannot be combined with beam_width or lexicon")
+
+
 def decode_batch(outputs: torch.Tensor, dataset, blank_index: int = 0, beam_width: Optional[int] = None,
-                 lexicon: Optional[CtcLexicon] = None) -> List[str]:
+                 lexicon: Optional[CtcLexicon] = None, grammar: Optional[CtcGrammar] = None) -> List[str]:
     """Decode a whole batch [B,T,V] with one kernel launch and one device->host copy: greedy (K5) by default, the top
-    hypothesis of ``ctc_beam_decode`` (K5b) when ``beam_width`` is given."""
+    hypothesis of ``ctc_beam_decode`` (K5b) when ``beam_width`` is given, the best sentence of ``grammar`` by
+    ``ctc_grammar_decode`` (K5d) when a grammar is given (the empty string for a clip without one)."""
+    _check_decoder(beam_width, lexicon, grammar)
+    if grammar is not None:
+        return grammar.texts(ctc_grammar_decode(outputs, grammar, blank_index=blank_index).words.cpu())
     if beam_width is None:
         ids, lens = ctc_greedy_decode(outputs, blank_index)
     else:
@@ -215,11 +324,14 @@ def decode_batch(outputs: torch.Tensor, dataset, blank_index: int = 0, beam_widt
     return [ids_to_text(row[:n], dataset) for row, n in zip(ids_h, lens_h)]
 
 
-def evaluate_model(model, test_loader, dataset, device, num_samples=5, verbose=True, beam_width=None, lexicon=None):
+def evaluate_model(model, test_loader, dataset, device, num_samples=5, verbose=True, beam_width=None, lexicon=None,
+                   grammar=None):
     """Reference utils.py:38-86 — forward, decode, naive positional character accuracy for the first
     ``num_samples`` items.  One batched decode (K5) per batch instead of one device sync per sample; with
-    ``beam_width`` the decode is ``ctc_beam_decode`` (K5b, optionally with ``lexicon``).
+    ``beam_width`` the decode is ``ctc_beam_decode`` (K5b, optionally with ``lexicon``), with ``grammar`` the best
+    sentence of that ``CtcGrammar`` (K5d).
     Prints the reference's lines when ``verbose`` and returns [(true_text, predicted_text, accuracy %)]."""
+    _check_decoder(beam_width, lexicon, grammar)
     model.eval()
     model.to(device)
     results = []
@@ -231,7 +343,7 @@ def evaluate_model(model, test_loader, dataset, device, num_samples=5, verbose=T
             if i >= num_samples:
                 break
             outputs = model(videos.to(device))
-            texts = decode_batch(outputs, dataset, beam_width=beam_width, lexicon=lexicon)
+            texts = decode_batch(outputs, dataset, beam_width=beam_width, lexicon=lexicon, grammar=grammar)
             for j in range(videos.size(0)):
                 n = i * test_loader.batch_size + j
                 if n >= num_samples:

@@ -288,6 +288,55 @@ AVS_API int avs_ctc_align(const float* logp, int n_clips, int n_steps, int vocab
                           float* out_path_score, int32_t* out_frame_token, int32_t* out_span, float* out_token_prob,
                           void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---------------------------------------------------------------- K5d: exact CTC decoding under a word-slot grammar
+ * A grammar has G slots; slot g lists words W_g, and a sentence is one word of each slot, in slot order, joined by
+ * single spaces (GRID: command colour preposition letter digit adverb, 64 000 sentences).  One CTA per clip runs over
+ * the union of every sentence's CTC lattice: word w (n labels) has its own chain lb, c0, blank, c1, ..., c_{n-1}, tb
+ * (2n + 1 states, K5c's transitions: stay, s-1, and s-2 only between different labels); each slot boundary g < G-1
+ * has one state SP_g carrying the space label, entered from tb(w) and c_last(w) of every word of slot g (and itself)
+ * and leading to lb(w') and c0(w') of every word of slot g+1.  Paths start in lb/c0 of slot 0 and end in tb/c_last of
+ * slot G-1.  Each (sentence, alignment) pair is one path, so, over the clip's first n = input_len frames, in fp64:
+ *   path_score   the best path's log-probability: bit for bit the largest avs_ctc_align path_score over the sentences
+ *                (the same adds in time order);
+ *   loglik       log sum over the grammar's sentences of p(sentence | x) (sentences outside the grammar excluded);
+ *   posterior[w] P(slot g = w): the mass of the paths through word w of slot g, divided by the grammar's total.
+ * Viterbi ties: in a chain the stay, then s-1, then s-2 (lb's s-1 is SP_{g-1}; c0's s-1 is lb and its s-2 SP_{g-1});
+ * at SP_g and at the end the stay, then the lowest word index, and within a word tb before c_last.  A NaN log-prob
+ * counts as -inf.
+ * Outputs per clip:
+ *   words[g]      index within slot g of the word along the best path;
+ *   span[g]       {first frame, end frame (exclusive)} of that word's labels along the best path;
+ *   mbr_words[g]  the arg-max over slot g of posterior (as written, f32), the lowest index on a tie: the decode that
+ *                 minimises the expected number of word errors.
+ * Per-clip status; the other clips of the batch are unaffected:
+ *   invalid (input_len outside [0, n_steps]): path_score and loglik NaN;
+ *   no path of non-zero probability (input_len too short for every sentence, 0 included, or the log-probs every path
+ *   needs are -inf or NaN): path_score and loglik -inf;
+ *   in both cases words, span and mbr_words are -1 and posterior NaN.
+ *
+ * Creation checks, before any CUDA call: 1 <= n_slots <= 16; slot g holds words slot_offsets[g] .. slot_offsets[g+1]
+ * - 1 (1 to 255 of them, no word twice in a slot); word w is word_ids[word_offsets[w] : word_offsets[w+1]], 1 to 64
+ * ids, each in [0, vocab) and neither the blank nor the space; slot_offsets[0] = word_offsets[0] = 0; 2 <= vocab <= 64;
+ * blank and space in [0, vocab) and different; at most 2 048 lattice states (sum over words of 2n + 1, plus G - 1).  It
+ * then uploads the lattice tables with a stream-ordered allocation and copy on `stream`.  destroy waits for the device. */
+typedef struct avs_ctc_grammar avs_ctc_grammar;
+AVS_API int avs_ctc_grammar_create(const int32_t* word_ids, const int32_t* word_offsets, const int32_t* slot_offsets,
+                                   int n_slots, int vocab, int blank, int space, void* stream, avs_ctc_grammar** out);
+AVS_API void avs_ctc_grammar_destroy(avs_ctc_grammar* grammar);
+/* Bytes of device workspace avs_ctc_grammar_decode needs: per clip and frame, the Viterbi backpointers (one byte per
+ * chain state, two per SP state) and the backward value of each SP state (8 bytes), when a clip's total exceeds 32 KB;
+ * below that they live in shared memory and this is 0 (GRID at n_steps = 75: 26 KB).  Also 0 for a NULL grammar and
+ * outside the limits of avs_ctc_grammar_decode. */
+AVS_API size_t avs_ctc_grammar_workspace_bytes(const avs_ctc_grammar* grammar, int n_clips, int n_steps);
+/* logp f32 [n_clips, n_steps, vocab]; input_len i32 [n_clips] (NULL = n_steps for every clip).  out_words,
+ * out_mbr_words i32 [n_clips, G]; out_span i32 [n_clips, G, 2]; out_path_score, out_loglik f32 [n_clips]; out_posterior
+ * f32 [n_clips, W] (W = slot_offsets[G], the words in grammar order).  Checked before any CUDA call: 1 <= n_steps <= 1024,
+ * vocab equal to the grammar's, n_clips >= 0 (0 is a no-op), the workspace size.  No host or device synchronisation. */
+AVS_API int avs_ctc_grammar_decode(const avs_ctc_grammar* grammar, const float* logp, int n_clips, int n_steps,
+                                   int vocab, const int32_t* input_len, int32_t* out_words, int32_t* out_span,
+                                   float* out_path_score, float* out_loglik, float* out_posterior,
+                                   int32_t* out_mbr_words, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------- whole sweep (K2 + K1 + K4)
  * The composed +-S sync sweep of SURVEY.md §3.2: for each clip, visual stats once, audio stats
  * per shift, detector score per shift, arg-max.  The handle owns its device workspace, two
