@@ -68,6 +68,8 @@ SIGNATURES = {
     "avs_gemm_split": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, _P, c_size_t, _P]),
     "avs_sweep_score_workspace_bytes": (c_size_t, [c_int, c_int]),
     "avs_sweep_score": (c_int, [_P, _P, c_int, c_int, c_int, c_int, _P, _P, _P, _P, c_int, _P, _P, _P, c_size_t, _P]),
+    "avs_sweep_score_pairs_workspace_bytes": (c_size_t, [c_int, c_int, c_int, c_int]),
+    "avs_sweep_score_pairs": (c_int, [_P, c_int, _P, c_int, c_int, c_int, c_int, _P, _P, _P, _P, c_int, _P, _P, _P, c_size_t, _P]),
     "avs_ctc_greedy": (c_int, [_P, c_int, c_int, c_int, c_int, _P, _P, _P]),
     "avs_ctc_lexicon_create": (c_int, [POINTER(c_int32), POINTER(c_int32), c_int, c_int, c_int, c_int, _P, POINTER(_P)]),
     "avs_ctc_lexicon_destroy": (None, [_P]),
@@ -99,6 +101,8 @@ SIGNATURES = {
     "avs_sweep_run_ragged_u8": (c_int, [_P, _P, _P, _P, c_int, _P, _P, _P]),
     "avs_sweep_run_windows": (c_int, [_P, _P, _P, c_int, _P, c_int, _P, _P, _P]),
     "avs_sweep_run_windows_u8": (c_int, [_P, _P, _P, c_int, _P, c_int, _P, _P, _P]),
+    "avs_sweep_run_pairs": (c_int, [_P, _P, _P, c_int, _P, c_int, _P, _P, _P]),
+    "avs_sweep_run_pairs_u8": (c_int, [_P, _P, _P, c_int, _P, c_int, _P, _P, _P]),
 }
 # tools build only (make EXPERIMENTS=1 -> libavsync_b200_exp.so, loaded by tools/ through use_experiments_build())
 EXPERIMENT_SIGNATURES = {

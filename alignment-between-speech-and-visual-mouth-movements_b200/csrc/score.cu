@@ -247,6 +247,29 @@ extern "C" int avs_sweep_score(const float* vstats, const float* astats, int n_c
 // relative error ~2^-16) instead of the fp32 CUDA-core GEMM.  The sweep handle asks for it when the STCNN itself runs in
 // bf16 (the visual statistics then carry ~1e-3 of relative error already); the fp32-grade modes and the public
 // avs_sweep_score keep fp32 FFMA accumulation.  The operands are packed on every call: w1 aliases live parameters.
+// hv[n_clips, hidden] = vstats . W1[:, :v_dim]^T + b1 at the start of `workspace` (sized by sweep_score_impl's rules);
+// shared by K4 and the cross-pair scores (pairs.cu), so that both compute hv with the same GEMM and the same splits.
+int avs::score_hidden_gemm(const float* vstats, int n_clips, int v_dim, int a_dim, const float* w1, const float* b1, int hidden,
+                           void* workspace, bool tensor_gemm, cudaStream_t st) {
+  float* hv = static_cast<float*>(workspace);
+  const int ld = v_dim + a_dim;
+  ProfScope ps(PROF_SCORE_GEMM, st);
+  float* partial = hv + align_up(static_cast<size_t>(n_clips) * hidden * sizeof(float), 256) / sizeof(float);
+  if (tensor_gemm) {
+    uint8_t* base = static_cast<uint8_t*>(workspace) + avs_sweep_score_workspace_bytes(n_clips, hidden);
+    __nv_bfloat16* ap = reinterpret_cast<__nv_bfloat16*>(base);
+    __nv_bfloat16* wp = reinterpret_cast<__nv_bfloat16*>(base + align_up(gemm_packed_bytes(n_clips, v_dim, 128), 256));
+    int dev = 0, n_sms = 148, rc;
+    AVS_CUDA(cudaGetDevice(&dev));
+    AVS_CUDA(cudaDeviceGetAttribute(&n_sms, cudaDevAttrMultiProcessorCount, dev));
+    if ((rc = gemm_pack(vstats, v_dim, n_clips, v_dim, 128, ap, st))) return rc;
+    if ((rc = gemm_pack(w1, ld, hidden, v_dim, 256, wp, st))) return rc;
+    return gemm_umma_nt_splitk(ap, wp, b1, hv, hidden, n_clips, hidden, v_dim, tensor_gemm_splits(v_dim), partial, n_sms, st);
+  }
+  return sgemm_nt_splitk(vstats, v_dim, w1, ld, b1, hv, n_clips, hidden, v_dim, score_splits(n_clips, hidden, v_dim),
+                         partial, st);
+}
+
 int avs::sweep_score_impl(const float* vstats, const float* astats, int n_clips, int n_shifts, int v_dim, int a_dim,
                           const float* w1, const float* b1, const float* w2, const float* b2, int hidden, float* out_scores,
                           int32_t* out_best, void* workspace, size_t workspace_bytes, bool tensor_gemm, void* stream) {
@@ -262,25 +285,7 @@ int avs::sweep_score_impl(const float* vstats, const float* astats, int n_clips,
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* hv = static_cast<float*>(workspace);
   const int ld = v_dim + a_dim;
-  int rc;
-  {
-    ProfScope ps(PROF_SCORE_GEMM, st);
-    float* partial = hv + align_up(static_cast<size_t>(n_clips) * hidden * sizeof(float), 256) / sizeof(float);
-    if (tensor_gemm) {
-      uint8_t* base = static_cast<uint8_t*>(workspace) + avs_sweep_score_workspace_bytes(n_clips, hidden);
-      __nv_bfloat16* ap = reinterpret_cast<__nv_bfloat16*>(base);
-      __nv_bfloat16* wp = reinterpret_cast<__nv_bfloat16*>(base + align_up(gemm_packed_bytes(n_clips, v_dim, 128), 256));
-      int dev = 0, n_sms = 148;
-      AVS_CUDA(cudaGetDevice(&dev));
-      AVS_CUDA(cudaDeviceGetAttribute(&n_sms, cudaDevAttrMultiProcessorCount, dev));
-      if ((rc = gemm_pack(vstats, v_dim, n_clips, v_dim, 128, ap, st))) return rc;
-      if ((rc = gemm_pack(w1, ld, hidden, v_dim, 256, wp, st))) return rc;
-      rc = gemm_umma_nt_splitk(ap, wp, b1, hv, hidden, n_clips, hidden, v_dim, tensor_gemm_splits(v_dim), partial, n_sms, st);
-    } else {
-      rc = sgemm_nt_splitk(vstats, v_dim, w1, ld, b1, hv, n_clips, hidden, v_dim, score_splits(n_clips, hidden, v_dim),
-                           partial, st);
-    }
-  }
+  int rc = score_hidden_gemm(vstats, n_clips, v_dim, a_dim, w1, b1, hidden, workspace, tensor_gemm, st);
   if (rc) return rc;
   ProfScope ps(PROF_SCORE, st);
   const size_t sm = (static_cast<size_t>(n_shifts) * a_dim + n_shifts) * sizeof(float);

@@ -41,6 +41,17 @@ size_t sweep_score_workspace_bytes_tensor(int n_clips, int hidden, int v_dim);
 int sweep_score_impl(const float* vstats, const float* astats, int n_clips, int n_shifts, int v_dim, int a_dim,
                      const float* w1, const float* b1, const float* w2, const float* b2, int hidden, float* out_scores,
                      int32_t* out_best, void* workspace, size_t workspace_bytes, bool tensor_gemm, void* stream);
+// K4's hidden-layer GEMM alone: hv[n_clips, hidden] = vstats . W1[:, :v_dim]^T + b1 at the start of `workspace`
+int score_hidden_gemm(const float* vstats, int n_clips, int v_dim, int a_dim, const float* w1, const float* b1, int hidden,
+                      void* workspace, bool tensor_gemm, cudaStream_t st);
+// K4x (pairs.cu): every video against every (track, shift); the pair form of sweep_score_impl.  The check covers every limit
+// and is made before any CUDA call; the workspace holds the hidden-layer GEMM's (tensor or fp32 form) and ha.
+int sweep_score_pairs_check(int n_videos, int n_audios, int n_shifts, int v_dim, int a_dim, int hidden);
+size_t sweep_score_pairs_workspace_bytes(int n_videos, int n_audios, int n_shifts, int hidden, int v_dim, bool tensor_gemm);
+int sweep_score_pairs_impl(const float* vstats, int n_videos, const float* astats, int n_audios, int n_shifts, int v_dim,
+                           int a_dim, const float* w1, const float* b1, const float* w2, const float* b2, int hidden,
+                           float* out_scores, int32_t* out_best, void* workspace, size_t workspace_bytes, bool tensor_gemm,
+                           void* stream);
 
 // ---- tcgen05 path ------------------------------------------------------------------------------
 // Geometry of one layer in the "parity-plane" activation layout (DESIGN.md §K2).

@@ -31,6 +31,10 @@ struct avs_sweep {
   float* astats = nullptr;  // [cap, K, 2*n_mfcc]
   float* d_scores_all = nullptr; int32_t* d_best_all = nullptr;  // host entry point results
   int cap = 0;
+  // run_pairs: statistics of the videos and of the tracks, each sized by its own count, and the K4x workspace
+  float* pair_vstats = nullptr; size_t pair_vstats_bytes = 0;  // [videos, 13824]
+  float* pair_astats = nullptr; size_t pair_astats_bytes = 0;  // [tracks, K, 2*n_mfcc]
+  void* ws_pairs = nullptr; size_t ws_pairs_bytes = 0;
   cudaStream_t side = nullptr, copy = nullptr;
   cudaEvent_t ev_fork = nullptr, ev_logmel = nullptr, ev_join = nullptr, ev_last = nullptr, ev_pre = nullptr, ev_head = nullptr, ev_conv2 = nullptr;
   bool has_last = false;
@@ -105,6 +109,7 @@ extern "C" void avs_sweep_destroy(avs_sweep* s) {
   if (s->has_last) cudaEventSynchronize(s->ev_last);  // the handle's last call may still be running
   cudaFree(s->ws_stcnn); cudaFree(s->ws_mfcc); cudaFree(s->ws_ragged); cudaFree(s->ws_score); cudaFree(s->vstats); cudaFree(s->astats);
   cudaFree(s->d_scores_all); cudaFree(s->d_best_all);
+  cudaFree(s->pair_vstats); cudaFree(s->pair_astats); cudaFree(s->ws_pairs);
   for (int i = 0; i < 2; ++i) {
     cudaFree(s->d_frames[i]); cudaFree(s->d_audio[i]);
     cudaFreeHost(s->h_frames[i]); cudaFreeHost(s->h_audio[i]);
@@ -357,6 +362,88 @@ extern "C" int avs_sweep_run_windows(avs_sweep* s, const avs_mfcc_ragged_plan* p
 extern "C" int avs_sweep_run_windows_u8(avs_sweep* s, const avs_mfcc_ragged_plan* plan, const uint8_t* frames, int stride_frames,
                                         const float* audio, int n_windows, float* out_scores, int32_t* out_best, void* stream) {
   return sweep_run_windows(s, plan, frames, true, stride_frames, audio, n_windows, out_scores, out_best, stream);
+}
+
+// run_pairs buffers, grown like ensure_capacity (geometric, stream-ordered on `st`), each by its own count.  The recorded
+// size is cleared before the allocation, so that a failed one leaves an empty buffer that the next call allocates again.
+static int grow(void** p, size_t* have, size_t need, cudaStream_t st) {
+  if (need <= *have) return AVS_OK;
+  const size_t bytes = std::max(need, *have + *have / 2);
+  if (*p) AVS_CUDA(cudaFreeAsync(*p, st));
+  *p = nullptr;
+  *have = 0;
+  AVS_CUDA(cudaMallocAsync(p, bytes, st));
+  *have = bytes;
+  return AVS_OK;
+}
+static int ensure_pairs_capacity(avs_sweep* s, int n_videos, int n_audios, cudaStream_t st) {
+  const size_t vrow = static_cast<size_t>(AVS_VSTATS) * sizeof(float), arow = static_cast<size_t>(s->K) * 2 * s->n_mfcc * sizeof(float);
+  int rc;
+  if ((rc = grow(reinterpret_cast<void**>(&s->pair_vstats), &s->pair_vstats_bytes, n_videos * vrow, st))) return rc;
+  if ((rc = grow(reinterpret_cast<void**>(&s->pair_astats), &s->pair_astats_bytes, n_audios * arow, st))) return rc;
+  return grow(&s->ws_pairs, &s->ws_pairs_bytes,
+              sweep_score_pairs_workspace_bytes(n_videos, n_audios, s->K, s->hidden, AVS_VSTATS, s->tensor_k4), st);
+}
+
+// Every video against every track: K1 of all tracks on the side stream (chunks of the handle's size, the handle's K1
+// workspaces) beside K2 of all videos on `st`, then K4x.  No audio branch hangs off the STCNN here: the two inputs are
+// independent, so K1 may start at once.
+static int sweep_run_pairs(avs_sweep* s, const avs_mfcc_ragged_plan* rp, const void* frames, bool frames_u8, int n_videos,
+                           const float* audio, int n_audios, float* out_scores, int32_t* out_best, void* stream) {
+  AVS_REQUIRE(s && frames && audio && out_scores && out_best, "null argument");
+  int rc;
+  if ((rc = sweep_score_pairs_check(n_videos, n_audios, s->K, AVS_VSTATS, 2 * s->n_mfcc, s->hidden))) return rc;
+  if (rp) {
+    int rn, rk, rq;
+    mfcc_ragged_shape(rp, &rn, &rk, &rq);
+    AVS_REQUIRE(n_audios == rn, "n_audios differs from the ragged plan's n_clips");
+    AVS_REQUIRE(rk == s->K, "the ragged plan's shift count differs from the sweep's");
+    AVS_REQUIRE(rq == s->n_mfcc, "the ragged plan's n_mfcc differs from the sweep's");
+    AVS_REQUIRE(mfcc_ragged_group(rp) == 0, "a windowed plan cannot be used for cross pairs");
+  }
+  if (n_videos == 0 || n_audios == 0) return AVS_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if ((rc = begin_call(s, st)) || (rc = ensure_pairs_capacity(s, n_videos, n_audios, st)) ||
+      (rp && (rc = ensure_ragged_ws(s, rp, n_audios, st))))
+    return rc;
+  const size_t arow = static_cast<size_t>(s->K) * 2 * s->n_mfcc;
+  AVS_CUDA(cudaEventRecord(s->ev_fork, st));
+  AVS_CUDA(cudaStreamWaitEvent(s->side, s->ev_fork, 0));
+  for (int c0 = 0; c0 < n_audios && !rc; c0 += s->chunk) {
+    const int n = std::min(s->chunk, n_audios - c0);
+    float* ast = s->pair_astats + c0 * arow;
+    if (rp) {
+      if (!(rc = mfcc_ragged_logmel_part(rp, audio, c0, n, s->ws_ragged, s->ws_ragged_bytes, s->side)))
+        rc = mfcc_ragged_stats_part(rp, c0, n, ast, s->ws_ragged, s->ws_ragged_bytes, s->side);
+    } else {
+      rc = avs_mfcc_stats_sweep(s->plan, audio + static_cast<size_t>(c0) * s->n_samples, n, ast, s->ws_mfcc, s->ws_mfcc_bytes,
+                                s->side);
+    }
+  }
+  AVS_CUDA(cudaEventRecord(s->ev_join, s->side));  // recorded even after a failure: `st` must wait for what was enqueued
+  const size_t fstride = kFrameElems * (frames_u8 ? 1 : sizeof(float));
+  for (int c0 = 0; c0 < n_videos && !rc; c0 += s->chunk) {
+    const int n = std::min(s->chunk, n_videos - c0);
+    rc = stcnn_forward_impl(s->net, static_cast<const uint8_t*>(frames) + c0 * fstride, frames_u8, AVS_T, n, s->chunk, true,
+                            StcnnHooks{}, nullptr, s->pair_vstats + static_cast<size_t>(c0) * AVS_VSTATS, nullptr, nullptr,
+                            s->ws_stcnn, s->ws_stcnn_bytes, st);
+  }
+  AVS_CUDA(cudaStreamWaitEvent(st, s->ev_join, 0));
+  if (!rc)
+    rc = sweep_score_pairs_impl(s->pair_vstats, n_videos, s->pair_astats, n_audios, s->K, AVS_VSTATS, 2 * s->n_mfcc, s->w1,
+                                s->b1, s->w2, s->b2, s->hidden, out_scores, out_best, s->ws_pairs, s->ws_pairs_bytes,
+                                s->tensor_k4, st);
+  const int rc2 = end_call(s, st);
+  return rc ? rc : rc2;
+}
+
+extern "C" int avs_sweep_run_pairs(avs_sweep* s, const avs_mfcc_ragged_plan* plan, const float* frames, int n_videos,
+                                   const float* audio, int n_audios, float* out_scores, int32_t* out_best, void* stream) {
+  return sweep_run_pairs(s, plan, frames, false, n_videos, audio, n_audios, out_scores, out_best, stream);
+}
+extern "C" int avs_sweep_run_pairs_u8(avs_sweep* s, const avs_mfcc_ragged_plan* plan, const uint8_t* frames, int n_videos,
+                                      const float* audio, int n_audios, float* out_scores, int32_t* out_best, void* stream) {
+  return sweep_run_pairs(s, plan, frames, true, n_videos, audio, n_audios, out_scores, out_best, stream);
 }
 
 static bool is_pinned(const void* p) {

@@ -5,7 +5,8 @@ Kept names / signatures: ``DetectorConfig``, ``get_video_fps``, ``shift_audio``,
 ``extract_visual_embeddings``, ``FeatureExtractor`` (``build_feature``), ``MisalignmentDetector``,
 ``load_lipnet``, ``save_detector``, ``load_detector``.  New batched entry points: ``SyncSweeper`` /
 ``sync_sweep`` (all clips x all shifts in three kernels, SURVEY.md section 3.2), with ``SyncSweeper.run_ragged`` and
-``audio_stats_sweep_ragged`` for batches whose clips differ in audio length and frame rate.
+``audio_stats_sweep_ragged`` for batches whose clips differ in audio length and frame rate, and ``SyncSweeper.run_pairs`` /
+``sweep_score_pairs`` for every video against every audio track.
 All arithmetic runs in libavsync_b200 (K1, K2, K4); there is no CPU fallback.
 """
 from __future__ import annotations
@@ -374,6 +375,16 @@ class MisalignmentDetector(nn.Module):
         return self.classifier(x).squeeze(-1)
 
 
+def _detector_params(detector: MisalignmentDetector, Dv: int, Da: int):
+    lin1, lin2 = detector.classifier[0], detector.classifier[3]
+    if lin1.in_features != Dv + Da:
+        raise RuntimeError(f"detector expects {lin1.in_features} features, got {Dv}+{Da}")
+    w = [N.f32c(t) for t in (lin1.weight, lin1.bias, lin2.weight, lin2.bias)]
+    for t in w:
+        N.require_cuda(t, "detector parameters")
+    return w, lin1.out_features
+
+
 def sweep_score(vstats: torch.Tensor, astats: torch.Tensor, detector: MisalignmentDetector):
     """K4: vstats [B,Dv], astats [B,K,Da] -> (scores [B,K] = sigmoid(detector(cat[v, a_k])), best [B])."""
     N.require_cuda(vstats, "vstats")
@@ -381,13 +392,7 @@ def sweep_score(vstats: torch.Tensor, astats: torch.Tensor, detector: Misalignme
     vstats, astats = N.f32c(vstats), N.f32c(astats)
     B, K, Da = astats.shape
     Dv = vstats.shape[1]
-    lin1, lin2 = detector.classifier[0], detector.classifier[3]
-    if lin1.in_features != Dv + Da:
-        raise RuntimeError(f"detector expects {lin1.in_features} features, got {Dv}+{Da}")
-    w1, b1, w2, b2 = (N.f32c(t) for t in (lin1.weight, lin1.bias, lin2.weight, lin2.bias))
-    for t in (w1, b1, w2, b2):
-        N.require_cuda(t, "detector parameters")
-    H = lin1.out_features
+    (w1, b1, w2, b2), H = _detector_params(detector, Dv, Da)
     L = N.lib()
     scores = torch.empty((B, K), dtype=torch.float32, device=vstats.device)
     best = torch.empty((B,), dtype=torch.int32, device=vstats.device)
@@ -396,6 +401,32 @@ def sweep_score(vstats: torch.Tensor, astats: torch.Tensor, detector: Misalignme
         N.check(L.avs_sweep_score(N.ptr(vstats), N.ptr(astats), B, K, Dv, Da, N.ptr(w1), N.ptr(b1), N.ptr(w2),
                                   N.ptr(b2), H, N.ptr(scores), N.ptr(best), N.ptr(ws), ws.numel(), N.stream_ptr()),
                 "sweep_score")
+    return scores, best
+
+
+def sweep_score_pairs(vstats: torch.Tensor, astats: torch.Tensor, detector: MisalignmentDetector):
+    """K4x: every video against every audio track at every shift.  vstats [Bv, Dv] (e.g. cached ``visual_stats``),
+    astats [Ba, K, Da] (``audio_stats_sweep``) -> (scores [Bv, Ba, K], best [Bv, Ba]) with
+    ``scores[v, a, k] = sigmoid(detector(cat[vstats[v], astats[a, k]]))`` and ``best`` the arg-max over k (first maximum,
+    NaN wins).  A pair's outputs depend on its video and its track only, bit for bit; they agree with ``sweep_score`` on
+    the same pair up to the last bits (include/avsync.h: avs_sweep_score_pairs).  No host synchronisation."""
+    N.require_cuda(vstats, "vstats")
+    N.require_cuda(astats, "astats")
+    if vstats.dim() != 2 or astats.dim() != 3:
+        raise RuntimeError(f"expected vstats [Bv, Dv] and astats [Ba, K, Da], got {tuple(vstats.shape)} and "
+                           f"{tuple(astats.shape)}")
+    vstats, astats = N.f32c(vstats), N.f32c(astats)
+    (Bv, Dv), (Ba, K, Da) = vstats.shape, astats.shape
+    (w1, b1, w2, b2), H = _detector_params(detector, Dv, Da)
+    scores = torch.empty((Bv, Ba, K), dtype=torch.float32, device=vstats.device)
+    best = torch.empty((Bv, Ba), dtype=torch.int32, device=vstats.device)
+    if Bv == 0 or Ba == 0:
+        return scores, best
+    L = N.lib()
+    ws = N.workspace(L.avs_sweep_score_pairs_workspace_bytes(Bv, Ba, K, H), vstats.device)
+    N.check(L.avs_sweep_score_pairs(N.ptr(vstats), Bv, N.ptr(astats), Ba, K, Dv, Da, N.ptr(w1), N.ptr(b1), N.ptr(w2),
+                                    N.ptr(b2), H, N.ptr(scores), N.ptr(best), N.ptr(ws), ws.numel(), N.stream_ptr()),
+            "sweep_score_pairs")
     return scores, best
 
 
@@ -502,6 +533,42 @@ class SyncSweeper:
         N.check(fn(self.handle.h, plan.handle.h, N.ptr(frames), int(stride_frames), N.ptr(audio), W, N.ptr(scores),
                    N.ptr(best), N.stream_ptr()), "sweep_run_windows")
         return scores, best - self.S, torch.from_numpy(starts).to(frames.device)
+
+    def run_pairs(self, frames: torch.Tensor, audio, fps=None):
+        """Every video against every audio track (active-speaker detection, track choice, cross-clip audits):
+        ``frames`` [Bv, 1, 75, 50, 100] (f32 or u8, as ``run``) and ``audio`` either [Ba, n_samples] (the sweeper's plan)
+        or a list of Ba 1-D CUDA f32 tensors of any lengths (a ragged plan), all on the device.  ``fps`` is the one frame
+        rate of the call (default: the sweeper's); it sets the shifts in samples of every track.  The STCNN runs once per
+        video and K1 once per track.  Returns ``(scores [Bv, Ba, 2S+1], best_shift_frames [Bv, Ba])``; pair (v, a) equals
+        ``sweep_score_pairs`` on the statistics of video v and track a (bit for bit in the fp32-grade modes) and agrees
+        with ``run`` / ``run_ragged`` on the cut pair up to the last bits (DESIGN.md §4.4 K4x)."""
+        N.require_cuda(frames, "frames")
+        frames = self.lipnet._check_frames(frames)
+        Bv = frames.shape[0]
+        fps = self.fps if fps is None else float(fps)
+        ragged = not isinstance(audio, torch.Tensor) or fps != self.fps
+        if ragged:
+            Ba = len(audio)
+        else:
+            N.require_cuda(audio, "audio")
+            audio = N.f32c(audio)
+            if audio.dim() != 2 or audio.shape[1] != self.n_samples:
+                raise RuntimeError(f"audio must be [Ba, {self.n_samples}] or a list of 1-D tensors, got {tuple(audio.shape)}")
+            Ba = audio.shape[0]
+        scores = torch.empty((Bv, Ba, self.K), dtype=torch.float32, device=frames.device)
+        best = torch.empty((Bv, Ba), dtype=torch.int32, device=frames.device)
+        if Bv == 0 or Ba == 0:
+            return scores, best
+        plan = None
+        if ragged:
+            audio = _ragged_audio(list(audio), Ba)
+            row = [shift_samples(k, fps, self.sample_rate) for k in self.shift_frames]
+            rp = mfcc_ragged_plan([a.numel() for a in audio], self.sample_rate, self.n_mfcc, np.array([row] * Ba, np.int32))
+            audio, plan = rp.pack(audio), rp.handle.h
+        fn = N.lib().avs_sweep_run_pairs_u8 if frames.dtype == torch.uint8 else N.lib().avs_sweep_run_pairs
+        N.check(fn(self.handle.h, plan, N.ptr(frames), Bv, N.ptr(audio), Ba, N.ptr(scores), N.ptr(best), N.stream_ptr()),
+                "sweep_run_pairs")
+        return scores, best - self.S
 
     def run_host(self, frames: np.ndarray, audio: np.ndarray):
         u8 = frames.dtype == np.uint8

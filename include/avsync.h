@@ -211,6 +211,24 @@ AVS_API int avs_sweep_score(const float* vstats, const float* astats, int n_clip
                     int hidden, float* out_scores, int32_t* out_best, void* workspace,
                     size_t workspace_bytes, void* stream);
 
+/* ---------------------------------------------------------------- K4x: cross-pair scores
+ * Every video against every audio track at every shift: out_scores[v, a, k] = sigmoid(detector(cat[vstats[v],
+ * astats[a, k]])) for vstats f32 [n_videos, v_dim] and astats f32 [n_audios, n_shifts, a_dim]; detector weights as K4.
+ * out_scores f32 [n_videos, n_audios, n_shifts]; out_best int32 [n_videos, n_audios], the arg-max over the pair's shifts
+ * with K4's rule (first maximum; a NaN wins).  hv = W1[:, :v_dim] . v + b1 comes from K4's fp32 split-K GEMM; then
+ * ha[a, k, h] = W1[h, v_dim:] . astats[a, k] (fp32 fma chain over ascending i from 0) and each score is one fp32 chain
+ * over ascending h of w2[h] * relu(hv + ha), + b2, K4's sigmoid.  A pair's outputs depend on its video and its track only.
+ * The ReLU propagates NaN: a NaN statistic gives NaN scores for its pairs only.  Limits (AVS_EINVAL before any CUDA
+ * call): n_videos, n_audios >= 0 (either 0: nothing is launched), n_shifts >= 1, v_dim % 8 == 0, a_dim in [1, 256],
+ * hidden in [1, 65536], n_audios * n_shifts <= 2^31 - 257, n_videos <= 8 388 480.  AVS_EWORKSPACE if the workspace is too small.
+ * The scores differ from avs_sweep_score's on the same pair in the last bits only (association of hv + W1a . a and the
+ * order of the sum over h; DESIGN.md §4.4 K4x). */
+AVS_API size_t avs_sweep_score_pairs_workspace_bytes(int n_videos, int n_audios, int n_shifts, int hidden);
+AVS_API int avs_sweep_score_pairs(const float* vstats, int n_videos, const float* astats, int n_audios, int n_shifts,
+                          int v_dim, int a_dim, const float* w1, const float* b1, const float* w2, const float* b2,
+                          int hidden, float* out_scores, int32_t* out_best, void* workspace,
+                          size_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------- K5: greedy CTC decode
  * Replaces the arithmetic of decode_prediction (utils.py:20-30): per step arg-max over the vocab
  * (first index on ties), drop repeats and blanks.  logp device f32 [n_clips, n_steps, vocab];
@@ -386,6 +404,17 @@ AVS_API int avs_sweep_run_windows(avs_sweep* sw, const avs_mfcc_ragged_plan* pla
 AVS_API int avs_sweep_run_windows_u8(avs_sweep* sw, const avs_mfcc_ragged_plan* plan, const uint8_t* frames,
                              int stride_frames, const float* audio, int n_windows, float* out_scores,
                              int32_t* out_best, void* stream);
+/* Cross pairs (K4x above): every one of n_videos clips' frames (device f32 or u8 [n_videos, 1, 75, 50, 100]) against
+ * every one of n_audios audio tracks at each of the handle's shifts.  plan == NULL: audio is [n_audios, n_samples] under
+ * the handle's uniform plan; otherwise plan is a ragged plan of n_audios clips (not a windowed one; n_shifts and n_mfcc
+ * the handle's) and audio is packed at its offsets.  The videos go through K2 in the handle's chunks, the tracks through
+ * K1 on the handle's side stream beside them, hv through the handle's own hidden-layer GEMM (the tensor-core form with a
+ * bf16 STCNN, as avs_sweep_run).  Outputs as avs_sweep_score_pairs; serialised and grown like the handle's other calls.
+ * In the fp32-grade modes the outputs equal avs_sweep_score_pairs on the statistics of K2 and K1, bit for bit. */
+AVS_API int avs_sweep_run_pairs(avs_sweep* sw, const avs_mfcc_ragged_plan* plan, const float* frames, int n_videos,
+                        const float* audio, int n_audios, float* out_scores, int32_t* out_best, void* stream);
+AVS_API int avs_sweep_run_pairs_u8(avs_sweep* sw, const avs_mfcc_ragged_plan* plan, const uint8_t* frames, int n_videos,
+                           const float* audio, int n_audios, float* out_scores, int32_t* out_best, void* stream);
 /* ---------------------------------------------------------------- decode metrics (SURVEY 8f-3)
  * Edit distances behind calculate_cer / calculate_wer (train.py:945-993) and the positional character
  * matches of evaluate_model (utils.py:83-86) for a batch of id sequences that are already on the device
