@@ -10,7 +10,7 @@ error behaviour) over the C-ABI library ``libavsync_b200.so`` (``include/avsync.
         load_lipnet, save_detector}                  utils.evaluate_model
     misalignment_detection_train.{SyncSweeper, sync_sweep, sweep_score_pairs, audio_stats_sweep_ragged, audio_stats_sweep_windows,
         window_bounds}, utils.{ctc_greedy_decode, ctc_beam_decode, CtcLexicon, ctc_forced_align, CtcAlignment,
-        align_words, ctc_grammar_decode, CtcGrammar, CtcGrammarResult}, dataset.{GRID_WORDS, GRID_SLOTS, grid_lexicon,
+        align_words, ctc_grammar_decode, CtcGrammar, CtcGrammarResult, ctc_loss}, model.LipNet.gru_head_train, dataset.{GRID_WORDS, GRID_SLOTS, grid_lexicon,
         grid_grammar, read_grid_align}                                                             (new, batched)
     distributed.{shard_range, sweep_sharded, gather_scores, ddp_detector_step, GraphedDetectorStep}        (new, multi-GPU)
 
@@ -20,7 +20,7 @@ repo root aliases it).
 from . import _native
 from .model import LipNet
 from .utils import (CtcAlignment, CtcGrammar, CtcGrammarResult, CtcLexicon, align_words, ctc_beam_decode,
-                    ctc_forced_align, ctc_grammar_decode, ctc_greedy_decode, decode_batch, decode_metrics,
+                    ctc_forced_align, ctc_grammar_decode, ctc_greedy_decode, ctc_loss, decode_batch, decode_metrics,
                     decode_prediction, evaluate_model)
 from .misalignment_detection_train import (DetectorConfig, FeatureExtractor, MisalignmentDataset, MisalignmentDetector,
                                            SyncSweeper, run_epoch,
@@ -38,4 +38,4 @@ __all__ = ["LipNet", "ctc_greedy_decode", "decode_batch", "decode_prediction", "
            "shift_samples", "get_video_fps", "resample_audio", "default_audio_loader", "sweep_score", "sweep_score_pairs", "sync_sweep", "visual_stats", "GridPreprocessor", "distributed",
            "CtcLexicon", "ctc_beam_decode", "GRID_WORDS", "grid_lexicon",
            "CtcAlignment", "ctc_forced_align", "align_words", "read_grid_align",
-           "CtcGrammar", "CtcGrammarResult", "ctc_grammar_decode", "GRID_SLOTS", "grid_grammar"]
+           "CtcGrammar", "CtcGrammarResult", "ctc_grammar_decode", "GRID_SLOTS", "grid_grammar", "ctc_loss"]

@@ -77,6 +77,12 @@ SIGNATURES = {
     "avs_ctc_beam": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P, c_size_t, _P]),
     "avs_ctc_align_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "avs_ctc_align": (c_int, [_P, c_int, c_int, c_int, c_int, _P, _P, c_int, _P, _P, _P, _P, _P, _P, _P, c_size_t, _P]),
+    "avs_ctc_loss_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "avs_ctc_loss": (c_int, [_P, c_int, c_int, c_int, c_int, _P, _P, c_int, _P, _P, c_int, _P, _P, _P, c_size_t, _P]),
+    "avs_bigru_train_workspace_bytes": (c_size_t, [c_int] * 6),
+    "avs_bigru_train_forward": (c_int, [c_int] * 4 + [_P] * 11 + [c_int, c_int, _P, _P, c_float, _P, _P, c_size_t, _P]),
+    "avs_bigru_train_backward": (c_int, [c_int] * 4 + [_P] * 11 + [c_int, c_int, _P, _P, c_float, _P] + [_P] * 10
+                                 + [_P, c_size_t, _P]),
     "avs_ctc_grammar_create": (c_int, [POINTER(c_int32), POINTER(c_int32), POINTER(c_int32), c_int, c_int, c_int, c_int,
                                        _P, POINTER(_P)]),
     "avs_ctc_grammar_destroy": (None, [_P]),

@@ -12,20 +12,13 @@
 // add is correctly rounded, so a float64 restatement doing the same adds in the same order (oracle/ctc_align_ref.py)
 // gets the same bits and takes the same decisions.
 #include <math.h>
-#include "common.cuh"
+#include "ctc_lattice.cuh"
 
 namespace {
 
-constexpr int kMaxSteps = 1024;
-constexpr int kMaxVocab = 64;
-constexpr int kMaxTarget = 512;
-constexpr int kMaxThreads = 256;
-constexpr int kPer = (2 * kMaxTarget + 1 + kMaxThreads - 1) / kMaxThreads;   // states per thread at most
+using namespace avs::ctc;
 constexpr size_t kSmemBackptr = 32768;   // one byte per (frame, state): in shared memory up to this size
 
-int n_threads(int max_target_len) {
-  return static_cast<int>(std::min<size_t>(kMaxThreads, avs::align_up(2 * max_target_len + 1, 32)));
-}
 size_t backptr_bytes(int n_steps, int max_target_len) {
   return static_cast<size_t>(n_steps) * (2 * max_target_len + 1);
 }
@@ -35,19 +28,6 @@ size_t smem_bytes(int n_steps, int max_target_len) {
   const size_t ints = (static_cast<size_t>(n_steps) + 2 * max_target_len) * sizeof(int);   // frame tokens, spans
   return dp + ints + (backptr_in_smem(n_steps, max_target_len) ? backptr_bytes(n_steps, max_target_len) : 0);
 }
-bool in_limits(int n_steps, int vocab, int blank, int max_target_len) {
-  return n_steps >= 1 && n_steps <= kMaxSteps && vocab >= 2 && vocab <= kMaxVocab && blank >= 0 && blank < vocab &&
-         max_target_len >= 0 && max_target_len <= kMaxTarget;
-}
-
-__device__ __forceinline__ double lp_of(float x) { return isnan(x) ? -INFINITY : static_cast<double>(x); }
-
-__device__ __forceinline__ double lse3(double a, double b, double c) {   // log(exp(a) + exp(b) + exp(c))
-  const double m = fmax(a, fmax(b, c));
-  if (m == -INFINITY) return -INFINITY;
-  return m + log(exp(a - m) + exp(b - m) + exp(c - m));
-}
-
 __global__ void ctc_align_kernel(
     const float* __restrict__ logp, int n_steps, int vocab, int blank, const int32_t* __restrict__ input_len,
     const int32_t* __restrict__ targets, int lmax, const int32_t* __restrict__ target_len, float* out_loglik,
@@ -80,12 +60,7 @@ __global__ void ctc_align_kernel(
 #pragma unroll
     for (int j = 0; j < kPer; ++j) {
       const int s = tid + j * nthr;
-      lab[j] = blank;
-      skip[j] = false;
-      if (s < S && (s & 1)) {
-        lab[j] = y[s >> 1];
-        skip[j] = s >= 3 && y[s >> 1] != y[(s >> 1) - 1];
-      }
+      state_label(y, blank, S, s, lab[j], skip[j]);
       e[j] = s < S ? lp[lab[j]] : 0.f;
     }
 #pragma unroll
@@ -114,7 +89,7 @@ __global__ void ctc_align_kernel(
         if (v2 > v) { v = v2; b = 2; }
         vn[s] = v + x;
         bpt[s] = b;
-        an[s] = lse3(ap[s], s >= 1 ? ap[s - 1] : -INFINITY, skip[j] ? ap[s - 2] : -INFINITY) + x;
+        an[s] = alpha_step(ap, s, skip[j], x);
       }
       cur ^= 1;
     }
@@ -125,7 +100,7 @@ __global__ void ctc_align_kernel(
       const double ps = vf[end];
       s_aligned = ps > -INFINITY;
       s_ps = ps;
-      s_ll = !s_aligned ? -INFINITY : S > 1 ? lse3(af[S - 1], af[S - 2], -INFINITY) : af[0];
+      s_ll = !s_aligned ? -INFINITY : alpha_final(af, S);
       if (s_aligned) {
         int s = end;
         for (int t = n - 1; t >= 1; --t) {

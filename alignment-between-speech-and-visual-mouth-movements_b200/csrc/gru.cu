@@ -11,6 +11,7 @@
 #include "sgemm.cuh"
 #include "gemm_umma.cuh"
 #include "gru_umma.cuh"
+#include "gru.cuh"
 
 struct avs_bigru {
   int in_dim, H, V, precision;
@@ -291,6 +292,78 @@ static int dup(float** dst, const float* src, size_t n, cudaStream_t st) {
   return AVS_OK;
 }
 
+__global__ void dropout_apply_kernel(const float* x, const uint8_t* __restrict__ mask, float scale, float* y, size_t n) {
+  for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < n; i += static_cast<size_t>(gridDim.x) * blockDim.x)
+    y[i] = x[i] * static_cast<float>(mask[i]) * scale;
+}
+
+int dropout_apply(const float* x, const uint8_t* mask, float scale, float* y, size_t n, cudaStream_t st) {
+  dropout_apply_kernel<<<static_cast<int>(std::min<size_t>(4096, (n + 255) / 256)), 256, 0, st>>>(x, mask, scale, y, n);
+  AVS_LAUNCHED();
+  return AVS_OK;
+}
+
+int transpose_whh(const float* w, float* wt, int H, cudaStream_t st) {
+  transpose_whh_kernel<<<256, 256, 0, st>>>(w, wt, H);
+  AVS_LAUNCHED();
+  return AVS_OK;
+}
+
+int head_forward(const HeadW* g, const float* emb, int B, int T, float* const xp[2], float* const outs[2],
+                        const uint8_t* const masks[2], float keep_scale, float* const* drop, __nv_bfloat16* ap,
+                        float* out_logp, cudaStream_t st) {
+  const int H = g->H, rows = B * T;
+  const size_t sm = static_cast<size_t>(2) * kGruClips * H * sizeof(float);
+  const float* x = emb;
+  const int ins[2] = {g->in_dim, 2 * H};
+  int rc;
+  for (int l = 0; l < 2; ++l) {
+    if (g->precision == AVS_PREC_FP32) {
+      ProfScope ps(PROF_GRU_GEMM, st);
+      if ((rc = sgemm_nt(x, ins[l], g->w_ih[l], ins[l], g->b_ih[l], xp[l], 6 * H, rows, 6 * H, ins[l], st))) return rc;
+    } else {
+      { ProfScope ps(PROF_GRU_PACK, st); if ((rc = gemm_pack(x, ins[l], rows, ins[l], 128, ap, st))) return rc; }
+      ProfScope ps(PROF_GRU_GEMM, st);
+      if ((rc = gemm_umma_nt(ap, g->w_ih_packed[l], g->b_ih[l], xp[l], 6 * H, rows, 6 * H, ins[l], g->n_sms, st))) return rc;
+    }
+    ProfScope psr(PROF_GRU_REC, st);
+#ifdef AVS_EXPERIMENTS
+    const bool force_fma = getenv("AVS_GRU_FMA") != nullptr;  // tools build: CUDA-core recurrence instead of the tcgen05 one
+#else
+    constexpr bool force_fma = false;
+#endif
+    if (g->w_hh_packed[l] != nullptr && !force_fma) {
+      if ((rc = gru_recurrence_umma(xp[l], g->w_hh_packed[l], g->b_hh[l], outs[l], B, T, st))) return rc;
+    } else if (H == kCluH) {
+      cudaLaunchConfig_t cfg{};
+      cfg.gridDim = dim3(kClu * cdiv(B, kCluClips), 2, 1);
+      cfg.blockDim = dim3(256, 1, 1);
+      cfg.dynamicSmemBytes = kCluSmem;
+      cfg.stream = st;
+      cudaLaunchAttribute attr[1];
+      attr[0].id = cudaLaunchAttributeClusterDimension;
+      attr[0].val.clusterDim.x = kClu; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+      cfg.attrs = attr; cfg.numAttrs = 1;
+      AVS_CUDA(cudaFuncSetAttribute(gru_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kCluSmem)));
+      AVS_CUDA(cudaLaunchKernelEx(&cfg, gru_cluster_kernel, static_cast<const float*>(xp[l]), g->w_hh[l], g->b_hh[l], outs[l], B, T));
+      AVS_LAUNCHED();
+    } else {
+      gru_recurrence_kernel<kGruClips><<<dim3(cdiv(B, kGruClips), 2), H, sm, st>>>(xp[l], g->w_hh_t[l], g->b_hh[l], outs[l], B, T, H);
+      AVS_LAUNCHED();
+    }
+    x = outs[l];
+    if (masks[l]) {
+      if ((rc = dropout_apply(outs[l], masks[l], keep_scale, drop[l], static_cast<size_t>(rows) * 2 * H, st))) return rc;
+      x = drop[l];
+    }
+  }
+  ProfScope psf(PROF_GRU_FC, st);
+  if ((rc = sgemm_nt(x, 2 * H, g->fc_w, 2 * H, g->fc_b, out_logp, g->V, rows, g->V, 2 * H, st))) return rc;
+  log_softmax_kernel<<<cdiv(rows, 4), 128, 0, st>>>(out_logp, rows, g->V);
+  AVS_LAUNCHED();
+  return AVS_OK;
+}
+
 }  // namespace avs
 
 using namespace avs;
@@ -374,53 +447,14 @@ extern "C" int avs_bigru_forward(const avs_bigru* g, const float* emb, int B, in
     set_error("bigru workspace too small: %zu < %zu", workspace_bytes, w.total);
     return AVS_EWORKSPACE;
   }
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int H = g->H, rows = B * T;
-  const size_t sm = static_cast<size_t>(2) * kGruClips * H * sizeof(float);
-  const float* x = emb;
-  float* outs[2] = {w.o1, w.o2};
-  const int ins[2] = {g->in_dim, 2 * H};
-  int rc;
+  HeadW p{g->in_dim, g->H, g->V, g->precision, g->n_sms};
   for (int l = 0; l < 2; ++l) {
-    if (g->precision == AVS_PREC_FP32) {
-      ProfScope ps(PROF_GRU_GEMM, st);
-      if ((rc = sgemm_nt(x, ins[l], g->w_ih[l], ins[l], g->b_ih[l], w.xp, 6 * H, rows, 6 * H, ins[l], st))) return rc;
-    } else {
-      { ProfScope ps(PROF_GRU_PACK, st); if ((rc = gemm_pack(x, ins[l], rows, ins[l], 128, w.ap, st))) return rc; }
-      ProfScope ps(PROF_GRU_GEMM, st);
-      if ((rc = gemm_umma_nt(w.ap, g->w_ih_packed[l], g->b_ih[l], w.xp, 6 * H, rows, 6 * H, ins[l], g->n_sms, st))) return rc;
-    }
-    ProfScope psr(PROF_GRU_REC, st);
-#ifdef AVS_EXPERIMENTS
-    const bool force_fma = getenv("AVS_GRU_FMA") != nullptr;  // tools build: CUDA-core recurrence instead of the tcgen05 one
-#else
-    constexpr bool force_fma = false;
-#endif
-    if (g->w_hh_packed[l] != nullptr && !force_fma) {
-      if ((rc = gru_recurrence_umma(w.xp, g->w_hh_packed[l], g->b_hh[l], outs[l], B, T, st))) return rc;
-    } else if (H == kCluH) {
-      cudaLaunchConfig_t cfg{};
-      cfg.gridDim = dim3(kClu * cdiv(B, kCluClips), 2, 1);
-      cfg.blockDim = dim3(256, 1, 1);
-      cfg.dynamicSmemBytes = kCluSmem;
-      cfg.stream = st;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = kClu; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-      cfg.attrs = attr; cfg.numAttrs = 1;
-      AVS_CUDA(cudaFuncSetAttribute(gru_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kCluSmem)));
-      AVS_CUDA(cudaLaunchKernelEx(&cfg, gru_cluster_kernel, static_cast<const float*>(w.xp), static_cast<const float*>(g->w_hh[l]),
-                                  static_cast<const float*>(g->b_hh[l]), outs[l], B, T));
-      AVS_LAUNCHED();
-    } else {
-      gru_recurrence_kernel<kGruClips><<<dim3(cdiv(B, kGruClips), 2), H, sm, st>>>(w.xp, g->w_hh_t[l], g->b_hh[l], outs[l], B, T, H);
-      AVS_LAUNCHED();
-    }
-    x = outs[l];
+    p.w_ih[l] = g->w_ih[l]; p.b_ih[l] = g->b_ih[l]; p.w_hh[l] = g->w_hh[l]; p.w_hh_t[l] = g->w_hh_t[l];
+    p.b_hh[l] = g->b_hh[l]; p.w_ih_packed[l] = g->w_ih_packed[l]; p.w_hh_packed[l] = g->w_hh_packed[l];
   }
-  ProfScope psf(PROF_GRU_FC, st);
-  if ((rc = sgemm_nt(w.o2, 2 * H, g->fc_w, 2 * H, g->fc_b, out_logp, g->V, rows, g->V, 2 * H, st))) return rc;
-  log_softmax_kernel<<<cdiv(rows, 4), 128, 0, st>>>(out_logp, rows, g->V);
-  AVS_LAUNCHED();
-  return AVS_OK;
+  p.fc_w = g->fc_w; p.fc_b = g->fc_b;
+  float* const xp[2] = {w.xp, w.xp};
+  float* const outs[2] = {w.o1, w.o2};
+  const uint8_t* const masks[2] = {nullptr, nullptr};
+  return head_forward(&p, emb, B, T, xp, outs, masks, 1.f, nullptr, w.ap, out_logp, static_cast<cudaStream_t>(stream));
 }

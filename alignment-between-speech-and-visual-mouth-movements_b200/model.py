@@ -4,7 +4,8 @@ Same constructor, attribute names and ``state_dict`` keys as the reference modul
 ``lipnet_final.pth`` loads in both the bare and the ``{'model_state_dict': ...}`` form,
 misalignment_detection_train.py:299-309), but ``forward`` does not call ATen/cuDNN: the
 STCNN runs in ``avs_stcnn_forward`` (K2) and the Bi-GRU head in ``avs_bigru_forward`` (K3).
-Eval mode only (the north-star path is inference; LipNet training is out of scope).
+``forward``, ``stcnn`` and ``gru_head`` are eval mode only; ``gru_head_train`` trains the Bi-GRU head on frozen STCNN
+embeddings (``avs_bigru_train_forward`` / ``avs_bigru_train_backward``, K3b).
 """
 from __future__ import annotations
 
@@ -142,7 +143,68 @@ class LipNet(nn.Module):
                 "bigru_forward")
         return out
 
+    def _head_params(self):
+        names = ["weight_ih_l0", "weight_hh_l0", "bias_ih_l0", "bias_hh_l0"]
+        return ([getattr(g, n + s) for g in (self.gru1, self.gru2) for n in names for s in ("", "_reverse")]
+                + [self.fc.weight, self.fc.bias])
+
+    def gru_head_train(self, emb: torch.Tensor, dropout: float = 0.0) -> torch.Tensor:
+        """gru1 -> dropout -> gru2 -> dropout -> fc -> log_softmax (model.py:84-95) with gradients: [B,T,6912] -> log-probs
+        [B,T,vocab] with a ``grad_fn`` whose backward (K3b) fills the ``.grad`` of ``gru1.*``, ``gru2.*`` and ``fc.*``.
+        The STCNN is frozen: ``emb`` must not require grad (take it from ``stcnn`` under ``torch.no_grad()``).  Works
+        whatever ``self.training`` is.  ``dropout`` is the reference's ``dropout_gru1`` / ``dropout_gru2`` rate; the keep
+        masks are drawn with torch's RNG.  With ``dropout=0`` the log-probs equal ``gru_head``'s bit for bit."""
+        if emb.requires_grad:
+            raise ValueError("emb requires grad, but the STCNN backward is not implemented: pass a detached embedding")
+        if not 0.0 <= dropout < 1.0:
+            raise ValueError(f"dropout must be in [0, 1), got {dropout}")
+        N.require_cuda(emb, "emb")
+        if emb.dim() != 3 or emb.shape[2] != self.conv_output_dim:
+            raise ValueError(f"emb must be [B, T, {self.conv_output_dim}], got {tuple(emb.shape)}")
+        N.device_check()
+        params = self._head_params()
+        for p in params:
+            N.require_cuda(p, "LipNet parameters")
+        B, T, _ = emb.shape
+        masks = (None, None)
+        if dropout > 0.0:
+            shape = (B, T, 2 * self.hidden_dim)
+            masks = tuple(torch.empty(shape, dtype=torch.uint8, device=emb.device).bernoulli_(1.0 - dropout)
+                          for _ in range(2))
+        stacked = [torch.stack([params[i], params[i + 1]]) for i in range(0, 16, 2)]   # [2][...]: forward, reverse
+        return _HeadTrain.apply(self, N.f32c(emb), masks, float(dropout), *stacked, params[16], params[17])
+
     def forward(self, x: torch.Tensor) -> torch.Tensor:
         """(B, 1, T, H, W) float32 -> (B, T, vocab) log-probabilities (model.py:57-97)."""
         with torch.no_grad():
             return self.gru_head(self.stcnn(x))
+
+
+class _HeadTrain(torch.autograd.Function):
+    """The head's training forward and backward over the 10 parameter tensors in avsync.h's stacked layout."""
+
+    @staticmethod
+    def forward(ctx, net, emb, masks, p, *params):
+        B, T, _ = emb.shape
+        L = N.lib()
+        w = [N.f32c(t) for t in params]
+        dims = (net.conv_output_dim, net.hidden_dim, net.vocab_size, N.PREC[net.precision])
+        out = torch.empty((B, T, net.vocab_size), dtype=torch.float32, device=emb.device)
+        ws = N.workspace(L.avs_bigru_train_workspace_bytes(*dims, B, T), emb.device)
+        N.check(L.avs_bigru_train_forward(*dims, *[N.ptr(t) for t in w], N.ptr(emb), B, T, N.ptr(masks[0]),
+                                          N.ptr(masks[1]), p, N.ptr(out), N.ptr(ws), ws.numel(), N.stream_ptr()),
+                "bigru_train_forward")
+        ctx.dims, ctx.p, ctx.masks, ctx.ws, ctx.w, ctx.emb = dims, p, masks, ws, w, emb
+        ctx.shapes = [t.shape for t in params]
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        B, T, _ = ctx.emb.shape
+        g = grad_out.to(torch.float32).contiguous()
+        grads = [torch.empty(s, dtype=torch.float32, device=g.device) for s in ctx.shapes]
+        N.check(N.lib().avs_bigru_train_backward(*ctx.dims, *[N.ptr(t) for t in ctx.w], N.ptr(ctx.emb), B, T,
+                                                 N.ptr(ctx.masks[0]), N.ptr(ctx.masks[1]), ctx.p, N.ptr(g),
+                                                 *[N.ptr(t) for t in grads], N.ptr(ctx.ws), ctx.ws.numel(),
+                                                 N.stream_ptr()), "bigru_train_backward")
+        return (None, None, None, None, *grads)

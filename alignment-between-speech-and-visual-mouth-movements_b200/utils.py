@@ -153,6 +153,74 @@ def ctc_forced_align(logp: torch.Tensor, targets: torch.Tensor, target_lens: tor
     return out
 
 
+class _CtcLoss(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, log_probs, targets, input_lengths, target_lengths, blank, reduction, zero_infinity):
+        B, T, V = log_probs.shape
+        L = N.lib()
+        nll = torch.empty((B,), dtype=torch.float32, device=log_probs.device)
+        ws = N.workspace(L.avs_ctc_loss_workspace_bytes(B, T, targets.shape[1]), log_probs.device)
+        N.check(L.avs_ctc_loss(N.ptr(log_probs), B, T, V, blank, N.ptr(input_lengths), N.ptr(targets), targets.shape[1],
+                               N.ptr(target_lengths), None, int(zero_infinity), N.ptr(nll), None, N.ptr(ws), ws.numel(),
+                               N.stream_ptr()), "ctc_loss")
+        ctx.save_for_backward(log_probs, targets, input_lengths, target_lengths)
+        ctx.blank, ctx.reduction, ctx.zero_infinity = blank, reduction, zero_infinity
+        if reduction == "none":
+            return nll
+        if reduction == "sum":
+            return nll.sum()
+        return (nll / target_lengths.clamp(min=1)).mean()
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        log_probs, targets, input_lengths, target_lengths = ctx.saved_tensors
+        B, T, V = log_probs.shape
+        if ctx.reduction == "none":
+            scale = grad_out
+        elif ctx.reduction == "sum":
+            scale = grad_out.expand(B)
+        else:
+            scale = grad_out / (target_lengths.clamp(min=1) * B)
+        scale = scale.to(torch.float32).contiguous()
+        L = N.lib()
+        nll = torch.empty((B,), dtype=torch.float32, device=log_probs.device)
+        grad = torch.empty_like(log_probs)
+        ws = N.workspace(L.avs_ctc_loss_workspace_bytes(B, T, targets.shape[1]), log_probs.device)
+        N.check(L.avs_ctc_loss(N.ptr(log_probs), B, T, V, ctx.blank, N.ptr(input_lengths), N.ptr(targets),
+                               targets.shape[1], N.ptr(target_lengths), N.ptr(scale), int(ctx.zero_infinity), N.ptr(nll),
+                               N.ptr(grad), N.ptr(ws), ws.numel(), N.stream_ptr()), "ctc_loss")
+        return grad, None, None, None, None, None, None
+
+
+def ctc_loss(log_probs: torch.Tensor, targets: torch.Tensor, input_lengths, target_lengths, blank: int = 0,
+             reduction: str = "mean", zero_infinity: bool = False) -> torch.Tensor:
+    """CTC loss (K5e) with its gradient, differentiable with respect to ``log_probs``.  Unlike
+    ``torch.nn.functional.ctc_loss``, log_probs are batch-first [B, T, V] like LipNet's output (and ``ctc_forced_align``'s
+    input), and targets are padded [B, Lmax].  ``reduction`` follows ``F.ctc_loss``: "none" gives the per-clip losses,
+    "sum" their sum, "mean" the batch mean of each loss divided by ``target_length.clamp(min=1)``.  ``zero_infinity``
+    turns the loss of a clip without an alignment of non-zero probability (+inf, NaN gradient) into 0 with gradient 0.
+    An invalid clip (an id outside [0, V) or equal to the blank, a length out of range) and a NaN log-prob inside
+    input_length give NaN.  The loss is the float64 forward of K5c, so ``ctc_loss(..., reduction="none")`` equals
+    ``-ctc_forced_align(...).loglik`` bit for bit on NaN-free log-probs.  One launch forward, one backward, no host sync.
+    Limits: 1 <= T <= 1024, 2 <= V <= 64, 0 <= Lmax <= 512."""
+    N.require_cuda(log_probs, "log_probs")
+    if log_probs.dim() != 3:
+        raise ValueError("log_probs must be [B, T, V] (batch first)")
+    if reduction not in ("none", "mean", "sum"):
+        raise ValueError(f"reduction must be 'none', 'mean' or 'sum', got {reduction!r}")
+    B = log_probs.shape[0]
+    dev = log_probs.device
+    targets = torch.as_tensor(targets)
+    if targets.dim() != 2 or targets.shape[0] != B:
+        raise ValueError(f"targets must be padded [B={B}, Lmax], got {tuple(targets.shape)}")
+    input_lengths, target_lengths = torch.as_tensor(input_lengths), torch.as_tensor(target_lengths)
+    if tuple(input_lengths.shape) != (B,) or tuple(target_lengths.shape) != (B,):
+        raise ValueError(f"input_lengths and target_lengths must be [B={B}]")
+    lp = log_probs.to(torch.float32).contiguous()
+    return _CtcLoss.apply(lp, _i32_on(targets, dev), _i32_on(input_lengths, dev), _i32_on(target_lengths, dev),
+                          int(blank), reduction, bool(zero_infinity))
+
+
 def align_words(logp: torch.Tensor, texts: Sequence[str], char_to_idx: Optional[Dict[str, int]] = None,
                 fps: float = 25.0, space: str = " ", blank_index: int = 0, input_lens: Optional[torch.Tensor] = None
                 ) -> List[Tuple[List[Tuple[str, float, float, float]], float]]:

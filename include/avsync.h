@@ -192,6 +192,35 @@ AVS_API size_t avs_bigru_workspace_bytes(const avs_bigru* head, int n_clips, int
 AVS_API int avs_bigru_forward(const avs_bigru* head, const float* emb, int n_clips, int n_steps,
                       float* out_logp, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---------------------------------------------------------------- K3 training forward and K3b backward
+ * Training of the head, the STCNN frozen.  Parameters as for avs_bigru_create, taken by pointer on every call (nothing is
+ * cached between optimizer steps).  The forward derives the transposed / packed weights into the workspace and enqueues
+ * avs_bigru_forward's kernels in its order: without keep masks its log-probs equal avs_bigru_forward's bit for bit.
+ * Dropout (reference dropout_gru1 / dropout_gru2) follows each GRU layer: y = x * keep_mask * (1 / (1 - dropout_p)),
+ * keep masks u8 [n_clips, n_steps, 2 * hidden] drawn by the caller; both NULL = no dropout.  The workspace keeps what
+ * the backward needs: pass the same workspace, parameters, embeddings and masks to avs_bigru_train_backward, which
+ * turns dL/dlogp f32 [n_clips, n_steps, vocab] into the gradients of all 18 head parameters, in the stacked layouts of
+ * the parameters (the fc weight and bias unstacked).  The embedding gets no gradient.  Deterministic: no atomics.
+ * Checked before any CUDA call: hidden a multiple of 32 in [32, 1024]; in_dim a positive multiple of 8 (of 32 unless
+ * precision is AVS_PREC_FP32); 1 <= vocab <= 4096; n_clips >= 0, n_steps >= 1, align8(n_clips * n_steps) *
+ * max(6 * hidden, in_dim, align8(vocab)) < 2^31; both masks or neither; 0 <= dropout_p < 1 with masks; null pointers;
+ * the workspace size.  n_clips = 0: the forward does nothing, the backward zeroes the gradients. */
+AVS_API size_t avs_bigru_train_workspace_bytes(int in_dim, int hidden, int vocab, int precision, int n_clips, int n_steps);
+AVS_API int avs_bigru_train_forward(int in_dim, int hidden, int vocab, int precision,
+                            const float* g1_w_ih, const float* g1_w_hh, const float* g1_b_ih, const float* g1_b_hh,
+                            const float* g2_w_ih, const float* g2_w_hh, const float* g2_b_ih, const float* g2_b_hh,
+                            const float* fc_w, const float* fc_b, const float* emb, int n_clips, int n_steps,
+                            const uint8_t* keep_mask1, const uint8_t* keep_mask2, float dropout_p, float* out_logp,
+                            void* workspace, size_t workspace_bytes, void* stream);
+AVS_API int avs_bigru_train_backward(int in_dim, int hidden, int vocab, int precision,
+                             const float* g1_w_ih, const float* g1_w_hh, const float* g1_b_ih, const float* g1_b_hh,
+                             const float* g2_w_ih, const float* g2_w_hh, const float* g2_b_ih, const float* g2_b_hh,
+                             const float* fc_w, const float* fc_b, const float* emb, int n_clips, int n_steps,
+                             const uint8_t* keep_mask1, const uint8_t* keep_mask2, float dropout_p,
+                             const float* grad_logp, float* d_g1_w_ih, float* d_g1_w_hh, float* d_g1_b_ih,
+                             float* d_g1_b_hh, float* d_g2_w_ih, float* d_g2_w_hh, float* d_g2_b_ih, float* d_g2_b_hh,
+                             float* d_fc_w, float* d_fc_b, void* workspace, size_t workspace_bytes, void* stream);
+
 /* fp32-grade GEMM on tcgen05 (the K3 input-projection kernel, exposed for unit tests and for the
  * DFT-as-GEMM comparison in profiles/): C[M,N] = A[M,K] . W[N,K]^T + bias[N], all device f32 row-major,
  * operands split hi/lo in bf16 (three products, fp32 accumulate).  K % 32 == 0, N % 4 == 0. */
@@ -305,6 +334,27 @@ AVS_API int avs_ctc_align(const float* logp, int n_clips, int n_steps, int vocab
                           const int32_t* targets, int target_stride, const int32_t* target_len, float* out_loglik,
                           float* out_path_score, int32_t* out_frame_token, int32_t* out_span, float* out_token_prob,
                           void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------- K5e: CTC loss and its gradient
+ * One CTA per clip over K5c's lattice and limits, in fp64: the forward (K5c's transition code) gives
+ * nll = -log p(y | x), equal bit for bit to -loglik of avs_ctc_align on NaN-free log-probs; with out_grad, a backward
+ * pass gives grad[b, t, k] = -scale[b] * gamma_t(k), gamma_t(k) the posterior occupancy of label k at frame t: the
+ * partial derivative of scale[b] * nll[b] with respect to logp[b, t, k] (torch's ctc_loss returns exp(lp) - gamma
+ * instead: the same gradient for logits after log_softmax).  Frames at or past input_len get gradient 0.
+ * Per-clip status; the other clips of the batch are unaffected:
+ *   invalid (as in avs_ctc_align): nll NaN, gradient NaN on every frame;
+ *   a NaN log-prob inside input_len: nll NaN, gradient NaN inside input_len;
+ *   no alignment of non-zero probability: nll +inf, gradient NaN inside input_len; with zero_infinity, 0 and 0. */
+/* Bytes of device workspace avs_ctc_loss needs (the forward variables, 8 bytes per (frame, state)); 0 outside the
+ * limits. */
+AVS_API size_t avs_ctc_loss_workspace_bytes(int n_clips, int n_steps, int max_target_len);
+/* logp, input_len, targets, target_stride, target_len as for avs_ctc_align.  scale f32 [n_clips] (device; may be NULL
+ * when out_grad is NULL); out_nll f32 [n_clips]; out_grad f32 [n_clips, n_steps, vocab] or NULL for the loss alone.
+ * Checked before any CUDA call: the limits of avs_ctc_align, null pointers, the workspace size.  No synchronisation. */
+AVS_API int avs_ctc_loss(const float* logp, int n_clips, int n_steps, int vocab, int blank, const int32_t* input_len,
+                         const int32_t* targets, int target_stride, const int32_t* target_len, const float* scale,
+                         int zero_infinity, float* out_nll, float* out_grad, void* workspace, size_t workspace_bytes,
+                         void* stream);
 
 /* ---------------------------------------------------------------- K5d: exact CTC decoding under a word-slot grammar
  * A grammar has G slots; slot g lists words W_g, and a sentence is one word of each slot, in slot order, joined by
