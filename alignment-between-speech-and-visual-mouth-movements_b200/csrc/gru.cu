@@ -442,6 +442,7 @@ extern "C" int avs_bigru_forward(const avs_bigru* g, const float* emb, int B, in
                                  size_t workspace_bytes, void* stream) {
   AVS_REQUIRE(g && emb && out_logp && workspace, "null argument");
   if (B <= 0 || T <= 0) return AVS_OK;
+  AVS_REQUIRE(static_cast<long long>(B) * T <= kHeadMaxRows, "n_clips * n_steps must be <= 8388480");
   GruWs w = carve(g, B, T, workspace);
   if (workspace_bytes < w.total) {
     set_error("bigru workspace too small: %zu < %zu", workspace_bytes, w.total);

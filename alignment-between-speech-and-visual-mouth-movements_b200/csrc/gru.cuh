@@ -3,6 +3,9 @@
 #pragma once
 #include "common.cuh"
 namespace avs {
+// Most rows (n_clips * n_steps) of one call: the fc product (and the fp32 projections, and the backward's dh2 and dx)
+// run on sgemm_nt's tiled kernel over all rows, whose grid has gridDim.y = ceil(rows / 128) <= 65535
+constexpr int kHeadMaxRows = 65535 * 128;
 // Parameters of the head, with the derived forms the kernels read: w_hh_t (generic recurrence), w_ih_packed
 // (tensor-core projections) and w_hh_packed (tcgen05 recurrence, H = 256), null where the precision does not use them.
 struct HeadW {

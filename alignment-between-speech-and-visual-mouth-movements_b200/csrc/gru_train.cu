@@ -30,6 +30,8 @@ namespace avs {
 namespace {
 
 constexpr int kBpttClips = 2;   // clips per CTA of the BPTT kernel (4 spills at 1024 threads)
+// transpose_pad_kernel's grid has gridDim.y = ceil(cols / 32) <= 65535, and the embedding's transpose has cols = in_dim
+constexpr int kTrainMaxInDim = 65535 * 32;
 
 struct TrainWs {
   float* w_hh_t[2];
@@ -90,6 +92,7 @@ bool head_args_ok(int in_dim, int H, int V, int precision, int B, int T) {
       B < 0 || T < 1)
     return false;
   if (precision != AVS_PREC_FP32 && in_dim % 32) return false;
+  if (static_cast<long long>(B) * T > kHeadMaxRows || in_dim > kTrainMaxInDim) return false;
   const long long width = std::max<long long>({6LL * H, in_dim, static_cast<long long>(align_up(V, 8))});
   return static_cast<long long>(align_up(static_cast<size_t>(B) * T, 8)) * width <= INT_MAX;
 }
@@ -101,6 +104,8 @@ int check_head_args(int in_dim, int H, int V, int precision, int B, int T, const
   AVS_REQUIRE(V >= 1 && V <= 4096, "vocab must be in [1, 4096]");
   AVS_REQUIRE(precision >= 0 && precision <= 2, "precision must be AVS_PREC_FP32, AVS_PREC_BF16 or AVS_PREC_BF16X3");
   AVS_REQUIRE(B >= 0 && T >= 1, "n_clips must be >= 0 and n_steps >= 1");
+  AVS_REQUIRE(static_cast<long long>(B) * T <= kHeadMaxRows, "n_clips * n_steps must be <= 8388480");
+  AVS_REQUIRE(in_dim <= kTrainMaxInDim, "in_dim must be <= 2097120");
   AVS_REQUIRE(head_args_ok(in_dim, H, V, precision, B, T), "n_clips * n_steps * max(6 * hidden, in_dim, vocab) must be < 2^31");
   AVS_REQUIRE((m1 == nullptr) == (m2 == nullptr), "pass both keep masks or neither");
   AVS_REQUIRE(m1 == nullptr || (p >= 0.f && p < 1.f), "dropout_p must be in [0, 1)");

@@ -188,7 +188,8 @@ AVS_API int avs_bigru_create(int in_dim, int hidden, int vocab,
                      const float* fc_w, const float* fc_b, int precision, void* stream, avs_bigru** out);
 AVS_API void avs_bigru_destroy(avs_bigru* head);
 AVS_API size_t avs_bigru_workspace_bytes(const avs_bigru* head, int n_clips, int n_steps);
-/* emb: device f32 [n_clips, n_steps, in_dim]; out_logp: device f32 [n_clips, n_steps, vocab]. */
+/* emb: device f32 [n_clips, n_steps, in_dim]; out_logp: device f32 [n_clips, n_steps, vocab].
+ * n_clips * n_steps <= 8 388 480 (AVS_EINVAL before any CUDA call): the fc product runs over all rows at once. */
 AVS_API int avs_bigru_forward(const avs_bigru* head, const float* emb, int n_clips, int n_steps,
                       float* out_logp, void* workspace, size_t workspace_bytes, void* stream);
 
@@ -202,8 +203,10 @@ AVS_API int avs_bigru_forward(const avs_bigru* head, const float* emb, int n_cli
  * turns dL/dlogp f32 [n_clips, n_steps, vocab] into the gradients of all 18 head parameters, in the stacked layouts of
  * the parameters (the fc weight and bias unstacked).  The embedding gets no gradient.  Deterministic: no atomics.
  * Checked before any CUDA call: hidden a multiple of 32 in [32, 1024]; in_dim a positive multiple of 8 (of 32 unless
- * precision is AVS_PREC_FP32); 1 <= vocab <= 4096; n_clips >= 0, n_steps >= 1, align8(n_clips * n_steps) *
- * max(6 * hidden, in_dim, align8(vocab)) < 2^31; both masks or neither; 0 <= dropout_p < 1 with masks; null pointers;
+ * precision is AVS_PREC_FP32) and <= 2 097 120; 1 <= vocab <= 4096; n_clips >= 0, n_steps >= 1,
+ * n_clips * n_steps <= 8 388 480, align8(n_clips * n_steps) * max(6 * hidden, in_dim, align8(vocab)) < 2^31 (the
+ * two limits are launch grids: 128 rows per CTA of the products over all rows, 32 embedding columns per CTA of the
+ * backward's transpose, at most 65535 CTAs each; the workspace size is 0 past them); both masks or neither; 0 <= dropout_p < 1 with masks; null pointers;
  * the workspace size.  n_clips = 0: the forward does nothing, the backward zeroes the gradients. */
 AVS_API size_t avs_bigru_train_workspace_bytes(int in_dim, int hidden, int vocab, int precision, int n_clips, int n_steps);
 AVS_API int avs_bigru_train_forward(int in_dim, int hidden, int vocab, int precision,

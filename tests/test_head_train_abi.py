@@ -87,6 +87,39 @@ def test_train_rejects_bad_arguments_without_a_device(native, fn):
         assert _train_call(L, fn, n_clips=0, ws=None)[0] == 0
 
 
+# sgemm_nt's tiled kernel has gridDim.y = ceil(rows / 128) and runs over all n_clips * n_steps rows (fc, the fp32
+# projections, the backward's dh2 and dx); transpose_pad_kernel has gridDim.y = ceil(cols / 32) and the backward transposes
+# the embedding (in_dim columns).  gridDim.y <= 65535.
+MAX_ROWS = 65535 * 128       # 8 388 480
+MAX_IN_DIM = 65535 * 32      # 2 097 120
+PAST_LIMITS = [  # (in_dim, hidden, vocab, prec, n_clips, n_steps), each just past one limit; message text
+    ((8, 32, 1, 0, MAX_ROWS + 1, 1), "n_clips * n_steps must be <= 8388480"),
+    ((8, 32, 1, 0, 1, MAX_ROWS + 1), "n_clips * n_steps must be <= 8388480"),
+    ((32, 32, 1, 2, 2796161, 3), "n_clips * n_steps must be <= 8388480"),   # 8 388 483 rows
+    ((MAX_IN_DIM + 8, 32, 1, 0, 1, 1), "in_dim must be <= 2097120"),
+    ((2097152, 32, 1, 2, 1, 1), "in_dim must be <= 2097120"),
+]
+INSIDE_LIMITS = [(8, 32, 1, 0, MAX_ROWS, 1), (8, 32, 1, 0, 1, MAX_ROWS), (32, 32, 1, 2, 2796160, 3),
+                 (MAX_IN_DIM, 32, 1, 0, 1, 1), (MAX_IN_DIM, 32, 1, 2, 1, 1)]
+
+
+@pytest.mark.parametrize("fn", ["forward", "backward"])
+def test_train_rejects_shapes_past_the_launch_limits_without_a_device(native, fn):
+    """Both shapes pass the older 2^31 bound on align8(rows) * width, but would fail a launch after kernels were queued."""
+    L = native.lib()
+    for (in_dim, H, V, prec, B, T), text in PAST_LIMITS:
+        assert L.avs_bigru_train_workspace_bytes(in_dim, H, V, prec, B, T) == 0, (in_dim, B, T)
+        rc, msg = _train_call(L, fn, in_dim=in_dim, hidden=H, vocab=V, prec=prec, n_clips=B, n_steps=T)
+        assert rc == -1 and text in msg, (in_dim, B, T, msg)
+
+
+def test_train_workspace_bytes_at_the_launch_limits(native):
+    """Just inside each limit the shape is accepted (no call: it would launch kernels on the fake pointers)."""
+    L = native.lib()
+    for args in INSIDE_LIMITS:
+        assert L.avs_bigru_train_workspace_bytes(*args) > 0, args
+
+
 def test_train_workspace_bytes(native):
     L = native.lib()
     small = L.avs_bigru_train_workspace_bytes(6912, 256, 39, 2, 1, 75)

@@ -246,6 +246,19 @@ def test_k3_bf16_head_is_the_bf16x3_head(A):
 
 
 @pytest.mark.gpu
+def test_k3_refuses_rows_past_the_fc_grid_limit(A):
+    """The fc product runs on sgemm_nt's tiled kernel over all n_clips * n_steps rows, gridDim.y = ceil(rows / 128) <=
+    65535: one row more is refused before any launch (the pointers past the handle are never touched)."""
+    N = A._native
+    head = Head(N, gru_params(32, 8, 1, seed=1), 8, 32, 1, "fp32")
+    fake = ctypes.c_void_p(256)
+    for B, T in ((65535 * 128 + 1, 1), (1, 65535 * 128 + 1), (2796161, 3)):
+        assert N.lib().avs_bigru_forward(head.handle.h, fake, B, T, fake, fake, 1 << 40, N.stream_ptr()) == -1
+        assert "n_clips * n_steps must be <= 8388480" in N.lib().avs_last_error_string().decode()
+    torch.cuda.synchronize()
+
+
+@pytest.mark.gpu
 def test_k3_lipnet_hidden128_gru_head_vs_f64(A):
     """The drop-in module with a non-default hidden size: LipNet(39, hidden_dim=128).gru_head at in_dim 6912 (generic
     recurrence, tcgen05 projections with N = 768)."""
